@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py --gpus 1 ... --dump-outputs DIR           # also write the last timed step's tokens / logits as .npy
 
 One "step" = `--tokens-per-step` (default 64) greedy decode tokens of the named model, batch 1.
 Workload at N=1: Qwen3-8B architecture, random-init weights exported with group size 64 through
@@ -69,7 +70,7 @@ def bench_checkpoint(model: str, gs: int, seed: int = 0) -> str:
 
     shape = synth.SHAPES[model]
     base = "/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK) else "/tmp"
-    d = os.path.join(base, "q3_bench")
+    d = os.path.join(base, f"q3_bench-{os.getuid()}")  # per user: another user's cache directory is not writable
     os.makedirs(d, exist_ok=True)
     path = os.path.join(d, f"{model}_gs{gs}_s{seed}.bin")
     want = synth.checkpoint_bytes(shape, gs)
@@ -321,6 +322,38 @@ def prefill_4b_line(args, device) -> dict:
 
 
 # ---------------------------------------------------------------------------------------------
+# outputs of the timed path (--dump-outputs)
+# ---------------------------------------------------------------------------------------------
+def device_logits(m) -> np.ndarray:
+    """The handle's device logits buffer (q3_logits_device) copied to the host without running a step: the logits the
+    last decode step computed."""
+    import types
+
+    import torch
+
+    from qwen3_rs_b200 import transformer as T
+
+    ptr = T.load_library().q3_logits_device(m._h)
+    buf = types.SimpleNamespace(__cuda_array_interface__={
+        "shape": (m.get_config().vocab_size,), "typestr": "<f4", "data": (ptr, False), "version": 2})
+    return torch.as_tensor(buf, device="cuda").cpu().numpy()
+
+
+def dump_last_step(m, tok0: int, pos0: int, tps: int, out_dir: str) -> None:
+    """Writes what the last timed step (q3_bench_decode: tps greedy tokens from tok0 at pos0) computed: decode_logits.npy,
+    the logits of its last position read from the device, and decode_tokens.npy, its greedy tokens.  q3_bench_decode keeps
+    the tokens on the device, so the step is run once more through q3_decode_greedy (the same launches on the same cache);
+    the rerun must leave bit-identical logits, or the tokens would not be the timed step's."""
+    logits = device_logits(m)
+    tokens = np.array(m.decode_greedy(tok0, pos0, tps), np.float64)
+    if not np.array_equal(device_logits(m), logits):
+        raise SystemExit("bench.py: the last timed step, run again, computed other logits")
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "decode_logits.npy"), logits)
+    np.save(os.path.join(out_dir, "decode_tokens.npy"), tokens)
+
+
+# ---------------------------------------------------------------------------------------------
 # main arm
 # ---------------------------------------------------------------------------------------------
 def main():
@@ -339,12 +372,16 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-prefill", action="store_true")
     ap.add_argument("--decode-path", type=int, default=-1)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's greedy tokens and last logits as DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        raise SystemExit("bench.py: --dump-outputs writes the CUDA path's outputs on one GPU (--impl ours, no torchrun)")
     need = (args.steps + args.warmup) * args.tokens_per_step + 8
     if args.ctx < need:
         args.ctx = need
@@ -412,6 +449,8 @@ def main():
     dev_ms, wall_ms = times.tolist()
     n_tok = args.steps * tps
     value = n_tok / (dev_ms / 1e3)
+    if args.dump_outputs:
+        dump_last_step(m, tok0, pos - tps, tps, args.dump_outputs)
 
     # ---- end to end through the reference-facing call: forward -> host logits -> host argmax ----
     # same positions as `value`: the cache below pos_start is refilled untimed, then every one of the n_tok

@@ -1,6 +1,7 @@
 import hashlib
 import json
 import os
+import shutil
 import sys
 
 import numpy as np
@@ -11,7 +12,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
-CKPT_DIR = os.environ.get("Q3_CKPT_DIR", "/tmp/q3_ckpt")
+# Q3_CKPT_DIR: keep the exported synthetic checkpoints between sessions (by default each session exports its own into a
+# temporary directory that it removes at the end)
+CKPT_DIR = os.environ.get("Q3_CKPT_DIR")
 
 
 def pytest_configure(config):
@@ -39,16 +42,17 @@ def golden_meta():
 
 
 @pytest.fixture(scope="session")
-def ckpt():
+def ckpt(tmp_path_factory):
     """ckpt(shape_name, group_size, seed) -> path of the exported synthetic checkpoint (cached)."""
     from qwen3_rs_b200 import synth
 
-    os.makedirs(CKPT_DIR, exist_ok=True)
+    d = CKPT_DIR or str(tmp_path_factory.mktemp("ckpt"))
+    os.makedirs(d, exist_ok=True)
 
     def get(name: str, gs: int = 64, seed: int = 0) -> str:
         if (name, gs, seed) == ("micro", 32, 7):
             return os.path.join(GOLDEN_DIR, "micro_gs32.bin")
-        path = os.path.join(CKPT_DIR, f"{name}_gs{gs}_s{seed}.bin")
+        path = os.path.join(d, f"{name}_gs{gs}_s{seed}.bin")
         want = synth.checkpoint_bytes(synth.SHAPES[name], gs)
         if not (os.path.exists(path) and os.path.getsize(path) == want):
             tmp = path + f".tmp{os.getpid()}"
@@ -56,7 +60,9 @@ def ckpt():
             os.replace(tmp, path)
         return path
 
-    return get
+    yield get
+    if not CKPT_DIR:
+        shutil.rmtree(d, ignore_errors=True)  # the Qwen3-0.6B checkpoint alone is 0.6 GB
 
 
 GOLDEN_CASES = [("micro", 32, 7), ("tiny", 64, 0), ("tiny-untied", 64, 1), ("small", 128, 2)]
