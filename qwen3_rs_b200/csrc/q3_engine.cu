@@ -1848,8 +1848,11 @@ extern "C" int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, cons
     const int Tpad = (T + 127) / 128 * 128, ng = K / gs;
     DevBuf dxq, dxsT, dwq, dws, dwsT, dout;
     if ((rc = dxq.alloc((size_t)Tpad * K)) || (rc = dxsT.alloc((size_t)ng * Tpad * 4)) || (rc = dwq.alloc((size_t)N * K)) ||
-        (rc = dws.alloc((size_t)N * ng * 4)) || (rc = dwsT.alloc((size_t)N * ng * 4)) || (rc = dout.alloc((size_t)T * N * 4)))
+        (rc = dws.alloc((size_t)N * ng * 4)) || (rc = dwsT.alloc((size_t)N * ng * 4)) || (rc = dout.alloc((size_t)Tpad * N * 4)))
         return rc;
+    // output sentinel: every byte 0xFF (a NaN) -- an element the kernel skips reads back as NaN, and the padding rows past T,
+    // which the epilogue must never store, are checked below
+    CK(cudaMemset(dout.p, 0xFF, (size_t)Tpad * N * 4));
     CK(cudaMemset(dxq.p, 0, (size_t)Tpad * K));
     CK(cudaMemcpy(dxq.p, xq, (size_t)T * K, cudaMemcpyHostToDevice));
     std::vector<float> xsT((size_t)ng * Tpad, 0.0f);
@@ -1868,6 +1871,13 @@ extern "C" int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, cons
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy(out, dout.p, (size_t)T * N * 4, cudaMemcpyDeviceToHost));
+    std::vector<uint32_t> pad((size_t)(Tpad - T) * N);
+    if (!pad.empty()) {
+        CK(cudaMemcpy(pad.data(), dout.as<float>() + (size_t)T * N, pad.size() * 4, cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < pad.size(); i++)
+            if (pad[i] != 0xFFFFFFFFu)
+                return fail(Q3_ECUDA, "GEMM wrote padding row %d (T %d) at column %d", T + (int)(i / N), T, (int)(i % N));
+    }
     return Q3_OK;
 }
 

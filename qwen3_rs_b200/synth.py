@@ -75,6 +75,9 @@ SHAPES: Dict[str, Shape] = {
     "small": Shape("small", 512, 1536, 4, 8, 4, vocab_size=4096, max_seq_len=512, tied=True),
     "micro": Shape("micro", 128, 384, 2, 2, 1, vocab_size=256, max_seq_len=64, tied=False),
     "small8": Shape("small8", 512, 2048, 3, 16, 8, vocab_size=4096, max_seq_len=256, tied=False),  # 8 kv heads: tensor parallel up to 8
+    # wider than 4096 like Qwen3-32B (5120): the dim > 4096 prefill norm kernel, and the graph decode path as the default (the
+    # persistent kernel declines this width); GQA 8, n_heads * 128 == dim; at T 640 every prefill GEMM has more tiles than SMs
+    "wide": Shape("wide", 5120, 3072, 2, 40, 5, vocab_size=4096, max_seq_len=2048, tied=False),
 }
 
 

@@ -11,7 +11,7 @@ import bench
 from oracle import binding as orc
 from qwen3_rs_b200 import transformer as T
 from qwen3_rs_b200.sampler import argmax_last
-from test_gpu_parity import LOGIT_TOL, check_layerwise
+from test_gpu_parity import LOGIT_TOL, check_layerwise, check_prefill_vs_oracle
 
 pytestmark = [pytest.mark.gpu, pytest.mark.slow]
 
@@ -97,3 +97,34 @@ def test_8b_attention_over_32k_cache_matches_oracle(big):
         np.testing.assert_allclose(v[0], vo[layer, npos].reshape(-1), rtol=0, atol=1e-4)
     finally:
         o.close()
+
+
+@pytest.mark.parametrize("name", ["qwen3-4b", "qwen3-8b"])
+def test_prefill_2048_prefix_chunk_rerun_invariance_and_oracle(big, name):
+    """The bench's prefill workload, T 2048 (up to 21 GEMM tiles per CTA): a rerun, the chunks 1000 + 1048 and a 48-token prefix
+    give bit-identical K / V rows of every layer (and logits); the 48-token prefill against the oracle.  Rows 0..47 sit in m-tile 0:
+    for n-tile n that is tile 16 n, which a CTA runs on its iteration 16 n / grid, so they cover later tile iterations too."""
+    from test_gpu_prefill_scale import assert_same_rows
+
+    m, path = big(name, 4096)
+    c = m.get_config()
+    toks = np.random.default_rng(7).integers(0, c.vocab_size, 2048).tolist()
+
+    def run(chunks):
+        m.reset()
+        for a, b in chunks:
+            lg = m.prefill(toks[a:b], a)
+        return lg
+
+    lg = run([(0, 2048)])
+    full = [m.kv_read(l, 0, 2048) for l in range(c.n_layers)]
+    for label, chunks in (("rerun", [(0, 2048)]), ("chunks 1000 + 1048", [(0, 1000), (1000, 2048)])):
+        lg2 = run(chunks)
+        for l in range(c.n_layers):
+            assert_same_rows([m.kv_read(l, 0, 2048)], [full[l]], 2048, f"{name} {label} (layer {l})")
+        assert np.array_equal(lg2, lg), f"{name} {label}: logits differ"
+    run([(0, 48)])
+    assert_same_rows([m.kv_read(l, 0, 48) for l in range(c.n_layers)], full, 48, f"{name} 48-token prefix")
+    del full
+    orc.set_threads(os.cpu_count() or 1)
+    check_prefill_vs_oracle(m, path, toks[:48], name, 64)

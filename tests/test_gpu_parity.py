@@ -213,7 +213,9 @@ def check_layerwise(m, o, o2, tokens, label=""):
     print(f"{label} layerwise |dx|/scale: gpu median {np.median(gpu_x):.2e} worst {gpu_x.max():.2e} "
           f"(>1e-3: {np.mean(gpu_x > 1e-3):.0%}); oracle re-association median {np.median(ref_x):.2e} "
           f"worst {ref_x.max():.2e} (>1e-3: {np.mean(ref_x > 1e-3):.0%}); |dlogit| gpu {gpu_lg:.2e} ref {ref_lg:.2e}")
-    assert np.median(gpu_x) <= 1e-5
+    # median: at round-off, unless the oracle's own re-association is not (2 layers of a 5120-wide synthetic model: layer 0
+    # flips an int8 activation at almost every position, see check_prefill_vs_oracle)
+    assert np.median(gpu_x) <= max(1e-5, 3 * np.median(ref_x))
     assert gpu_x.max() <= 3 * ref_x.max() + 1e-3
     assert gpu_lg <= LOGIT_TOL
 
@@ -638,14 +640,36 @@ def test_prefill_matches_oracle(models, ckpt, name, gs, seed, T):
     every layer and the logits of the last token.  Layer 0 depends only on embedding -> norm -> QKV GEMM -> QK-norm / RoPE
     (nothing can cascade): 1e-4.  Deeper layers see the attention output re-quantised to int8: most rows agree to float
     round-off (median), a flipped int8 moves a row by a quantisation step, bounded by the fast-mode envelope."""
-    m, o = models(name, gs, seed), orc.Model(ckpt(name, gs, seed))
-    c = o.config
+    m = models(name, gs, seed)
     rng = np.random.default_rng(T + 1)
-    toks = rng.integers(0, c["vocab_size"], T).tolist()
+    check_prefill_vs_oracle(m, ckpt(name, gs, seed), rng.integers(0, m.get_config().vocab_size, T).tolist(), f"{name} gs{gs}")
+
+
+def check_prefill_vs_oracle(m, path, toks, label, ctx=None):
+    """The checks of test_prefill_matches_oracle for model `m` against the oracle of checkpoint `path` on prompt `toks`."""
+    o, o2 = orc.Model(path, ctx), orc.Model(path, ctx)
+    try:
+        _check_prefill_vs_oracle(m, o, o2, toks, label)
+    finally:
+        o.close()
+        o2.close()
+
+
+def _check_prefill_vs_oracle(m, o, o2, toks, label):
+    c = o.config
+    T = len(toks)
     o.reset()
+    o2.reset()
+    xd = o.dump_residuals()
     for p, t in enumerate(toks):
         lo = o.forward(t, p)
+        orc.set_perturb(1)  # the oracle's own re-association noise on layer 0: o2 runs it on the same embedding row, sums re-associated
+        try:
+            o2.forward_layers(xd[0], p, 0, 1)
+        finally:
+            orc.set_perturb(0)
     ko, vo = o.kv_cache()
+    ko2, vo2 = o2.kv_cache()
     m.reset()
     lg = m.prefill(toks, 0)
     kvd = c["n_kv_heads"] * c["head_dim"]
@@ -660,8 +684,16 @@ def test_prefill_matches_oracle(models, ckpt, name, gs, seed, T):
             # the rows here (24 / 130 on small gs128, 60 / 200 on small gs64; the sequential decode path flips the very same rows:
             # scripts/diag/prefill_rows.py).  On the CPU alone (scripts/diag/layer0_ties.py, tests/test_oracle.py): 57 % of these
             # rows hold an element within 1e-6 of a tie, and moving the normalisation factor by ONE ulp changes 23 % of them.
-            rows_off = float(np.mean(ek.max(axis=1) > 1e-4))
-            assert np.median(ek) <= 1e-6 and np.median(ev) <= 1e-6 and rows_off <= 0.4 and ek.max() <= 2e-2, (rows_off, float(ek.max()))
+            # A row flips when ANY of its dim elements does, so the share of such rows grows with the width (dim 512: <= 30 %,
+            # 2560 .. 5120: 75 .. 95 %) -- and with it the median error.  The yardstick is therefore the oracle itself with
+            # re-associated sums (o2): the GPU must not flip more rows, nor by more, than that does (and never more than a step).
+            ek2 = np.abs(ko2[0, :T].reshape(T, kvd) - kr)
+            ev2 = np.abs(vo2[0, :T].reshape(T, kvd) - vr)
+            rows_off, rows_ref = float(np.mean(ek.max(axis=1) > 1e-4)), float(np.mean(ek2.max(axis=1) > 1e-4))
+            print(f"{label} prefill layer 0: rows off the oracle {rows_off:.0%} (oracle re-association {rows_ref:.0%}), median |dK| "
+                  f"{np.median(ek):.1e} ({np.median(ek2):.1e}), max {ek.max():.1e} ({ek2.max():.1e})")
+            assert np.median(ek) <= max(1e-6, 3 * np.median(ek2)) and np.median(ev) <= max(1e-6, 3 * np.median(ev2)), label
+            assert rows_off <= max(0.4, 1.25 * rows_ref) and ek.max() <= 2e-2, (rows_off, rows_ref, float(ek.max()))
         # deeper layers: an upstream flip perturbs every later element a little (and, through attention, later tokens), so only the
         # noise level is checked here -- the attention kernel itself is compared with float64 in test_prefill_attention_kernels_...
         assert np.median(ev) <= 1e-2 * max(1.0, float(np.abs(vr).max())), (l, float(np.median(ev)))
@@ -669,11 +701,13 @@ def test_prefill_matches_oracle(models, ckpt, name, gs, seed, T):
         k1, v1 = m.kv_read(l, T, 1)
         assert not k1.any() and not v1.any()
     err = float(np.abs(lg - lo).max())
-    print(f"{name} gs{gs} prefill T={T} vs oracle: max|dlogit| {err:.2e} (|logit| max {np.abs(lo).max():.1f})")
+    print(f"{label} prefill T={T} vs oracle: max|dlogit| {err:.2e} (|logit| max {np.abs(lo).max():.1f})")
     assert err <= 0.05 * float(np.abs(lo).max()) + LOGIT_TOL
 
 
-@pytest.mark.parametrize("T,pos0,n_heads,n_kv", [(70, 0, 8, 2), (33, 45, 4, 4), (129, 3, 16, 2), (200, 0, 2, 1)])
+@pytest.mark.parametrize("T,pos0,n_heads,n_kv", [(70, 0, 8, 2), (33, 45, 4, 4), (129, 3, 16, 2), (200, 0, 2, 1),
+                                                 (1000, 1100, 40, 5), (517, 1531, 16, 8),
+                                                 pytest.param(2048, 0, 32, 8, marks=pytest.mark.slow)])
 def test_prefill_attention_kernels_against_float64(T, pos0, n_heads, n_kv):
     """The batched causal attention alone (the tensor-core kernel q3_prefill runs -- FP16 hi / lo split --, the f32 CUDA-core
     kernel and the first tensor-core version, 3xTF32) against a float64 softmax attention: f32-class accuracy (1e-5 of the
