@@ -206,11 +206,10 @@ int q3_op_expf(int device, const float *x, int n, float *out);
 int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, const int8_t *wq, const float *ws,
                   int T, int N, int K, int gs, int exact, float *out);
 /* layers.rs:374-419 for T query tokens at once (the batched prefill's causal attention): q [T][n_heads*128] after QK-norm
- * and RoPE, k / v [pos0+T][n_kv*128] cache rows, out [T][n_heads*128].  f32_cuda_cores == 0: the tensor-core kernel
- * q3_prefill runs (mma.sync m16n8k16 on an FP16 hi / lo split of the operands, f32 accumulation); 1: the f32 CUDA-core
- * kernel; 2: the first tensor-core version (mma.sync TF32 with the 3xTF32 split). */
+ * and RoPE, k / v [pos0+T][n_kv*128] cache rows, out [T][n_heads*128].  The tensor-core kernel q3_prefill runs
+ * (mma.sync m16n8k16 on an FP16 hi / lo split of the operands, f32 accumulation). */
 int q3_op_prefill_attention(int device, const float *q, const float *k, const float *v, int T, int pos0, int n_heads,
-                            int n_kv, int f32_cuda_cores, float *out);
+                            int n_kv, float *out);
 /* Timing helper: the tensor-core GEMM alone on device-resident pseudo-random operands (CUDA events, best of reps,
  * milliseconds per launch).  mode 0 / 1 as `exact` above; mode 2 = dense ceiling of the same tiling and pipeline (no group
  * structure: all of K accumulated in one TMEM buffer, one drain per tile) -- the measured int8 peak the group-scaled

@@ -106,7 +106,7 @@ struct q3_handle {
     unsigned long long bar_base = 0, xbar_base = 0;
     int *d_status = nullptr;  // device abort flag raised by a timed-out wait inside the kernel
     unsigned long long *part_buf[2] = {nullptr, nullptr};            // TP landing zones [tp][dim] (inside xchg: peers write them)
-    unsigned long long *zq = nullptr, *za = nullptr, *zh = nullptr, *zp = nullptr, *zr[2] = {nullptr, nullptr}; // local (payload, epoch) zones
+    unsigned long long *zq = nullptr, *za = nullptr, *zh = nullptr, *zr[2] = {nullptr, nullptr}; // local (payload, epoch) zones
     int logits_root = -1;     // TP: >= 0 = only this rank receives the other ranks' vocabulary shards (q3_tp_set_logits_root)
     bool poisoned = false;    // a wait timed out under tensor parallelism: the ranks' epoch / barrier sequences may have diverged
     unsigned long long *d_best = nullptr, *d_bar = nullptr;
@@ -128,7 +128,6 @@ struct q3_handle {
     // batched prefill (tcgen05 GEMM) state
     bool pf_ok = false;
     std::string pf_why;
-    int pf_attn_kind = 0;     // 0: tensor cores, FP16 hi/lo split (default); 1: Q3_PF_ATTN_F32=1, f32 on the CUDA cores; 2: Q3_PF_ATTN_TF32=1, 3xTF32
     __half *pf_kvh = nullptr; // [4][pf_kvh_rows][KV_l] halves: this layer's K / V rows split into hi / lo (k_pf_split_kv)
     size_t pf_kvh_rows = 0;
     int pf_cap = 0;          // token capacity of the buffers below (multiple of 128)
@@ -616,7 +615,6 @@ static int build_mega(q3_handle *h, const float *rms_att_all, const float *rms_f
             {&h->zq, (size_t)h->AH_l + 2 * (size_t)h->KV_l},
             {&h->za, (size_t)h->AH_l / 4 + (size_t)h->AH_l / gs},
             {&h->zh, (size_t)h->H_l},
-            {&h->zp, (size_t)h->n_heads_l * MEGA_MAX_SPLITS * ATTN_PART_STRIDE},
             {&h->zr[0], (size_t)dim},
             {&h->zr[1], (size_t)dim}};
         for (auto &z : zones) {
@@ -632,7 +630,7 @@ static int build_mega(q3_handle *h, const float *rms_att_all, const float *rms_f
     CK(cudaMemset(h->d_status, 0, 64));
     int *d_status = h->d_status;
     a.x = h->x;
-    a.zq = h->zq; a.za = h->za; a.zh = h->zh; a.zp = h->zp; a.zr[0] = h->zr[0]; a.zr[1] = h->zr[1];
+    a.zq = h->zq; a.za = h->za; a.zh = h->zh; a.zr[0] = h->zr[0]; a.zr[1] = h->zr[1];
     a.attn_part = h->attn_part; a.att_cnt = h->att_cnt;
     a.dbg = getenv("Q3_MEGA_DBG") ? atoi(getenv("Q3_MEGA_DBG")) : 0;
     a.bar = h->d_bar; a.status = d_status; a.tokpos = h->d_tokpos; a.history = h->d_history;
@@ -859,19 +857,10 @@ static int prefill_init(q3_handle *h) {
         return 0;
     }
     if (!get_encode_fn()) { h->pf_why = "cuTensorMapEncodeTiled unavailable"; return 0; }
-    h->pf_attn_kind = getenv("Q3_PF_ATTN_F32") ? 1 : getenv("Q3_PF_ATTN_TF32") ? 2 : 0;
     CK(cudaFuncSetAttribute(k_pf_attention_h<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
     CK(cudaFuncSetAttribute(k_pf_attention_h<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
     CK(cudaFuncSetAttribute(k_pf_attention_h<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
     CK(cudaFuncSetAttribute(k_pf_attention_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFA_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFA_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFA_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFA_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_tc<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFT_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_tc<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFT_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_tc<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFT_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_tc<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFT_SMEM));
     int rc;
     for (auto &W : h->layers) {
         if ((rc = prefill_prepare_tensor(h, W.qkv))) return rc;
@@ -966,7 +955,7 @@ static int prefill_run(q3_handle *h, const int *tokens_host, int T, int pos0) {
     const int gs = c.group_size, dim = c.dim, AH = h->AH_l, KV = h->KV_l, H = h->H_l;
     int rc;
     if ((rc = prefill_reserve(h, T))) return rc;
-    if (h->pf_attn_kind == 0 && (size_t)pos0 + T > h->pf_kvh_rows) { // hi / lo copy of one layer's K / V rows (grow-only)
+    if ((size_t)pos0 + T > h->pf_kvh_rows) { // hi / lo copy of one layer's K / V rows (grow-only)
         if (h->pf_kvh) cudaFree(h->pf_kvh);
         h->pf_kvh = nullptr;
         h->pf_kvh_rows = 0;
@@ -1004,35 +993,16 @@ static int prefill_run(q3_handle *h, const int *tokens_host, int T, int pos0) {
         if ((rc = launch_gemm_q8<PF_EPI_QKV>(gs, mx_dim, W.qkv.map, g, s))) return rc;
         dim3 rg((h->n_heads_l + h->n_kv_l + 3) / 4, T);
         k_pf_qknorm_rope<<<rg, 128, 0, s>>>(h->pf_q, kc_l, W.q_ln, W.k_ln, h->rope, pos0, h->n_heads_l, h->n_kv_l, AH, KV);
-        if (h->pf_attn_kind == 0) { // tensor cores, FP16 hi / lo split: K / V rows 0 .. pos0+T-1 of this layer split once, then streamed
-            const size_t rows = (size_t)pos0 + T, plane = h->pf_kvh_rows * KV;
-            k_pf_split_kv<<<h->num_sms * 4, 256, 0, s>>>(kc_l, vc_l, h->pf_kvh, rows * KV / 4, plane);
-            const int bq = PFH_R / h->kv_mul;
-            dim3 ag(h->n_kv_l, (T + bq - 1) / bq);
-            switch (h->kv_mul) {
-            case 1: k_pf_attention_h<1><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-            case 2: k_pf_attention_h<2><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-            case 4: k_pf_attention_h<4><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-            case 8: k_pf_attention_h<8><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-            }
-        } else if (h->pf_attn_kind == 1) { // f32 on the CUDA cores (kept for comparison: Q3_PF_ATTN_F32=1)
-            const int bq = PFA_R / h->kv_mul;
-            dim3 ag(h->n_kv_l, (T + bq - 1) / bq);
-            switch (h->kv_mul) {
-            case 1: k_pf_attention<1><<<ag, 256, PFA_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 2: k_pf_attention<2><<<ag, 256, PFA_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 4: k_pf_attention<4><<<ag, 256, PFA_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 8: k_pf_attention<8><<<ag, 256, PFA_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            }
-        } else { // tensor cores, 3xTF32 (the first tensor-core version, kept for comparison: Q3_PF_ATTN_TF32=1)
-            const int bq = PFT_R / h->kv_mul;
-            dim3 ag(h->n_kv_l, (T + bq - 1) / bq);
-            switch (h->kv_mul) {
-            case 1: k_pf_attention_tc<1><<<ag, 128, PFT_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 2: k_pf_attention_tc<2><<<ag, 128, PFT_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 4: k_pf_attention_tc<4><<<ag, 128, PFT_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            case 8: k_pf_attention_tc<8><<<ag, 128, PFT_SMEM, s>>>(h->pf_q, kc_l, vc_l, h->pf_att, T, pos0, AH, KV); break;
-            }
+        // attention on the tensor cores, FP16 hi / lo split: K / V rows 0 .. pos0+T-1 of this layer split once, then streamed
+        const size_t rows = (size_t)pos0 + T, plane = h->pf_kvh_rows * KV;
+        k_pf_split_kv<<<h->num_sms * 4, 256, 0, s>>>(kc_l, vc_l, h->pf_kvh, rows * KV / 4, plane);
+        const int bq = PFH_R / h->kv_mul;
+        dim3 ag(h->n_kv_l, (T + bq - 1) / bq);
+        switch (h->kv_mul) {
+        case 1: k_pf_attention_h<1><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
+        case 2: k_pf_attention_h<2><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
+        case 4: k_pf_attention_h<4><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
+        case 8: k_pf_attention_h<8><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
         }
         GS_DISPATCH(gs, (k_pf_quantize<GS><<<T, 256, 0, s>>>(h->pf_att, h->pf_xq, h->pf_xsT, AH, Tpad)));
         PrefillGemmArgs o{};
@@ -1171,7 +1141,7 @@ static int create_impl(const char *path, int ctx_len, int device, int tp_rank, i
     {   // exchange buffer (see q3_handle::xchg); logits live inside it
         auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
         size_t o = 0;
-        h->off_part[0] = o; o = al(o + (size_t)tp_size * dim * 8); // f32, or (value, epoch) words with MEGA_LL
+        h->off_part[0] = o; o = al(o + (size_t)tp_size * dim * 8); // (value, epoch) words
         h->off_part[1] = o; o = al(o + (size_t)tp_size * dim * 8);
         h->off_best = o; o = al(o + (size_t)tp_size * h->num_sms * 8);
         h->off_flags = o; o = al(o + 64 * 4);
@@ -1211,7 +1181,7 @@ static int create_impl(const char *path, int ctx_len, int device, int tp_rank, i
     TRY(build_graphs(h));
     h->graph_launches_per_step = h->launches_per_step;
     TRY(build_mega(h, ck.rms_att, ck.rms_ffn, ck.q_ln, ck.k_ln));
-    if (h->mega_ok && !getenv("Q3_NO_MEGA")) {
+    if (h->mega_ok) {
         h->decode_path = 1;
         h->launches_per_step = 1;
     }
@@ -1645,7 +1615,7 @@ extern "C" int q3_prefill(q3_handle *h, const int *tokens, int n, int pos0, floa
     for (int i = 0; i < n; i++)
         if (tokens[i] < 0 || tokens[i] >= h->cfg.vocab_size) return fail(Q3_EINVAL, "index out of bounds: token %d", tokens[i]);
     CK(cudaSetDevice(h->device));
-    if (!h->pf_ok || h->exact || getenv("Q3_NO_PREFILL_GEMM")) {
+    if (!h->pf_ok || h->exact) {
         // sequential decode steps: same results as n forwards by construction (exact mode, TP, odd shapes)
         for (int i = 0; i < n; i++) {
             int rc = q3_forward(h, tokens[i], pos0 + i, i == n - 1 ? last_logits_host : nullptr);
@@ -1906,9 +1876,9 @@ extern "C" int q3_op_sample(int device, const float *logits, int n, float temper
 
 // Causal prefill attention alone (layers.rs:374-419 for T query tokens at positions pos0 .. pos0+T-1 over a cache of pos0+T rows):
 // q [T][n_heads*128] (already normalised + rotated), k / v [pos0+T][n_kv*128], out [T][n_heads*128].
-// f32_cuda_cores != 0: the CUDA-core f32 kernel; 0: the tensor-core (3xTF32) kernel q3_prefill runs.
+// The kernel is the one q3_prefill runs (k_pf_attention_h over a hi / lo split of K / V).
 extern "C" int q3_op_prefill_attention(int device, const float *q, const float *k, const float *v, int T, int pos0, int n_heads, int n_kv,
-                                       int f32_cuda_cores, float *out) {
+                                       float *out) {
     CK(cudaSetDevice(device));
     if (!q || !k || !v || !out || T <= 0 || pos0 < 0 || n_kv <= 0 || n_heads % n_kv) return fail(Q3_EINVAL, "bad attention arguments");
     const int kv_mul = n_heads / n_kv;
@@ -1922,30 +1892,20 @@ extern "C" int q3_op_prefill_attention(int device, const float *q, const float *
     CK(cudaMemcpy(dq.p, q, (size_t)T * AH * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dk.p, k, (size_t)nk * KV * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dv.p, v, (size_t)nk * KV * 4, cudaMemcpyHostToDevice));
-#define PFA_CASE(KM)                                                                                                                        \
-    case KM:                                                                                                                                \
-        if (f32_cuda_cores == 1) {                                                                                                          \
-            CK(cudaFuncSetAttribute(k_pf_attention<KM>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFA_SMEM));                            \
-            k_pf_attention<KM><<<dim3(n_kv, (T + PFA_R / KM - 1) / (PFA_R / KM)), 256, PFA_SMEM>>>(dq.as<float>(), dk.as<float>(), dv.as<float>(), \
-                                                                                                 dout.as<float>(), T, pos0, AH, KV);         \
-        } else if (f32_cuda_cores == 0) {                                                                                                   \
-            CK(cudaFuncSetAttribute(k_pf_attention_h<KM>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));                          \
-            k_pf_split_kv<<<296, 256>>>(dk.as<float>(), dv.as<float>(), dkvh.as<__half>(), (size_t)nk * KV / 4, (size_t)nk * KV);            \
-            k_pf_attention_h<KM><<<dim3(n_kv, (T + PFH_R / KM - 1) / (PFH_R / KM)), 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(),      \
-                                                                                                   (size_t)nk * KV, dout.as<float>(), T, pos0, AH, KV); \
-        } else {                                                                                                                            \
-            CK(cudaFuncSetAttribute(k_pf_attention_tc<KM>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFT_SMEM));                         \
-            k_pf_attention_tc<KM><<<dim3(n_kv, (T + PFT_R / KM - 1) / (PFT_R / KM)), 128, PFT_SMEM>>>(dq.as<float>(), dk.as<float>(), dv.as<float>(), \
-                                                                                                    dout.as<float>(), T, pos0, AH, KV);      \
-        }                                                                                                                                   \
-        break;
+    CK(cudaFuncSetAttribute(k_pf_attention_h<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
+    CK(cudaFuncSetAttribute(k_pf_attention_h<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
+    CK(cudaFuncSetAttribute(k_pf_attention_h<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
+    CK(cudaFuncSetAttribute(k_pf_attention_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
+    const size_t plane = (size_t)nk * KV;
+    k_pf_split_kv<<<296, 256>>>(dk.as<float>(), dv.as<float>(), dkvh.as<__half>(), plane / 4, plane);
+    const int bq = PFH_R / kv_mul;
+    dim3 ag(n_kv, (T + bq - 1) / bq);
     switch (kv_mul) {
-        PFA_CASE(1)
-        PFA_CASE(2)
-        PFA_CASE(4)
-        PFA_CASE(8)
+    case 1: k_pf_attention_h<1><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
+    case 2: k_pf_attention_h<2><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
+    case 4: k_pf_attention_h<4><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
+    case 8: k_pf_attention_h<8><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
     }
-#undef PFA_CASE
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy(out, dout.p, (size_t)T * AH * 4, cudaMemcpyDeviceToHost));

@@ -49,11 +49,7 @@ constexpr int MEGA_CTHREADS = MEGA_NCW * 32;        // 512 consumer threads
 // + one producer warp per consumer group.  (A producer warpgroup that hands its registers to the consumers with
 // setmaxnreg was tried: ptxas cannot allocate this kernel's consumer path in 112-120 registers without spilling and
 // refuses -- see DESIGN.md.)
-#ifndef MEGA_HELPER
-#define MEGA_HELPER 0
-#endif
-constexpr int MEGA_NHELP = MEGA_HELPER ? 2 : 0;       // helper warps (see MEGA_HELPER below)
-constexpr int MEGA_THREADS = MEGA_CTHREADS + 32 * MEGA_GROUPS + 32 * MEGA_NHELP;
+constexpr int MEGA_THREADS = MEGA_CTHREADS + 32 * MEGA_GROUPS;
 #ifndef MEGA_NSTAGE_
 #define MEGA_NSTAGE_ 4
 #endif
@@ -63,49 +59,6 @@ constexpr int MEGA_SCRATCH = 40960;                 // xq/xs or attention buffer
 constexpr int MEGA_MAX_TP = 8;
 constexpr int MEGA_MAX_SPLITS = ATTN_MAX_SPLITS;
 constexpr int MEGA_EDGES = 6;                       // epochs per layer: one per step kind (0 qkv .. 4 down), one spare; the head step uses the next layer's 0
-
-// tuning switches (compile-time; scripts/ab_variants.py builds and times the alternatives on one box)
-#ifndef MEGA_PREFETCH_W
-#define MEGA_PREFETCH_W 1   // L2-prefetch the next norm / QK-norm / RoPE weights at the end of the preceding step
-#endif
-#ifndef MEGA_ATTN_NP
-#define MEGA_ATTN_NP 2      // positions per warp iteration in the attention loop
-#endif
-#ifndef MEGA_PSLEEP
-#define MEGA_PSLEEP 0       // ns the producers sleep per iteration while waiting for their turn on a slot
-#endif
-#ifndef MEGA_X_ONCE
-#define MEGA_X_ONCE 0       // load the activation registers once per phase when n_kt == 1 (measured: -9 %, register pressure)
-#endif
-#ifndef MEGA_POLL_SLEEP
-#define MEGA_POLL_SLEEP 0   // ns between two polls of a word that has not arrived yet (measured: 0 best, 64: -1.4 %, 200: -1.9 %)
-#endif
-#ifndef MEGA_LLPART
-#define MEGA_LLPART 0       // 1: attention split partials as (value, epoch) words, head h merged by split h % nsplit (measured: +7.8 % us/token -- rejected)
-#endif
-#ifndef MEGA_LAZY_SYNC
-#define MEGA_LAZY_SYNC 0    // 1: no CTA-wide sync at the end of the o_proj / gate-up / down steps (the next prologue syncs before it rewrites the
-                            // activation; down_proj's activation lives in a second buffer so that gate/up stragglers may still read the first)
-#endif
-#ifndef MEGA_ATTN_V2
-#define MEGA_ATTN_V2 1      // 1: position loop with lane = cached position (skewed dot products, one softmax update per 32 positions);
-                            // 0: the round-1 loop (lane = 4 dims, online softmax per position in every lane)
-#endif
-#ifndef MEGA_HELPER
-#define MEGA_HELPER 0       // 1: two helper warps poll + quantise the SwiGLU outputs (the down_proj activation, 96 KB of flagged words per CTA) in the
-                            // background WHILE the consumers are still streaming gate/up rows; the down prologue then only waits for them
-#endif
-#ifndef MEGA_INLINE_PRO
-#define MEGA_INLINE_PRO 0   // 1: the three prologues inlined into the step loop (each has a single call site)
-#endif
-#if MEGA_INLINE_PRO
-#define MEGA_PRO_INLINE __forceinline__
-#else
-#define MEGA_PRO_INLINE __noinline__
-#endif
-#ifndef MEGA_EARLY_W
-#define MEGA_EARLY_W 1      // issue the norm-weight loads BEFORE polling for the activation (one loaded round trip instead of two)
-#endif
 
 enum { PH_QKV = 0, PH_O = 1, PH_GU = 2, PH_DN = 3, PH_HEAD = 4 };
 
@@ -139,8 +92,7 @@ struct MegaArgs {
     unsigned long long *zh;          // [H_l]                  SwiGLU outputs
     unsigned long long *zr[2];       // [dim]                  o_proj / down rows, reduced over the TP ranks (this rank's copy)
     unsigned long long *part[2][MEGA_MAX_TP]; // TP only: [o|down][rank] -> that rank's landing zone [tp][dim] (peer memory)
-    float *attn_part;                // [n_heads_l][MEGA_MAX_SPLITS][ATTN_PART_STRIDE] split partials (nsplit > 1, MEGA_LLPART == 0)
-    unsigned long long *zp;          // the same as (value, epoch) words (MEGA_LLPART): [n_heads_l][MEGA_MAX_SPLITS][ATTN_PART_STRIDE]
+    float *attn_part;                // [n_heads_l][MEGA_MAX_SPLITS][ATTN_PART_STRIDE] split partials (nsplit > 1)
     unsigned *att_cnt;               // [n_layers][n_kv_l] arrivals of the splits of a kv head (returns to 0 within the launch)
     float *logits[MEGA_MAX_TP];      // full-vocab logits buffer of every rank
     unsigned long long *best[MEGA_MAX_TP]; // [tp][grid] argmax candidates of every rank
@@ -265,9 +217,8 @@ __device__ __forceinline__ unsigned long long ll_load1(const unsigned long long 
     return x;
 }
 __device__ __forceinline__ bool ll_ok(unsigned long long w, unsigned epoch) { return (unsigned)(w >> 32) == epoch; }
-// called after a failed poll: back off, and give up (abort flag, status `code`) after ~1-2 s -- a protocol bug must never hang the GPU
+// called after a failed poll: give up (abort flag, status `code`) after ~1-2 s -- a protocol bug must never hang the GPU
 __device__ __noinline__ bool ll_give_up(const MegaArgs &a, unsigned &spins, int code) {
-    if (MEGA_POLL_SLEEP) __nanosleep(MEGA_POLL_SLEEP);
     if ((++spins & 255u) == 0) {
         if (*(volatile int *)a.status) return true;
         if (spins > (1u << 20)) {
@@ -450,8 +401,8 @@ constexpr int MEGA_MAXV = (MEGA_MAX_KT + 4 * MEGA_CTHREADS - 1) / (4 * MEGA_CTHR
 // src: 0 = embedding row of tokpos[0], 1 = a.x (teacher-forced entry), 2 = sx (this CTA's copy of the residual stream in
 // shared memory; a thread always owns the same elements).  zone/epoch: pending GEMV rows to add (or null).
 template <int GS>
-__device__ MEGA_PRO_INLINE void prologue_norm(const MegaArgs &a, const float *w, int src, const unsigned long long *zone, unsigned epoch,
-                                              uint8_t *sxq, float *sxs, float *sred, float *sx, int KT, int G, Prof &pr) {
+__device__ __noinline__ void prologue_norm(const MegaArgs &a, const float *w, int src, const unsigned long long *zone, unsigned epoch,
+                                           uint8_t *sxq, float *sxs, float *sred, float *sx, int KT, int G, Prof &pr) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int n4 = a.dim >> 2;
     constexpr int MAXV = MEGA_MAXV;
@@ -459,12 +410,10 @@ __device__ MEGA_PRO_INLINE void prologue_norm(const MegaArgs &a, const float *w,
     float ss = 0.0f;
     // the norm weights do not depend on the activation: with the weight stream saturating the memory system a global
     // round trip costs ~1.3 us, so their loads are issued before the poll below instead of after it
-    if (MEGA_EARLY_W) {
 #pragma unroll
-        for (int k = 0; k < MAXV; k++) {
-            const int i4 = tid + k * MEGA_CTHREADS;
-            wv[k] = (i4 < n4) ? __ldg(reinterpret_cast<const float4 *>(w) + i4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
+    for (int k = 0; k < MAXV; k++) {
+        const int i4 = tid + k * MEGA_CTHREADS;
+        wv[k] = (i4 < n4) ? __ldg(reinterpret_cast<const float4 *>(w) + i4) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
 #pragma unroll
     for (int k = 0; k < MAXV; k++) {
@@ -521,13 +470,6 @@ __device__ MEGA_PRO_INLINE void prologue_norm(const MegaArgs &a, const float *w,
         }
     }
     prof_mark(pr, 32); // x (+ pending rows) arrived
-    if (!MEGA_EARLY_W) {
-#pragma unroll
-        for (int k = 0; k < MAXV; k++) {
-            const int i4 = tid + k * MEGA_CTHREADS;
-            wv[k] = (i4 < n4) ? __ldg(reinterpret_cast<const float4 *>(w) + i4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-    }
     ss = warp_sum(ss);
     if (lane == 0) sred[warp] = ss;
     csync(); // also: every warp has left the previous GEMV, sxq may be rewritten
@@ -565,7 +507,7 @@ __device__ MEGA_PRO_INLINE void prologue_norm(const MegaArgs &a, const float *w,
 // o_proj input: the attention output arrives already normalised and quantised (attention_item), packed 4 int8 per word in the
 // chunk order of this phase's shared-memory activation, followed by the group scales -- the prologue is a polled copy.
 template <int GS>
-__device__ MEGA_PRO_INLINE void prologue_attn_poll(const MegaArgs &a, unsigned epoch, uint8_t *sxq, float *sxs) {
+__device__ __noinline__ void prologue_attn_poll(const MegaArgs &a, unsigned epoch, uint8_t *sxq, float *sxs) {
     const int tid = threadIdx.x;
     const int nq = a.AH_l >> 2, ng = a.AH_l / GS; // nq is a multiple of 32
     unsigned spins = 0;
@@ -611,7 +553,7 @@ __device__ __forceinline__ void quant_ll_one(const MegaArgs &a, const unsigned l
     }
 }
 template <int GS>
-__device__ MEGA_PRO_INLINE void prologue_quant_ll(const MegaArgs &a, const unsigned long long *z, unsigned epoch, int n, uint8_t *sxq, float *sxs, int KT, int G) {
+__device__ __noinline__ void prologue_quant_ll(const MegaArgs &a, const unsigned long long *z, unsigned epoch, int n, uint8_t *sxq, float *sxs, int KT, int G) {
     const int tid = threadIdx.x, lane = tid & 31;
     const int n4 = n >> 2;
     unsigned long long wa[4] = {0, 0, 0, 0}, wb[4] = {0, 0, 0, 0};
@@ -721,11 +663,6 @@ __device__ __forceinline__ void publish_head(const MegaArgs &a, int head, int la
 struct RingPos {
     unsigned it, fullp;
 };
-// warps that take part in the position loop: all 16 when their partials fit the scratch area, else one group
-template <int KVMUL>
-struct AttnWarps {
-    static constexpr int N = MEGA_ATTN_V2 ? MEGA_NCW : ((KVMUL * MEGA_NCW * 512 + 8192 <= MEGA_SCRATCH) ? MEGA_NCW : MEGA_GW);
-};
 __device__ __forceinline__ void gsync(int grp) { // the 8 warps of one consumer group
     asm volatile("bar.sync %0, %1;" ::"r"(2 + grp), "n"(MEGA_GW * 32) : "memory");
 }
@@ -735,16 +672,11 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
                                                uint8_t *scratch, unsigned ep_q, unsigned ep_a, Prof &pr, RingPos &rp, uint32_t ring_s, int slot_bytes,
                                                uint64_t *myfull, uint64_t *empty) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    constexpr int NATT = AttnWarps<KVMUL>::N; // warps in the position loop
-    float4 *sq = reinterpret_cast<float4 *>(scratch);                 // [KVMUL][32]
-    float4 *sk = sq + KVMUL * 32;                                     // [32]
-    float4 *sv = sk + 32;                                             // [32]
-    float *sm_m = reinterpret_cast<float *>(sv + 32);                 // [NATT][KVMUL]
-    float *sm_l = sm_m + NATT * KVMUL;                                // [NATT][KVMUL]
-    float4 *sm_acc = reinterpret_cast<float4 *>(sm_l + NATT * KVMUL); // [NATT][KVMUL][32]
-    static_assert(MEGA_ATTN_V2 ? ((KVMUL * 32 + 64) * 16 + (2 * MEGA_GW * 32 + 16 + 8 * HEAD_DIM) * 4 <= MEGA_SCRATCH)
-                               : ((KVMUL * 32 + 64) * 16 + 2 * NATT * KVMUL * 4 + NATT * KVMUL * 512 <= MEGA_SCRATCH),
-                  "attention scratch");
+    float4 *sq = reinterpret_cast<float4 *>(scratch);  // [KVMUL][32]
+    float4 *sk = sq + KVMUL * 32;                      // [32]
+    float4 *sv = sk + 32;                              // [32]
+    float *sbase = reinterpret_cast<float *>(sv + 32); // behind q / k / v: scores, then the merge of the two groups
+    static_assert((KVMUL * 32 + 64) * 16 + (2 * MEGA_GW * 32 + 16 + 8 * HEAD_DIM) * 4 <= MEGA_SCRATCH, "attention scratch");
     static_assert(KVMUL + 2 <= MEGA_NCW, "one warp per gathered row");
     const int n = pos + 1;
     const int per = (n + nsplit - 1) / nsplit;
@@ -782,7 +714,6 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
     const float scale = __fdiv_rn(1.0f, sqrtf((float)HEAD_DIM));
     float4 A = make_float4(0.f, 0.f, 0.f, 0.f);
     float M = -INFINITY, L = 0.0f;
-#if MEGA_ATTN_V2
     {
         // The cache rows t0 .. t1 of this kv head arrive through the weight ring: stages of MEGA_KV_ROWS = 32 positions (K tile, then
         // V tile, 16 KB each, [position][128] f32), issued by the producers behind the QKV weights; stages alternate between the two
@@ -792,8 +723,8 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
         //            512 B apart, so the same chunk index in every lane would be a 32-way bank conflict; skewed, a quarter warp
         //            touches 8 distinct bank groups, and the matching q chunks are consecutive addresses); the PARTS partial sums
         //            of a head are exchanged through shared memory;
-        //   softmax: ONE update per 32 positions -- a warp maximum, one exp per lane, a warp sum (the round-1 loop redid the whole
-        //            online update, 2 exps, in all 32 lanes for every single position);
+        //   softmax: ONE update per 32 positions -- a warp maximum, one exp per lane, a warp sum (a loop with lane = dims redoes
+        //            the whole online update, 2 exps, in all 32 lanes for every single position);
         //   P V    : lane = dims; the weight of position j comes from lane j by shuffle.
         // Row `pos` itself is not in the cache yet when its tile is fetched: that lane / iteration reads sk / sv instead.
         constexpr int PARTS = MEGA_GW / KVMUL, DPP = HEAD_DIM / PARTS, CPP = DPP / 4; // dims / 16-byte chunks per part
@@ -801,7 +732,6 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
         static_assert(MEGA_GW % KVMUL == 0 && (CPP & (CPP - 1)) == 0, "head / part split");
         const int grp = warp / MEGA_GW, wl = warp % MEGA_GW;
         const int head = wl % KVMUL, part = wl / KVMUL;
-        float *sbase = reinterpret_cast<float *>(sv + 32);                              // behind q / k / v
         float *sS = sbase + grp * (MEGA_GW * 32);                                       // [grp][part][head][32] partial scores
         const uint32_t sq_s = smem_u32(sq) + head * 512, sk_s = smem_u32(sk), sv_s = smem_u32(sv);
         float m = -INFINITY, l = 0.0f;
@@ -953,190 +883,10 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
             L = xs_l[warp];
         }
     }
-#else
-    float4 qv[KVMUL];
-    float m[KVMUL], l[KVMUL];
-    float4 acc[KVMUL];
-#pragma unroll
-    for (int h = 0; h < KVMUL; h++) {
-        qv[h] = sq[h * 32 + lane];
-        m[h] = -INFINITY;
-        l[h] = 0.0f;
-        acc[h] = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    // The cache rows t0 .. t1 of this kv head arrive through the weight ring: stages of MEGA_KV_ROWS positions (K tile, then V
-    // tile, 16 KB each, [position][128] f32), issued by the producers behind the QKV weights -- normally they are already in
-    // shared memory here.  Stages alternate between the consumer groups like weight stages (all of them to group 0 when only
-    // one group's partials fit the scratch area); inside a stage warp w of the group owns positions 4w .. 4w+3.
-    // Row `pos` itself is not in the cache yet when its tile is fetched: it is taken from sk / sv.
-    constexpr int NP = 2; // positions per pass
-    const int grp = warp / MEGA_GW, wl = warp % MEGA_GW;
-    const int nst = (t1 - t0 + MEGA_KV_ROWS - 1) / MEGA_KV_ROWS;
-    for (int st = 0; st < nst; st++) {
-        const int owner = NATT == MEGA_NCW ? (st & 1) : 0;
-        if (owner == grp) {
-            const int slot = rp.it % MEGA_NSTAGE;
-            mbar_wait(&myfull[slot], (rp.fullp >> slot) & 1, a.status);
-            rp.fullp ^= 1u << slot;
-            const uint32_t kb = ring_s + slot * slot_bytes + lane * 16, vb = kb + MEGA_KV_ROWS * HEAD_DIM * 4;
-#pragma unroll 1
-            for (int half = 0; half < 4 / NP; half++) {
-                const int r0 = wl * 4 + half * NP; // row inside the stage
-                const int t = t0 + st * MEGA_KV_ROWS + r0;
-                float4 kv[NP], vv[NP];
-#pragma unroll
-                for (int j = 0; j < NP; j++) {
-                    const int tj = t + j;
-                    kv[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    vv[j] = kv[j];
-                    if (tj < t1) {
-                        if (tj == pos) {
-                            kv[j] = sk[lane];
-                            vv[j] = sv[lane];
-                        } else {
-                            const int4 ki = lds128(kb + (r0 + j) * HEAD_DIM * 4), vi = lds128(vb + (r0 + j) * HEAD_DIM * 4);
-                            kv[j] = make_float4(__int_as_float(ki.x), __int_as_float(ki.y), __int_as_float(ki.z), __int_as_float(ki.w));
-                            vv[j] = make_float4(__int_as_float(vi.x), __int_as_float(vi.y), __int_as_float(vi.z), __int_as_float(vi.w));
-                        }
-                    }
-                }
-                if (t < t1) { // warp-uniform
-                    float sc[NP][KVMUL];
-#pragma unroll
-                    for (int j = 0; j < NP; j++)
-#pragma unroll
-                        for (int h = 0; h < KVMUL; h++) sc[j][h] = qv[h].x * kv[j].x + qv[h].y * kv[j].y + qv[h].z * kv[j].z + qv[h].w * kv[j].w;
-#pragma unroll
-                    for (int j = 0; j < NP; j++)
-#pragma unroll
-                        for (int h = 0; h < KVMUL; h++) sc[j][h] = (t + j < t1) ? __fmul_rn(warp_sum(sc[j][h]), scale) : -INFINITY;
-#pragma unroll
-                    for (int h = 0; h < KVMUL; h++) {
-                        float mn = m[h];
-#pragma unroll
-                        for (int j = 0; j < NP; j++) mn = fmaxf(mn, sc[j][h]);
-                        const float corr = expf(m[h] - mn);
-                        l[h] *= corr;
-                        acc[h].x *= corr;
-                        acc[h].y *= corr;
-                        acc[h].z *= corr;
-                        acc[h].w *= corr;
-#pragma unroll
-                        for (int j = 0; j < NP; j++) {
-                            const float pj = expf(sc[j][h] - mn); // exp(-inf) = 0 for the positions past the end
-                            l[h] += pj;
-                            acc[h].x += pj * vv[j].x;
-                            acc[h].y += pj * vv[j].y;
-                            acc[h].z += pj * vv[j].z;
-                            acc[h].w += pj * vv[j].w;
-                        }
-                        m[h] = mn;
-                    }
-                }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty[slot]);
-        }
-        rp.it++;
-    }
-    prof_mark(pr, 36); // position loop done
-    if (warp < NATT) {
-#pragma unroll
-        for (int h = 0; h < KVMUL; h++) {
-            if (lane == 0) {
-                sm_m[warp * KVMUL + h] = m[h];
-                sm_l[warp * KVMUL + h] = l[h];
-            }
-            sm_acc[(warp * KVMUL + h) * 32 + lane] = acc[h];
-        }
-    }
-    csync();
-    // warp h < KVMUL merges the NATT warp partials of query head h (lane w owns partial w: one exp per lane)
-    if (warp < KVMUL) {
-        const int h = warp;
-        const float mw = lane < NATT ? sm_m[lane * KVMUL + h] : -INFINITY;
-        M = warp_max(mw);
-        const float cw = (mw == -INFINITY) ? 0.0f : expf(mw - M);
-        L = warp_sum(lane < NATT ? sm_l[lane * KVMUL + h] * cw : 0.0f);
-#pragma unroll 4
-        for (int w = 0; w < NATT; w++) {
-            const float c = __shfl_sync(0xffffffffu, cw, w);
-            const float4 aw = sm_acc[(w * KVMUL + h) * 32 + lane];
-            A.x += aw.x * c;
-            A.y += aw.y * c;
-            A.z += aw.z * c;
-            A.w += aw.w * c;
-        }
-    }
-#endif
     if (nsplit == 1) { // the only split of its kv head: A / L is the attention output
         if (warp < KVMUL) publish_head<GS>(a, kvh * KVMUL + warp, lane, A, L, ep_a);
         return;
     }
-#if MEGA_LLPART
-    // Several splits: every split publishes its partial (acc[128], m, l per query head) as (value, epoch) words; query head h of
-    // the group is merged by the split h % nsplit -- no fence, no counter: the merger polls the nsplit partials of its head.
-    if (warp < KVMUL) {
-        unsigned long long *dst = a.zp + ((size_t)(kvh * KVMUL + warp) * MEGA_MAX_SPLITS + split) * ATTN_PART_STRIDE;
-        ll_store(dst + lane * 4 + 0, A.x, ep_a);
-        ll_store(dst + lane * 4 + 1, A.y, ep_a);
-        ll_store(dst + lane * 4 + 2, A.z, ep_a);
-        ll_store(dst + lane * 4 + 3, A.w, ep_a);
-        if (lane == 0) {
-            ll_store(dst + HEAD_DIM, M, ep_a);
-            ll_store(dst + HEAD_DIM + 1, L, ep_a);
-        }
-    }
-    prof_mark(pr, 37); // split partial published
-    if (warp < KVMUL && (warp % nsplit) == split) {
-        const int head = kvh * KVMUL + warp;
-        const unsigned long long *pb = a.zp + (size_t)head * MEGA_MAX_SPLITS * ATTN_PART_STRIDE;
-        unsigned spins = 0;
-        // lane s: statistics of split s (one round trip for all splits once they are there)
-        float ms = -INFINITY, ls = 0.0f;
-        if (lane < nsplit) {
-            unsigned long long x, y;
-            while (true) {
-                ll_load2(pb + (size_t)lane * ATTN_PART_STRIDE + HEAD_DIM, x, y);
-                if ((ll_ok(x, ep_a) && ll_ok(y, ep_a)) || ll_give_up(a, spins, 12)) break;
-            }
-            ms = __uint_as_float((unsigned)x);
-            ls = __uint_as_float((unsigned)y);
-        }
-        const float Mx = warp_max(ms);
-        const float cs = lane < nsplit ? expf(ms - Mx) : 0.0f;
-        const float Ls = warp_sum(ls * cs);
-        float4 As = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll 1
-        for (int s0 = 0; s0 < nsplit; s0 += 4) { // accumulators four splits at a time, all eight loads in flight together
-            unsigned long long w[4][4];
-            while (true) {
-                bool ok = true;
-#pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    if (s0 + j < nsplit) {
-                        const unsigned long long *src = pb + (size_t)(s0 + j) * ATTN_PART_STRIDE + lane * 4;
-                        ll_load2(src, w[j][0], w[j][1]);
-                        ll_load2(src + 2, w[j][2], w[j][3]);
-                        ok = ok && ll_ok(w[j][0], ep_a) && ll_ok(w[j][1], ep_a) && ll_ok(w[j][2], ep_a) && ll_ok(w[j][3], ep_a);
-                    }
-                }
-                if (ok || ll_give_up(a, spins, 12)) break;
-            }
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const float c = __shfl_sync(0xffffffffu, cs, (s0 + j) & 31);
-                if (s0 + j < nsplit) {
-                    As.x += __uint_as_float((unsigned)w[j][0]) * c;
-                    As.y += __uint_as_float((unsigned)w[j][1]) * c;
-                    As.z += __uint_as_float((unsigned)w[j][2]) * c;
-                    As.w += __uint_as_float((unsigned)w[j][3]) * c;
-                }
-            }
-        }
-        publish_head<GS>(a, head, lane, As, Ls, ep_a);
-    }
-#else
     if (warp < KVMUL) {
         float *dst = a.attn_part + ((size_t)(kvh * KVMUL + warp) * MEGA_MAX_SPLITS + split) * ATTN_PART_STRIDE;
         reinterpret_cast<float4 *>(dst)[lane] = A;
@@ -1145,7 +895,7 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
             dst[HEAD_DIM + 1] = L;
         }
     }
-    unsigned *flag = reinterpret_cast<unsigned *>(sm_m); // the position-loop statistics have been consumed above
+    unsigned *flag = reinterpret_cast<unsigned *>(sbase); // group 1's hand-over, consumed above
     csync();
     if (tid == 0) {
         __threadfence();
@@ -1186,7 +936,6 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
         }
         publish_head<GS>(a, head, lane, As, Ls, ep_a);
     }
-#endif
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1284,10 +1033,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
     uint8_t *sxq = scratch;                                          // up to 16384 B
     float *sxs = reinterpret_cast<float *>(scratch + 16384);         // up to 512 groups
     float *sred = reinterpret_cast<float *>(scratch + 16384 + 2048); // 16 floats (+ argmax scratch at +32)
-    // down_proj's activation: its own buffer under MEGA_LAZY_SYNC (written while gate/up stragglers may still be reading sxq)
-    uint8_t *sxq_dn = (MEGA_LAZY_SYNC || MEGA_HELPER) ? scratch + 20480 : sxq;
-    float *sxs_dn = (MEGA_LAZY_SYNC || MEGA_HELPER) ? reinterpret_cast<float *>(scratch + 20480 + 16384) : sxs;
-    static_assert(20480 + 16384 + 2048 <= MEGA_SCRATCH, "second activation buffer");
     // full barriers are per (consumer group, slot): a waiter can only tell adjacent mbarrier phases
     // apart, and with ownership alternating between the groups a group would otherwise skip the
     // other group's use of a slot and mistake the phase before it for its own.
@@ -1328,76 +1073,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
 
     const int L0 = a.layer0, L1 = a.layer1;
 
-#if MEGA_HELPER
-    if (warp >= MEGA_NCW + MEGA_GROUPS) {
-        // =============================== HELPERS ===============================
-        // Per layer: wait until the consumers have entered the gate/up step (barrier 4: the down activation buffer of the previous layer
-        // is free), then quantise the SwiGLU outputs group by group as their flagged words arrive -- a half-warp per group of GS values
-        // (lane = one float4, exactly prologue_quant_ll's grouping, so the int8 / scales are the same bits) -- and report (barrier 5).
-        if (a.dbg & 4) return;
-        const int hw = warp - MEGA_NCW - MEGA_GROUPS;
-        constexpr int LPG = GS / 4;                       // lanes per group
-        constexpr int GPW = 32 / LPG;                     // groups a warp handles at once
-        const int ngroups = a.H_l / GS, nunits = (ngroups + GPW - 1) / GPW; // units of GPW groups
-        const int KT = a.g[PH_DN].KT, G = a.g[PH_DN].G;
-        for (int l = L0; l < L1; l++) {
-            asm volatile("bar.sync 4, %0;" ::"n"(MEGA_CTHREADS + 64) : "memory");
-            const unsigned ep = ll_epoch(a.ll_base, (unsigned)(MEGA_EDGES * (l - L0) + 3));
-            // units hw, hw + 2, ...; a unit that is not complete yet is skipped and revisited (pending bits), with a short sleep per
-            // fruitless round so that the spinning does not take issue slots from the consumers
-            unsigned pend[8];
-#pragma unroll
-            for (int w = 0; w < 8; w++) pend[w] = 0;
-            int left = 0;
-            for (int u = hw; u < nunits; u += 2) {
-                pend[(u >> 1) >> 5] |= 1u << ((u >> 1) & 31);
-                left++;
-            }
-            unsigned spins = 0;
-            bool dead = false;
-            while (left > 0 && !dead) {
-                int progressed = 0;
-                for (int u = hw; u < nunits; u += 2) {
-                    const int bit = u >> 1;
-                    if (!((pend[bit >> 5] >> (bit & 31)) & 1u)) continue;
-                    const int i4 = u * 32 + lane; // float4 index into the H_l vector
-                    const bool in = i4 * 4 < a.H_l;
-                    unsigned long long w0 = 0, w1 = 0, w2 = 0, w3 = 0;
-                    if (in) {
-                        ll_load2(a.zh + (size_t)i4 * 4, w0, w1);
-                        ll_load2(a.zh + (size_t)i4 * 4 + 2, w2, w3);
-                    }
-                    const bool ok = !in || (ll_ok(w0, ep) && ll_ok(w1, ep) && ll_ok(w2, ep) && ll_ok(w3, ep));
-                    if (!__all_sync(0xffffffffu, ok)) continue;
-                    float4 y = make_float4(__uint_as_float((unsigned)w0), __uint_as_float((unsigned)w1), __uint_as_float((unsigned)w2), __uint_as_float((unsigned)w3));
-                    uint32_t packed;
-                    float scale;
-                    quantize_group4<GS>(y, packed, scale);
-                    if (in) {
-                        xq_store<GS>(sxq_dn, i4, packed, KT, G);
-                        if ((i4 % (GS / 4)) == 0) sxs_dn[i4 / (GS / 4)] = scale;
-                    }
-                    pend[bit >> 5] &= ~(1u << (bit & 31));
-                    left--;
-                    progressed++;
-                }
-                if (!progressed) {
-                    __nanosleep(200);
-                    if ((++spins & 63u) == 0) {
-                        if (*(volatile int *)a.status) dead = true;
-                        else if (spins > (1u << 22)) {
-                            atomicExch(a.status, 8);
-                            dead = true;
-                        }
-                    }
-                }
-            }
-            __syncwarp();
-            asm volatile("bar.sync 5, %0;" ::"n"(MEGA_CTHREADS + 64) : "memory");
-        }
-        return;
-    }
-#endif
     if (warp >= MEGA_NCW) {
         // =============================== PRODUCERS ===============================
         // One producer thread per consumer group: the serial wait -> expect_tx -> bulk-copy loop of a single
@@ -1425,7 +1100,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
                 const unsigned use = it / MEGA_NSTAGE;
                 long long t0 = clock64();
                 while (issued[slot] != use) {
-                    if (MEGA_PSLEEP) __nanosleep(MEGA_PSLEEP);
                     if (clock64() - t0 > 4000000000LL) { atomicExch(a.status, 4); break; }
                 }
             }
@@ -1448,7 +1122,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
         auto kvpush = [&](int layer) {
             if (!has_item) return;
             for (int t = pt0, si = 0; t < pt1; t += MEGA_KV_ROWS, si++) {
-                const int owner = AttnWarps<KVMUL>::N == MEGA_NCW ? (si & 1) : 0;
+                const int owner = si & 1;
                 if (owner != pw) {
                     it++;
                     continue;
@@ -1458,7 +1132,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
                     const unsigned use = it / MEGA_NSTAGE;
                     long long tw = clock64();
                     while (issued[slot] != use) {
-                        if (MEGA_PSLEEP) __nanosleep(MEGA_PSLEEP);
                         if (clock64() - tw > 4000000000LL) { atomicExch(a.status, 4); break; }
                     }
                 }
@@ -1571,17 +1244,10 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
             prologue_attn_poll<GS>(a, ep_prev, sxq, sxs);
             ph = PH_O;
         } else {
-#if MEGA_HELPER
-            asm volatile("bar.sync 5, %0;" ::"n"(MEGA_CTHREADS + 64) : "memory"); // the helper warps have built the down activation
-#else
-            prologue_quant_ll<GS>(a, a.zh, ep_prev, a.H_l, sxq_dn, sxs_dn, a.g[PH_DN].KT, a.g[PH_DN].G); // quantize(hb), layers.rs:478
-#endif
+            prologue_quant_ll<GS>(a, a.zh, ep_prev, a.H_l, sxq, sxs, a.g[PH_DN].KT, a.g[PH_DN].G); // quantize(hb), layers.rs:478
             ph = PH_DN;
         }
         prof_mark(pr, 1 + 3 * kind);
-#if MEGA_HELPER
-        if (kind == 3 && !(a.dbg & 4)) asm volatile("bar.arrive 4, %0;" ::"n"(MEGA_CTHREADS + 64) : "memory"); // gate/up starts: helpers may build this layer's down activation
-#endif
         // ------------------------------ GEMV ------------------------------
         if (kind != 1) {
             const MegaGemv &g = a.g[ph];
@@ -1622,13 +1288,11 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
             } else {
                 // row phases: batches of 32 rows x n_kt K tiles x up to 4 stages of 8 rows
                 const unsigned ep_out = ep_step;
-                const bool x_once = MEGA_X_ONCE && g.n_kt == 1; // the whole activation fits the registers: load it once per phase
-                if (x_once) load_x<GS>(xr, kind == 4 ? sxq_dn : sxq, kind == 4 ? sxs_dn : sxs, 0, g.KT, g.G, lane);
                 for (int b0 = 0; b0 < count; b0 += MEGA_BATCH) {
                     const int nb = count - b0 < MEGA_BATCH ? count - b0 : MEGA_BATCH;
                     float acc0 = 0.f, acc1 = 0.f; // this warp's rows in its (up to) two stages of the batch
                     for (int kt = 0; kt < g.n_kt; kt++) {
-                        if (!x_once) load_x<GS>(xr, kind == 4 ? sxq_dn : sxq, kind == 4 ? sxs_dn : sxs, kt, g.KT, g.G, lane);
+                        load_x<GS>(xr, sxq, sxs, kt, g.KT, g.G, lane);
                         prof_mark(pr, 58);
                         for (int sidx = 0; MEGA_GW * sidx < nb; sidx++) {
                             if ((sidx & 1) == grp) { // stages alternate between the two consumer groups
@@ -1724,17 +1388,17 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
         }
         // pull what the next step's first instructions will miss on (static weights, HBM-cold) into L2:
         // the next RMSNorm weight, or the QK-norm weights + this position's RoPE row
-        if (MEGA_PREFETCH_W && (kind == 2 || kind == 4)) {
+        if (kind == 2 || kind == 4) {
             const float *wn = kind == 2 ? a.rms_ffn + (size_t)l * a.dim : (l + 1 < L1 ? a.rms_att + (size_t)(l + 1) * a.dim : a.rms_final);
             if (tid * 32 < a.dim) asm volatile("prefetch.global.L2 [%0];" ::"l"(wn + tid * 32));
-        } else if (MEGA_PREFETCH_W && kind == 0 && tid < 12) {
+        } else if (kind == 0 && tid < 12) {
             const float *wn = tid < 4 ? a.q_ln + (size_t)l * HEAD_DIM + tid * 32 : tid < 8 ? a.k_ln + (size_t)l * HEAD_DIM + (tid - 4) * 32
                                                                                    : a.rope + (size_t)pos * HEAD_DIM + (tid - 8) * 32;
             asm volatile("prefetch.global.L2 [%0];" ::"l"(wn));
         }
         // results carry their own flags: the only thing to wait for is this CTA's own warps (sxq / scratch are about to be rewritten)
         if (kind == 5) grid_barrier(a, bs, true, pr);
-        else if (!(MEGA_LAZY_SYNC && kind >= 2)) csync();
+        else csync();
         prof_mark(pr, 3 + 3 * kind);
     }
 

@@ -318,7 +318,6 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
         // across tile boundaries), independent of the tile producer.  History: as eight 512-byte bulk copies per stage issued by the
         // tile producer from a divergent single-lane branch, the scale traffic -- not the tensor pipe, not the epilogue -- set the
         // pace of the whole kernel (8B gate/up: 650 us; the same kernel with the scale traffic switched off: 457 us).
-#ifndef PF_DBG_NOSCALE // (timing experiment: no scale-row traffic at all, the epilogue scales with stale shared memory)
         if (!DENSE) {
             int sc = 0; // running pair count
             for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x) {
@@ -336,7 +335,6 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
                 }
             }
         }
-#endif
     } else if (warp == PF_MMA_WARP) {
         // ------------------------------- MMA issuer (whole warp runs the loop, one elected lane issues) -------------------------------
         // instruction descriptor: D = S32, A = B = signed int8, both K-major, N = 128, M = 128
@@ -435,11 +433,9 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
 #pragma unroll 1
                 for (int c = 0; c < npair; c++, pt++) {
                     const uint32_t ps = pt & 1, sl = pt & (PF_SRING - 1);
-#ifndef PF_DBG_NOSCALE
                     if (!s_ok) pf_wait(sb + PF_BAR_SFULL + 8 * sl, (pt / PF_SRING) & 1); // the pair's scale rows landed
                     // the next pair's scale rows: asked for here, looked at when they are needed (never, after the very last pair)
                     s_ok = pf_try(sb + PF_BAR_SFULL + 8 * ((pt + 1) & (PF_SRING - 1)), ((pt + 1) / PF_SRING) & 1);
-#endif
                     pf_drain_pair<MODE>(acc, d0, d1, tq + ps * (2 * PF_BN), wsx + sl * 2048, xsx + sl * 2048, sb + PF_BAR_TEMPTY + 16 * ps, lane,
                                         tq + (ps ^ 1) * (2 * PF_BN), sb + PF_BAR_TFULL + 8 * (ps ^ 1), ((pt + 1) >> 1) & 1);
                     __syncwarp();
@@ -606,298 +602,15 @@ __global__ void __launch_bounds__(128) k_pf_qknorm_rope(float *q, float *kc_laye
     reinterpret_cast<float4 *>(p)[lane] = r;
 }
 
-// Causal attention for T query tokens over the cache (key positions 0..pos0+t for query t), f32 on the
-// CUDA cores, flash-attention tiling (layers.rs:374-419 with an online softmax).  One CTA = one kv head
-// x a tile of BQ = 64/KVMUL query tokens, i.e. 64 query rows (token, head-in-group) that all share the
-// same K/V stream; key tiles of 32 positions go through shared memory.  256 threads: thread (ty, tx)
-// owns a 4-row x 2-key micro-tile of the score tile and a 4-row x 8-dim micro-tile of the output.
-constexpr int PFA_R = 64, PFA_BK = 32, PFA_LD = HEAD_DIM + 4, PFA_LDP = PFA_BK + 4;
-constexpr int PFA_SMEM = (PFA_R * PFA_LD + 2 * PFA_BK * PFA_LD + PFA_R * PFA_LDP) * 4;
-
-template <int KVMUL>
-__global__ void __launch_bounds__(256, 2) k_pf_attention(const float *__restrict__ q, const float *__restrict__ kc,
-                                                         const float *__restrict__ vc, float *out, int T, int pos0, int AH, int KV) {
-    extern __shared__ __align__(16) float pfa_smem[];
-    float *Qs = pfa_smem;                 // [64][132]
-    float *Ks = Qs + PFA_R * PFA_LD;      // [32][132]
-    float *Vs = Ks + PFA_BK * PFA_LD;     // [32][132]
-    float *Ps = Vs + PFA_BK * PFA_LD;     // [64][36]
-    constexpr int BQ = PFA_R / KVMUL;
-    const int kvh = blockIdx.x, q0 = blockIdx.y * BQ;
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const float scale = __fdiv_rn(1.0f, sqrtf((float)HEAD_DIM));
-    // Q tile: row r <-> (token q0 + r / KVMUL, head kvh*KVMUL + r % KVMUL)
-    for (int i = tid; i < PFA_R * 32; i += 256) {
-        const int r = i >> 5, c4 = i & 31;
-        const int tq = q0 + r / KVMUL;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (tq < T) v = reinterpret_cast<const float4 *>(q + (size_t)tq * AH + (size_t)(kvh * KVMUL + r % KVMUL) * HEAD_DIM)[c4];
-        *reinterpret_cast<float4 *>(Qs + r * PFA_LD + c4 * 4) = v;
-    }
-    float m[4], l[4], acc[4][8];
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        m[i] = -INFINITY;
-        l[i] = 0.0f;
-#pragma unroll
-        for (int j = 0; j < 8; j++) acc[i][j] = 0.0f;
-    }
-    int last_q = q0 + BQ - 1;
-    if (last_q > T - 1) last_q = T - 1;
-    const int nkeys = pos0 + last_q + 1; // causal horizon of the last query in the tile
-    const float *kb = kc + (size_t)kvh * HEAD_DIM, *vb = vc + (size_t)kvh * HEAD_DIM;
-    for (int k0 = 0; k0 < nkeys; k0 += PFA_BK) {
-        __syncthreads(); // previous tile fully consumed (also orders the Q tile stores on the first pass)
-        for (int i = tid; i < PFA_BK * 32; i += 256) {
-            const int p = i >> 5, c4 = i & 31;
-            float4 kv = make_float4(0.f, 0.f, 0.f, 0.f), vv = kv;
-            if (k0 + p < nkeys) {
-                kv = reinterpret_cast<const float4 *>(kb + (size_t)(k0 + p) * KV)[c4];
-                vv = reinterpret_cast<const float4 *>(vb + (size_t)(k0 + p) * KV)[c4];
-            }
-            *reinterpret_cast<float4 *>(Ks + p * PFA_LD + c4 * 4) = kv;
-            *reinterpret_cast<float4 *>(Vs + p * PFA_LD + c4 * 4) = vv;
-        }
-        __syncthreads();
-        // scores: rows 4*ty..+3, keys tx and tx+16 (adjacent lanes read adjacent rows: with the 132-float
-        // row pitch that is the conflict-free pattern for 128-bit shared loads)
-        float sc[4][2];
-#pragma unroll
-        for (int i = 0; i < 4; i++) sc[i][0] = sc[i][1] = 0.0f;
-#pragma unroll 8
-        for (int d4 = 0; d4 < 32; d4++) {
-            float4 kq[2], qq[4];
-#pragma unroll
-            for (int j = 0; j < 2; j++) kq[j] = *reinterpret_cast<const float4 *>(Ks + (tx + 16 * j) * PFA_LD + d4 * 4);
-#pragma unroll
-            for (int i = 0; i < 4; i++) qq[i] = *reinterpret_cast<const float4 *>(Qs + (4 * ty + i) * PFA_LD + d4 * 4);
-#pragma unroll
-            for (int i = 0; i < 4; i++)
-#pragma unroll
-                for (int j = 0; j < 2; j++)
-                    sc[i][j] += qq[i].x * kq[j].x + qq[i].y * kq[j].y + qq[i].z * kq[j].z + qq[i].w * kq[j].w;
-        }
-        // online softmax per row (a row's 32 scores live in the 16 lanes that share ty)
-#pragma unroll
-        for (int i = 0; i < 4; i++) {
-            const int r = 4 * ty + i;
-            const int qpos = pos0 + q0 + r / KVMUL;
-            float s0 = (k0 + tx <= qpos) ? __fmul_rn(sc[i][0], scale) : -INFINITY;
-            float s1 = (k0 + tx + 16 <= qpos) ? __fmul_rn(sc[i][1], scale) : -INFINITY;
-            float mx = fmaxf(s0, s1);
-#pragma unroll
-            for (int o = 8; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-            const float mn = fmaxf(m[i], mx);
-            const float corr = (mn == -INFINITY) ? 1.0f : expf(m[i] - mn);
-            const float p0 = (s0 == -INFINITY) ? 0.0f : expf(s0 - mn);
-            const float p1 = (s1 == -INFINITY) ? 0.0f : expf(s1 - mn);
-            float ps = p0 + p1;
-#pragma unroll
-            for (int o = 8; o > 0; o >>= 1) ps += __shfl_xor_sync(0xffffffffu, ps, o);
-            l[i] = l[i] * corr + ps;
-            m[i] = mn;
-#pragma unroll
-            for (int j = 0; j < 8; j++) acc[i][j] *= corr;
-            Ps[r * PFA_LDP + tx] = p0;
-            Ps[r * PFA_LDP + tx + 16] = p1;
-        }
-        __syncthreads();
-        // out[r][8*tx .. +7] += sum_p P[r][p] * V[p][8*tx .. +7]
-#pragma unroll 4
-        for (int p = 0; p < PFA_BK; p++) {
-            const float4 v0 = *reinterpret_cast<const float4 *>(Vs + p * PFA_LD + 8 * tx);
-            const float4 v1 = *reinterpret_cast<const float4 *>(Vs + p * PFA_LD + 8 * tx + 4);
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const float pr = Ps[(4 * ty + i) * PFA_LDP + p];
-                acc[i][0] += pr * v0.x; acc[i][1] += pr * v0.y; acc[i][2] += pr * v0.z; acc[i][3] += pr * v0.w;
-                acc[i][4] += pr * v1.x; acc[i][5] += pr * v1.y; acc[i][6] += pr * v1.z; acc[i][7] += pr * v1.w;
-            }
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        const int r = 4 * ty + i;
-        const int tq = q0 + r / KVMUL;
-        if (tq < T) {
-            const float inv = __fdiv_rn(1.0f, l[i]);
-            float *dst = out + (size_t)tq * AH + (size_t)(kvh * KVMUL + r % KVMUL) * HEAD_DIM + 8 * tx;
-            reinterpret_cast<float4 *>(dst)[0] = make_float4(__fmul_rn(acc[i][0], inv), __fmul_rn(acc[i][1], inv), __fmul_rn(acc[i][2], inv), __fmul_rn(acc[i][3], inv));
-            reinterpret_cast<float4 *>(dst)[1] = make_float4(__fmul_rn(acc[i][4], inv), __fmul_rn(acc[i][5], inv), __fmul_rn(acc[i][6], inv), __fmul_rn(acc[i][7], inv));
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------
-// Causal attention on the tensor cores: mma.sync m16n8k8 TF32 with the 3xTF32 split (x = hi + lo, hi = tf32(x),
-// lo = tf32(x - hi); a*b ~ hi*hi + hi*lo + lo*hi), which keeps the products at f32-class accuracy (relative error ~2^-21
-// instead of TF32's 2^-11: the attention output is re-quantised to int8 right after, and a coarser score would flip far
-// more int8 values than the f32 path does).  Same tiling idea as k_pf_attention: one CTA = one kv head x 64 query rows
-// (64 / KVMUL tokens x the KVMUL heads that share the K / V stream), 4 warps x 16 rows, key tiles of 32 positions whose
-// K and V rows are split into hi / lo once when they are staged in shared memory.
-//   S = Q K^T : A = Q fragment (split on the fly), B = K tile (key-major = "col" operand), 4 n-tiles x 16 k-steps
-//   O += P V  : the accumulator fragment of S doubles as the A fragment of P when the 8 keys of a k-step are taken in the
-//               order (0,2,4,6,1,3,5,7) -- the same permutation is applied to the rows of V in the B fragment, no shuffles.
-// ------------------------------------------------------------------------------------------
-constexpr int PFT_R = 64, PFT_BK = 32, PFT_LD = HEAD_DIM + 4;
-constexpr int PFT_SMEM = (PFT_R * PFT_LD + 4 * PFT_BK * PFT_LD) * 4;
-
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void split_tf32(float x, uint32_t &hi, uint32_t &lo) {
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hi) : "f"(x));
-    const float r = __fsub_rn(x, __uint_as_float(hi));
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(lo) : "f"(r));
-}
-
-template <int KVMUL>
-__global__ void __launch_bounds__(128, 2) k_pf_attention_tc(const float *__restrict__ q, const float *__restrict__ kc,
-                                                            const float *__restrict__ vc, float *out, int T, int pos0, int AH, int KV) {
-    extern __shared__ __align__(16) float pft_smem[];
-    float *Qs = pft_smem;                   // [64][132] f32
-    float *Kh = Qs + PFT_R * PFT_LD;        // [32][132] tf32 hi
-    float *Kl = Kh + PFT_BK * PFT_LD;       // [32][132] tf32 lo
-    float *Vh = Kl + PFT_BK * PFT_LD;
-    float *Vl = Vh + PFT_BK * PFT_LD;
-    constexpr int BQ = PFT_R / KVMUL;
-    const int kvh = blockIdx.x, q0 = blockIdx.y * BQ;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
-    const float scale = __fdiv_rn(1.0f, sqrtf((float)HEAD_DIM));
-    // Q tile: row r <-> (token q0 + r / KVMUL, head kvh*KVMUL + r % KVMUL)
-    for (int i = tid; i < PFT_R * 32; i += 128) {
-        const int r = i >> 5, c4 = i & 31;
-        const int tq = q0 + r / KVMUL;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (tq < T) v = reinterpret_cast<const float4 *>(q + (size_t)tq * AH + (size_t)(kvh * KVMUL + r % KVMUL) * HEAD_DIM)[c4];
-        *reinterpret_cast<float4 *>(Qs + r * PFT_LD + c4 * 4) = v;
-    }
-    const int r0 = warp * 16 + g, r1 = r0 + 8;             // this thread's two rows of the tile
-    const int qp0 = pos0 + q0 + r0 / KVMUL, qp1 = pos0 + q0 + r1 / KVMUL; // their absolute positions
-    float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.0f, l1 = 0.0f;
-    float o[16][4];
-#pragma unroll
-    for (int j = 0; j < 16; j++) o[j][0] = o[j][1] = o[j][2] = o[j][3] = 0.0f;
-    int last_q = q0 + BQ - 1;
-    if (last_q > T - 1) last_q = T - 1;
-    const int nkeys = pos0 + last_q + 1; // causal horizon of the last query in the tile
-    const float *kb = kc + (size_t)kvh * HEAD_DIM, *vb = vc + (size_t)kvh * HEAD_DIM;
-    for (int k0 = 0; k0 < nkeys; k0 += PFT_BK) {
-        __syncthreads(); // previous tile fully consumed (also orders the Q tile stores on the first pass)
-        for (int i = tid; i < PFT_BK * 32; i += 128) {
-            const int p = i >> 5, c4 = i & 31;
-            float4 kv = make_float4(0.f, 0.f, 0.f, 0.f), vv = kv;
-            if (k0 + p < nkeys) {
-                kv = reinterpret_cast<const float4 *>(kb + (size_t)(k0 + p) * KV)[c4];
-                vv = reinterpret_cast<const float4 *>(vb + (size_t)(k0 + p) * KV)[c4];
-            }
-            uint32_t h[4], lo[4];
-            split_tf32(kv.x, h[0], lo[0]); split_tf32(kv.y, h[1], lo[1]); split_tf32(kv.z, h[2], lo[2]); split_tf32(kv.w, h[3], lo[3]);
-            *reinterpret_cast<uint4 *>(Kh + p * PFT_LD + c4 * 4) = make_uint4(h[0], h[1], h[2], h[3]);
-            *reinterpret_cast<uint4 *>(Kl + p * PFT_LD + c4 * 4) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-            split_tf32(vv.x, h[0], lo[0]); split_tf32(vv.y, h[1], lo[1]); split_tf32(vv.z, h[2], lo[2]); split_tf32(vv.w, h[3], lo[3]);
-            *reinterpret_cast<uint4 *>(Vh + p * PFT_LD + c4 * 4) = make_uint4(h[0], h[1], h[2], h[3]);
-            *reinterpret_cast<uint4 *>(Vl + p * PFT_LD + c4 * 4) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-        }
-        __syncthreads();
-        // ---- S = Q K^T (16 rows x 32 keys per warp) ----
-        float s[4][4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) s[j][0] = s[j][1] = s[j][2] = s[j][3] = 0.0f;
-#pragma unroll 4
-        for (int ks = 0; ks < 16; ks++) {
-            const int d0 = ks * 8 + t;
-            uint32_t ah[4], al[4];
-            split_tf32(Qs[r0 * PFT_LD + d0], ah[0], al[0]);
-            split_tf32(Qs[r1 * PFT_LD + d0], ah[1], al[1]);
-            split_tf32(Qs[r0 * PFT_LD + d0 + 4], ah[2], al[2]);
-            split_tf32(Qs[r1 * PFT_LD + d0 + 4], ah[3], al[3]);
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const int krow = (8 * j + g) * PFT_LD + d0;
-                const uint32_t bh0 = __float_as_uint(Kh[krow]), bh1 = __float_as_uint(Kh[krow + 4]);
-                const uint32_t bl0 = __float_as_uint(Kl[krow]), bl1 = __float_as_uint(Kl[krow + 4]);
-                mma_tf32(s[j], al, bh0, bh1);
-                mma_tf32(s[j], ah, bl0, bl1);
-                mma_tf32(s[j], ah, bh0, bh1);
-            }
-        }
-        // ---- online softmax: thread holds keys k0 + 8j + {2t, 2t+1} of rows r0 (s[j][0..1]) and r1 (s[j][2..3]) ----
-        float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int key = k0 + 8 * j + 2 * t;
-            s[j][0] = (key <= qp0) ? __fmul_rn(s[j][0], scale) : -INFINITY;
-            s[j][1] = (key + 1 <= qp0) ? __fmul_rn(s[j][1], scale) : -INFINITY;
-            s[j][2] = (key <= qp1) ? __fmul_rn(s[j][2], scale) : -INFINITY;
-            s[j][3] = (key + 1 <= qp1) ? __fmul_rn(s[j][3], scale) : -INFINITY;
-            mx0 = fmaxf(mx0, fmaxf(s[j][0], s[j][1]));
-            mx1 = fmaxf(mx1, fmaxf(s[j][2], s[j][3]));
-        }
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-        const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);
-        const float c0 = (mn0 == -INFINITY) ? 1.0f : expf(m0 - mn0), c1 = (mn1 == -INFINITY) ? 1.0f : expf(m1 - mn1);
-        m0 = mn0;
-        m1 = mn1;
-        l0 *= c0;
-        l1 *= c1;
-#pragma unroll
-        for (int j = 0; j < 16; j++) {
-            o[j][0] *= c0;
-            o[j][1] *= c0;
-            o[j][2] *= c1;
-            o[j][3] *= c1;
-        }
-        // ---- O += P V: k-step j = keys 8j .. 8j+7 in the order (0,2,4,6,1,3,5,7) ----
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const float p00 = (s[j][0] == -INFINITY) ? 0.0f : expf(s[j][0] - mn0), p01 = (s[j][1] == -INFINITY) ? 0.0f : expf(s[j][1] - mn0);
-            const float p10 = (s[j][2] == -INFINITY) ? 0.0f : expf(s[j][2] - mn1), p11 = (s[j][3] == -INFINITY) ? 0.0f : expf(s[j][3] - mn1);
-            l0 += p00 + p01;
-            l1 += p10 + p11;
-            uint32_t ah[4], al[4]; // a0 (r0, k = t) = P[r0][2t], a1 (r1, t) = P[r1][2t], a2 (r0, t+4) = P[r0][2t+1], a3 (r1, t+4) = P[r1][2t+1]
-            split_tf32(p00, ah[0], al[0]);
-            split_tf32(p10, ah[1], al[1]);
-            split_tf32(p01, ah[2], al[2]);
-            split_tf32(p11, ah[3], al[3]);
-            const int vrow0 = (8 * j + 2 * t) * PFT_LD + g, vrow1 = vrow0 + PFT_LD;
-#pragma unroll
-            for (int n = 0; n < 16; n++) {
-                const uint32_t bh0 = __float_as_uint(Vh[vrow0 + 8 * n]), bh1 = __float_as_uint(Vh[vrow1 + 8 * n]);
-                const uint32_t bl0 = __float_as_uint(Vl[vrow0 + 8 * n]), bl1 = __float_as_uint(Vl[vrow1 + 8 * n]);
-                mma_tf32(o[n], al, bh0, bh1);
-                mma_tf32(o[n], ah, bl0, bl1);
-                mma_tf32(o[n], ah, bh0, bh1);
-            }
-        }
-    }
-    // row sums live spread over the quad
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-    const float i0 = __fdiv_rn(1.0f, l0), i1 = __fdiv_rn(1.0f, l1);
-    const int tq0 = q0 + r0 / KVMUL, tq1 = q0 + r1 / KVMUL;
-    float *d0 = out + (size_t)tq0 * AH + (size_t)(kvh * KVMUL + r0 % KVMUL) * HEAD_DIM + 2 * t;
-    float *d1 = out + (size_t)tq1 * AH + (size_t)(kvh * KVMUL + r1 % KVMUL) * HEAD_DIM + 2 * t;
-#pragma unroll
-    for (int n = 0; n < 16; n++) {
-        if (tq0 < T) *reinterpret_cast<float2 *>(d0 + 8 * n) = make_float2(__fmul_rn(o[n][0], i0), __fmul_rn(o[n][1], i0));
-        if (tq1 < T) *reinterpret_cast<float2 *>(d1 + 8 * n) = make_float2(__fmul_rn(o[n][2], i1), __fmul_rn(o[n][3], i1));
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// Causal attention on the tensor cores, second version: mma.sync m16n8k16 on an FP16 hi / lo split with f32 accumulation.
-//   x = hi + lo, hi = fp16(x), lo = fp16(x - hi);  a*b ~ hi*hi + hi*lo + lo*hi   (relative error ~2^-21, as the 3xTF32 form)
-// Against the TF32 kernel above: a k16 MMA covers twice the depth of a k8 one (half the MMA count), the operands are half as
-// wide in shared memory, fragments come in with ldmatrix (4 8x8 tiles per instruction instead of 32-bit loads), and K / V are
-// split ONCE per layer by k_pf_split_kv instead of by every CTA that streams them -- the tiles then arrive with cp.async,
+// Causal attention for T query tokens over the cache (key positions 0..pos0+t for query t; layers.rs:374-419 with an online
+// softmax) on the tensor cores: mma.sync m16n8k16 on an FP16 hi / lo split with f32 accumulation.
+//   x = hi + lo, hi = fp16(x), lo = fp16(x - hi);  a*b ~ hi*hi + hi*lo + lo*hi   (relative error ~2^-21 instead of 2^-11 for a
+//   single FP16 or TF32 product: the attention output is re-quantised to int8 right after, and a coarser score would flip far
+//   more int8 values than f32 arithmetic does).
+// FP16 rather than TF32 operands: a k16 MMA covers twice the depth of a TF32 k8 one (half the MMA count), the operands are half
+// as wide in shared memory, and fragments come in with ldmatrix (4 8x8 tiles per instruction instead of 32-bit loads).  K / V
+// are split ONCE per layer by k_pf_split_kv rather than by every CTA that streams them -- the tiles then arrive with cp.async,
 // double-buffered, no ALU work on the way.
 //   FP16 range: hi overflows beyond 65504 (K is QK-normalised, P <= 1; V / Q of that size do not occur), and a lo part below
 //   6.1e-5 is subnormal -- an absolute error of <= 3e-8 per element, far below the f32 round-off of the sums it enters.

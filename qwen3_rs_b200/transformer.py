@@ -96,7 +96,7 @@ ABI = {
     "q3_op_gemm_q8": (_i, [_i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "q3_op_sample": (_i, [_i, _vp, _i, _f, _f, C.POINTER(C.c_ulonglong), C.POINTER(_i)]),
     "q3_bench_gemm_q8": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(_f)]),
-    "q3_op_prefill_attention": (_i, [_i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "q3_op_prefill_attention": (_i, [_i, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "q3_op_rmsnorm": (_i, [_i, _vp, _vp, _i, _vp]),
     "q3_op_quantize_q80": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
     "q3_op_quantize_q80_dev": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
@@ -408,14 +408,14 @@ def op_sample(logits, temperature: float, topp: float, rng_state: int, device: i
     return tok.value, st.value
 
 
-def op_prefill_attention(q, k, v, pos0: int, n_heads: int, n_kv: int, f32_cuda_cores=0, device: int = 0):
-    """Causal attention of T = q.shape[0] query tokens at positions pos0.. over k / v rows [pos0 + T][n_kv * 128].
-    f32_cuda_cores: 0 = the tensor-core kernel q3_prefill runs (FP16 hi / lo split), 1 / True = f32 on the CUDA cores, 2 = 3xTF32."""
+def op_prefill_attention(q, k, v, pos0: int, n_heads: int, n_kv: int, device: int = 0):
+    """Causal attention of T = q.shape[0] query tokens at positions pos0.. over k / v rows [pos0 + T][n_kv * 128], with the
+    tensor-core kernel q3_prefill runs (FP16 hi / lo split)."""
     q = np.ascontiguousarray(q, np.float32)
     k = np.ascontiguousarray(k, np.float32)
     v = np.ascontiguousarray(v, np.float32)
     out = np.empty_like(q)
-    _check(load_library().q3_op_prefill_attention(device, _ptr(q), _ptr(k), _ptr(v), q.shape[0], pos0, n_heads, n_kv, int(f32_cuda_cores), _ptr(out)))
+    _check(load_library().q3_op_prefill_attention(device, _ptr(q), _ptr(k), _ptr(v), q.shape[0], pos0, n_heads, n_kv, _ptr(out)))
     return out
 
 

@@ -695,7 +695,7 @@ def _check_prefill_vs_oracle(m, o, o2, toks, label):
             assert np.median(ek) <= max(1e-6, 3 * np.median(ek2)) and np.median(ev) <= max(1e-6, 3 * np.median(ev2)), label
             assert rows_off <= max(0.4, 1.25 * rows_ref) and ek.max() <= 2e-2, (rows_off, rows_ref, float(ek.max()))
         # deeper layers: an upstream flip perturbs every later element a little (and, through attention, later tokens), so only the
-        # noise level is checked here -- the attention kernel itself is compared with float64 in test_prefill_attention_kernels_...
+        # noise level is checked here -- the attention kernel itself is compared with float64 in test_prefill_attention_against_float64
         assert np.median(ev) <= 1e-2 * max(1.0, float(np.abs(vr).max())), (l, float(np.median(ev)))
         assert ev.max() <= 0.05 * np.abs(vr).max() + 1e-2 and ek.max() <= 0.05 * np.abs(kr).max() + 1e-2
         k1, v1 = m.kv_read(l, T, 1)
@@ -708,10 +708,10 @@ def _check_prefill_vs_oracle(m, o, o2, toks, label):
 @pytest.mark.parametrize("T,pos0,n_heads,n_kv", [(70, 0, 8, 2), (33, 45, 4, 4), (129, 3, 16, 2), (200, 0, 2, 1),
                                                  (1000, 1100, 40, 5), (517, 1531, 16, 8),
                                                  pytest.param(2048, 0, 32, 8, marks=pytest.mark.slow)])
-def test_prefill_attention_kernels_against_float64(T, pos0, n_heads, n_kv):
-    """The batched causal attention alone (the tensor-core kernel q3_prefill runs -- FP16 hi / lo split --, the f32 CUDA-core
-    kernel and the first tensor-core version, 3xTF32) against a float64 softmax attention: f32-class accuracy (1e-5 of the
-    value scale), i.e. the operand split loses nothing that matters to the int8 re-quantisation behind it."""
+def test_prefill_attention_against_float64(T, pos0, n_heads, n_kv):
+    """The batched causal attention alone (the tensor-core kernel q3_prefill runs, FP16 hi / lo split) against a float64
+    softmax attention: f32-class accuracy (1e-5 of the value scale), i.e. the operand split loses nothing that matters to the
+    int8 re-quantisation behind it."""
     rng = np.random.default_rng(T + pos0)
     hd, nk = 128, pos0 + T
     q = rng.standard_normal((T, n_heads * hd)).astype(np.float32)
@@ -727,8 +727,7 @@ def test_prefill_attention_kernels_against_float64(T, pos0, n_heads, n_kv):
         s[mask] = -np.inf
         p = np.exp(s - s.max(axis=1, keepdims=True))
         ref[:, h * hd:(h + 1) * hd] = (p / p.sum(axis=1, keepdims=True)) @ vh
-    for kind, label in ((0, "fp16 hi/lo"), (1, "f32"), (2, "3xTF32")):
-        out = T_mod.op_prefill_attention(q, k, v, pos0, n_heads, n_kv, f32_cuda_cores=kind)
-        err = float(np.abs(out - ref).max())
-        print(f"prefill attention T={T} pos0={pos0} heads {n_heads}/{n_kv} {label}: max err {err:.2e}")
-        assert err <= 2e-5 * max(1.0, float(np.abs(ref).max()))
+    out = T_mod.op_prefill_attention(q, k, v, pos0, n_heads, n_kv)
+    err = float(np.abs(out - ref).max())
+    print(f"prefill attention T={T} pos0={pos0} heads {n_heads}/{n_kv}: max err {err:.2e}")
+    assert err <= 2e-5 * max(1.0, float(np.abs(ref).max()))

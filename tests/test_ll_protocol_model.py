@@ -1,4 +1,4 @@
-"""Model check of the persistent kernel's flagged exchange (q3_mega.cuh, MEGA_LL; DESIGN.md section 4).
+"""Model check of the persistent kernel's flagged exchange (q3_mega.cuh, ll_store; DESIGN.md section 4).
 
 The o_proj / down rows travel as (value, epoch) words with NO barrier between writer and reader, pushed into every rank's
 landing zone; the zones are reused one layer later.  This is a discrete-event model of exactly the dependency structure the
