@@ -201,8 +201,8 @@ int q3_op_expf(int device, const float *x, int n, float *out);
  * operands): out[T][N] = per-token tensor.rs:23-62 matmul of x (int8[T][K] + f32[T][K/gs]) with
  * row-major w (int8[N][K] + f32[N][K/gs]).  N, K multiples of 128.  The int32 group dots are exact either way;
  * exact == 1: the f32 group terms are unfused and added in group order -- bit-identical to the per-token GEMV in exact
- * mode; exact == 0: the drain q3_prefill runs (fused multiply-add per group, same order of groups); exact == 2: see
- * q3_bench_gemm_q8 (raw integer dots over all of K, scales ignored). */
+ * mode; exact == 0: the drain q3_prefill runs (fused multiply-add per group, same order of groups).  Any other value of
+ * exact is Q3_EINVAL. */
 int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, const int8_t *wq, const float *ws,
                   int T, int N, int K, int gs, int exact, float *out);
 /* layers.rs:374-419 for T query tokens at once (the batched prefill's causal attention): q [T][n_heads*128] after QK-norm
@@ -211,9 +211,7 @@ int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, const int8_t *w
 int q3_op_prefill_attention(int device, const float *q, const float *k, const float *v, int T, int pos0, int n_heads,
                             int n_kv, float *out);
 /* Timing helper: the tensor-core GEMM alone on device-resident pseudo-random operands (CUDA events, best of reps,
- * milliseconds per launch).  mode 0 / 1 as `exact` above; mode 2 = dense ceiling of the same tiling and pipeline (no group
- * structure: all of K accumulated in one TMEM buffer, one drain per tile) -- the measured int8 peak the group-scaled
- * kernel is compared with. */
+ * milliseconds per launch).  mode 0 / 1 as `exact` above; any other mode is Q3_EINVAL. */
 int q3_bench_gemm_q8(int device, int T, int N, int K, int gs, int mode, int reps, float *ms_out);
 /* sampler.rs:116-136 Sampler::sample with temperature > 0 on host-supplied logits (n f32): one draw on the device;
  * *rng_state is Sampler::rng_state before the call and after it. */

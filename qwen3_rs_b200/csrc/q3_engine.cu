@@ -632,7 +632,6 @@ static int build_mega(q3_handle *h, const float *rms_att_all, const float *rms_f
     a.x = h->x;
     a.zq = h->zq; a.za = h->za; a.zh = h->zh; a.zr[0] = h->zr[0]; a.zr[1] = h->zr[1];
     a.attn_part = h->attn_part; a.att_cnt = h->att_cnt;
-    a.dbg = getenv("Q3_MEGA_DBG") ? atoi(getenv("Q3_MEGA_DBG")) : 0;
     a.bar = h->d_bar; a.status = d_status; a.tokpos = h->d_tokpos; a.history = h->d_history;
     // until q3_tp_connect every "peer" slot points at this rank's own buffers
     for (int r = 0; r < MEGA_MAX_TP; r++) {
@@ -792,11 +791,11 @@ static int make_map_scales(CUtensorMap *map, const float *base, int groups, int 
     return 0;
 }
 
-template <int GS, int EPI, int MODE>
+template <int GS, int EPI, bool EXACT>
 static int launch_gemm_q8_t(const CUtensorMap &mx, const CUtensorMap &mw, const PrefillGemmArgs &a, cudaStream_t s) {
     static bool attr = false;
     if (!attr) {
-        CK(cudaFuncSetAttribute(k_gemm_q8<GS, EPI, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
+        CK(cudaFuncSetAttribute(k_gemm_q8<GS, EPI, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
         attr = true;
     }
     static int num_sms = 0;
@@ -809,24 +808,21 @@ static int launch_gemm_q8_t(const CUtensorMap &mx, const CUtensorMap &mw, const 
     int rc;
     if ((rc = make_map_scales(&mxs, a.xsT, a.K / GS, a.Tpad)) || (rc = make_map_scales(&mws, a.wsT, a.K / GS, a.N))) return rc;
     const int tiles = (a.N / PF_BN) * (a.Tpad / PF_BM); // persistent: one CTA per SM walks the tiles
-    k_gemm_q8<GS, EPI, MODE><<<tiles < num_sms ? tiles : num_sms, PF_THREADS, PF_SMEM, s>>>(mx, mw, mxs, mws, a);
+    k_gemm_q8<GS, EPI, EXACT><<<tiles < num_sms ? tiles : num_sms, PF_THREADS, PF_SMEM, s>>>(mx, mw, mxs, mws, a);
     return 0;
 }
-// mode 0: the fast drain (what q3_prefill runs); 1: reference-order f32 fold (bit-identical to matmul); 2: dense ceiling
-// (timing experiment: no group structure, one drain per tile) -- the int32 group dots are the same in modes 0 and 1
+// mode 0: the fast drain (what q3_prefill runs); 1: the exact drain, reference-order f32 fold (bit-identical to matmul), built
+// for the plain store epilogue only -- the operator and timing entry points are its only callers.  The int32 group dots are
+// the same in both modes.
 template <int EPI>
 static int launch_gemm_q8(int gs, const CUtensorMap &mx, const CUtensorMap &mw, const PrefillGemmArgs &a, cudaStream_t s, int mode = 0) {
     int rc = 0;
-    if (mode == 1) {
-        GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, EPI, 1>(mx, mw, a, s)));
-    } else if (mode >= 2 && mode <= 5) {
-        if (EPI != PF_EPI_STORE) return fail(Q3_EINVAL, "timing-experiment modes only with the plain store epilogue");
-        if (mode == 2) GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, PF_EPI_STORE, 2>(mx, mw, a, s)));
-        if (mode == 3) GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, PF_EPI_STORE, 3>(mx, mw, a, s)));
-        if (mode == 4) GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, PF_EPI_STORE, 4>(mx, mw, a, s)));
-        if (mode == 5) GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, PF_EPI_STORE, 5>(mx, mw, a, s)));
+    if (mode == 0) {
+        GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, EPI, false>(mx, mw, a, s)));
+    } else if (mode == 1 && EPI == PF_EPI_STORE) {
+        GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, PF_EPI_STORE, true>(mx, mw, a, s)));
     } else {
-        GS_DISPATCH(gs, (rc = launch_gemm_q8_t<GS, EPI, 0>(mx, mw, a, s)));
+        return fail(Q3_EINVAL, "prefill GEMM mode %d: 0 = fast drain, 1 = exact drain (plain store epilogue only)", mode);
     }
     return rc;
 }
@@ -925,8 +921,9 @@ static int prefill_tp_rowparallel(q3_handle *h, int which, const CUtensorMap &mx
     h->pf_xbar_count++;
     k_pf_xbarrier<<<1, 32, 0, h->stream>>>(h->pf_peers[which], h->tp_size, h->tp_rank, h->pf_xbar_count * (unsigned long long)h->tp_size, h->d_status);
     const size_t n4 = (size_t)T * h->cfg.dim / 4;
-    static const int rsag = getenv("Q3_PF_TP_RSAG") ? atoi(getenv("Q3_PF_TP_RSAG")) : -1; // -1: by group size; 0 / 1: forced (tests)
-    if (rsag == 1 || (rsag < 0 && h->tp_size > 2)) { // reduce-scatter, barrier, all-gather: 2 (tp-1)/tp blocks over NVLink instead of tp-1
+    // tp > 2: reduce-scatter, barrier, all-gather -- 2 (tp-1)/tp blocks over NVLink instead of tp-1.  At tp 2 both move one block,
+    // and the one-pass all-reduce saves the second barrier.
+    if (h->tp_size > 2) {
         k_pf_reduce_scatter<<<h->num_sms * 2, 256, 0, h->stream>>>(h->pf_peers[which], g.out, h->tp_size, h->tp_rank, n4);
         h->pf_xbar_count++;
         k_pf_xbarrier<<<1, 32, 0, h->stream>>>(h->pf_peers[which], h->tp_size, h->tp_rank, h->pf_xbar_count * (unsigned long long)h->tp_size, h->d_status);
@@ -1815,6 +1812,7 @@ extern "C" int q3_op_gemm_q8(int device, const int8_t *xq, const float *xs, cons
     int rc = op_prologue(device, gs);
     if (rc) return rc;
     if (T <= 0 || N % 128 || K % 128 || K % gs || (K / gs) % 2) return fail(Q3_EINVAL, "need N %% 128 == 0, K %% 128 == 0 and an even number of groups per row");
+    if (exact != 0 && exact != 1) return fail(Q3_EINVAL, "exact must be 0 (fast drain) or 1 (exact drain), not %d", exact);
     const int Tpad = (T + 127) / 128 * 128, ng = K / gs;
     DevBuf dxq, dxsT, dwq, dws, dwsT, dout;
     if ((rc = dxq.alloc((size_t)Tpad * K)) || (rc = dxsT.alloc((size_t)ng * Tpad * 4)) || (rc = dwq.alloc((size_t)N * K)) ||
@@ -1913,7 +1911,7 @@ extern "C" int q3_op_prefill_attention(int device, const float *q, const float *
 }
 
 // Timing helper: the tcgen05 GEMM alone on device-resident random operands, CUDA events; mode as in q3_op_gemm_q8
-// (0 fast drain, 1 exact drain, 2 dense int8 ceiling of the same tiling).  ms_out = milliseconds per launch (best of reps).
+// (0 fast drain, 1 exact drain).  ms_out = milliseconds per launch (best of reps).
 __global__ void k_fill_i8(int8_t *p, size_t n, unsigned seed) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         unsigned h = (unsigned)i * 2654435761u + seed;
@@ -1927,7 +1925,7 @@ __global__ void k_fill_f32(float *p, size_t n, float v) {
 extern "C" int q3_bench_gemm_q8(int device, int T, int N, int K, int gs, int mode, int reps, float *ms_out) {
     int rc = op_prologue(device, gs);
     if (rc) return rc;
-    if (T <= 0 || N % 128 || K % 128 || K % gs || (K / gs) % 2 || reps < 1 || mode < 0 || mode > 5) return fail(Q3_EINVAL, "bad gemm bench arguments");
+    if (T <= 0 || N % 128 || K % 128 || K % gs || (K / gs) % 2 || reps < 1 || (mode != 0 && mode != 1)) return fail(Q3_EINVAL, "bad gemm bench arguments");
     const int Tpad = (T + 127) / 128 * 128, ng = K / gs;
     DevBuf dxq, dxsT, dwq, dwsT, dout;
     if ((rc = dxq.alloc((size_t)Tpad * K)) || (rc = dxsT.alloc((size_t)ng * Tpad * 4)) || (rc = dwq.alloc((size_t)N * K)) ||
@@ -1943,24 +1941,6 @@ extern "C" int q3_bench_gemm_q8(int device, int T, int N, int K, int gs, int mod
     a.T = T; a.Tpad = Tpad; a.N = N; a.K = K; a.wsT = dwsT.as<float>(); a.xsT = dxsT.as<float>(); a.out = dout.as<float>(); a.ld_out = N;
     if ((rc = launch_gemm_q8<PF_EPI_STORE>(gs, mx, mw, a, 0, mode))) return rc; // warm-up
     CK(cudaDeviceSynchronize());
-    if (getenv("Q3_PF_TRACE")) { // one extra launch with the in-kernel stamps of CTA 0 switched on; dumped to stderr (cycles, relative)
-#if PF_TRACE
-        DevBuf dtr;
-        if ((rc = dtr.alloc((size_t)4 * PF_TRACE_N * 8))) return rc;
-        CK(cudaMemset(dtr.p, 0, (size_t)4 * PF_TRACE_N * 8));
-        PrefillGemmArgs at = a;
-        at.trace = dtr.as<long long>();
-        if ((rc = launch_gemm_q8<PF_EPI_STORE>(gs, mx, mw, at, 0, mode))) return rc;
-        CK(cudaDeviceSynchronize());
-        std::vector<long long> tr((size_t)4 * PF_TRACE_N);
-        CK(cudaMemcpy(tr.data(), dtr.p, tr.size() * 8, cudaMemcpyDeviceToHost));
-        const long long t0 = tr[PF_TRACE_N]; // first commit
-        fprintf(stderr, "pair  mma:slot_free  mma:committed   (MMA warp of CTA 0, cycles after the first commit; T %d N %d K %d mode %d)\n", T, N, K, mode);
-        for (int i = 0; i < 48; i++) fprintf(stderr, "%4d %14lld %14lld\n", i, tr[i] ? tr[i] - t0 : -1, tr[PF_TRACE_N + i] - t0);
-#else
-        fprintf(stderr, "Q3_PF_TRACE: this library was built without -DPF_TRACE=1 (python scripts/ab_variants.py build trace:PF_TRACE=1, then Q3_LIB=...)\n");
-#endif
-    }
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));

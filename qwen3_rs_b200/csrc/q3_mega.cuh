@@ -105,9 +105,6 @@ struct MegaArgs {
     int layer0, layer1, from_embed, run_head, feedback, gather_logits;
     unsigned ll_base;                // epoch counter before this launch, already reduced mod 2^32 - 1 (host-tracked, same on every TP rank)
     unsigned long long *prof;        // optional [grid][MEGA_PROF_EVENTS] clock64 stamps (thread 0 of each CTA)
-    int dbg;                         // timing experiments only (env Q3_MEGA_DBG; results are garbage): 1 = every bulk copy reads the
-                                     // same L2-resident bytes (no HBM traffic), 2 = grid barrier skipped, 4 = prologues / polls skipped,
-                                     // 8 = attention position loop without arithmetic (the K / V stream alone)
 };
 // In-kernel profiler: thread 0 of every CTA appends (clock64 << 8 | tag).  Tags: 0 start; 1 + 3*kind + {0 prologue done,
 // 1 GEMV done, 2 step-end sync done} for step kinds 0..5; >= 32 finer marks inside the prologues and the grid barrier.
@@ -746,12 +743,6 @@ __device__ __forceinline__ void attention_item(const MegaArgs &a, int layer, int
                 rp.fullp ^= 1u << slot;
                 const uint32_t kt = ring_s + slot * slot_bytes, vt = kt + MEGA_KV_ROWS * HEAD_DIM * 4;
                 const int tb = t0 + st * MEGA_KV_ROWS, t = tb + lane; // first position of the stage, this lane's position
-                if (a.dbg & 8) { // timing experiment: the K / V stream through the ring without the arithmetic
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&empty[slot]);
-                    rp.it++;
-                    continue;
-                }
                 const uint32_t krow = (t == pos ? sk_s : kt + lane * (HEAD_DIM * 4)) + part * (DPP * 4);
                 const uint32_t qrow = sq_s + part * (DPP * 4);
                 // four chunks per round: eight 128-bit loads in flight, four independent partial sums
@@ -952,7 +943,6 @@ struct BarState {
 // through a leader CTA.
 __device__ __noinline__ void grid_barrier(const MegaArgs &a, BarState &bs, bool cross, Prof &pr) {
     csync();
-    if (a.dbg & 2) return;
     prof_mark(pr, 40); // all consumer warps of this CTA done
     const bool x = cross && a.tp_size > 1;
     if (threadIdx.x == 0) {
@@ -1106,7 +1096,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
             mbar_wait(&empty[slot], ((it / MEGA_NSTAGE) & 1) ^ 1, a.status);
             uint64_t *fb = &full[owner * MEGA_NSTAGE + slot];
             mbar_expect_tx(fb, bytes);
-            bulk_g2s(ring + (size_t)slot * slot_bytes, (a.dbg & 1) ? a.g[0].base + (size_t)blockIdx.x * 36864 : src, bytes, fb, policy);
+            bulk_g2s(ring + (size_t)slot * slot_bytes, src, bytes, fb, policy);
             __threadfence_block();
             issued[slot] = it / MEGA_NSTAGE + 1;
             prof_mark(pr, 64 + slot);
@@ -1219,9 +1209,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
         const unsigned ep_prev = ll_epoch(a.ll_base, (unsigned)(MEGA_EDGES * (l - L0) + kind - 1)); // of the preceding step of this layer
         int ph = PH_QKV;
         // ------------------------------ prologue ------------------------------
-        if (a.dbg & 4) {
-            ph = kind == 0 ? PH_QKV : kind == 2 ? PH_O : kind == 3 ? PH_GU : kind == 4 ? PH_DN : PH_HEAD;
-        } else if (kind == 0 || kind == 3 || kind == 5) {
+        if (kind == 0 || kind == 3 || kind == 5) {
             // RMSNorm + quantize of the residual stream (qwen3.rs:134-136, 159-161, 72-75)
             const float *w = kind == 0 ? a.rms_att + (size_t)l * a.dim : kind == 3 ? a.rms_ffn + (size_t)l * a.dim : a.rms_final;
             const bool emb = kind == 0 && l == L0 && a.from_embed;

@@ -52,21 +52,7 @@ struct PrefillGemmArgs {
     float *q;          // [T][AH]
     float *kc, *vc;    // layer base of the caches [seq][KV]
     int AH, KV, pos0;
-    long long *trace;  // optional (Q3_PF_TRACE): [20][PF_TRACE_N] clock64 stamps of CTA 0 -- MMA thread: pair may be reused / pair committed;
-                       // epilogue warp 0: pair complete seen / pair released
 };
-constexpr int PF_TRACE_N = 512;
-#ifndef PF_TRACE
-#define PF_TRACE 0 // 1: build with the in-kernel pipeline stamps (a variant library for scripts/diag/gemm_trace.py; costs registers in the drain loop)
-#endif
-#if PF_TRACE
-#define PF_STAMP(row, idx)                                                                                  \
-    do {                                                                                                    \
-        if (a.trace && blockIdx.x == 0 && (idx) < PF_TRACE_N) a.trace[(row) * PF_TRACE_N + (idx)] = clock64(); \
-    } while (0)
-#else
-#define PF_STAMP(row, idx) do { } while (0)
-#endif
 
 __device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t saddr) {
     // K-major, SWIZZLE_128B: 8-row atoms of 128 B, atoms 1024 B apart (SBO), LBO unused (=1), version 1
@@ -138,22 +124,13 @@ __device__ __forceinline__ void pf_wait_ld() { asm volatile("tcgen05.wait::ld.sy
 // 16 accumulator columns of one group: acc[j] += (f32(dot_j) * ws_j) * xs.
 // EXACT: unfused multiplies and add, i.e. the reference's left fold term by term (tensor.rs:59-61) -- bit-identical.
 // fast: the same exact int32 dots; p = ws * xs is formed first (it does not depend on the TMEM read), then one packed FMA.
-// VAR: 0 fast, 1 EXACT, 3 = timing experiment "TMEM reads but no arithmetic" (the 16 values are folded into one register)
-template <int VAR>
+template <bool EXACT>
 __device__ __forceinline__ void pf_scale16(float *acc, const uint32_t (&d)[16], uint32_t ws_saddr, float xs) {
-    constexpr bool EXACT_ = VAR == 1;
-    if (VAR >= 3) {
-        uint32_t x = 0;
-#pragma unroll
-        for (int j = 0; j < 16; j++) x ^= d[j];
-        acc[0] = __uint_as_float(__float_as_uint(acc[0]) ^ x);
-        return;
-    }
     const float2 xs2 = make_float2(xs, xs);
 #pragma unroll
     for (int j4 = 0; j4 < 4; j4++) {
         const float4 w = lds128f(ws_saddr + 16 * j4);
-        if (EXACT_) {
+        if (EXACT) {
             acc[4 * j4 + 0] = __fadd_rn(acc[4 * j4 + 0], __fmul_rn(__fmul_rn((float)(int)d[4 * j4 + 0], w.x), xs));
             acc[4 * j4 + 1] = __fadd_rn(acc[4 * j4 + 1], __fmul_rn(__fmul_rn((float)(int)d[4 * j4 + 1], w.y), xs));
             acc[4 * j4 + 2] = __fadd_rn(acc[4 * j4 + 2], __fmul_rn(__fmul_rn((float)(int)d[4 * j4 + 2], w.z), xs));
@@ -192,42 +169,24 @@ __device__ __forceinline__ void sts128f(uint32_t saddr, float4 v) {
 // MMA warp as soon as its second chunk has landed in registers (group 0 two scaling blocks before group 1).
 // ws0 / xsa: shared addresses of this thread's 32 weight scales / its token scale for the pair's first group (the second group's
 // follow 512 B later).  tempty_bar: the slot's two "drained" barriers (group 0, group 1).
-template <int VAR>
+template <bool EXACT>
 __device__ __forceinline__ void pf_drain_pair(float (&acc)[PF_COLS], uint32_t (&d0)[16], uint32_t (&d1)[16], uint32_t taddr, uint32_t ws0, uint32_t xsa,
                                               uint32_t tempty_bar, int lane, uint32_t nxt_taddr, uint32_t nxt_bar, uint32_t nxt_parity) {
-    if (VAR >= 4) { // timing experiments: 4 = the hand-shake alone; 5 = the arithmetic on whatever the chunk registers hold (no TMEM read)
-        if (VAR == 5) {
-            const float xs = lds_f32(xsa), xsb = lds_f32(xsa + 512);
-            pf_scale16<0>(acc, d0, ws0, xs);
-            pf_scale16<0>(acc + 16, d1, ws0 + 64, xs);
-            pf_scale16<0>(acc, d0, ws0 + 512, xsb);
-            pf_scale16<0>(acc + 16, d1, ws0 + 512 + 64, xsb);
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) {
-            pf_arrive(tempty_bar);
-            pf_arrive(tempty_bar + 8);
-        }
-        pf_wait(nxt_bar, nxt_parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        return;
-    }
     const float xs = lds_f32(xsa);
     pf_wait_ld(); // d0 = group 0, columns 0..15
     PF_LD16(d1, taddr + 16);
-    pf_scale16<VAR>(acc, d0, ws0, xs);
+    pf_scale16<EXACT>(acc, d0, ws0, xs);
     pf_wait_ld();
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncwarp();
     if (lane == 0) pf_arrive(tempty_bar); // group 0 of the pair is in registers: its accumulator may be refilled already
     PF_LD16(d0, taddr + PF_BN);
     const float xsb = lds_f32(xsa + 512);
-    pf_scale16<VAR>(acc + 16, d1, ws0 + 64, xs);
+    pf_scale16<EXACT>(acc + 16, d1, ws0 + 64, xs);
     pf_wait_ld();
     PF_LD16(d1, taddr + PF_BN + 16);
     const uint32_t nxt_ok = pf_try(nxt_bar, nxt_parity); // asked now, looked at after the scaling block below
-    pf_scale16<VAR>(acc, d0, ws0 + 512, xsb);
+    pf_scale16<EXACT>(acc, d0, ws0 + 512, xsb);
     pf_wait_ld();
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncwarp();
@@ -235,24 +194,19 @@ __device__ __forceinline__ void pf_drain_pair(float (&acc)[PF_COLS], uint32_t (&
     if (!nxt_ok) pf_wait(nxt_bar, nxt_parity);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     PF_LD16(d0, nxt_taddr); // first chunk of the next pair: in flight while the last chunk of this one is scaled
-    pf_scale16<VAR>(acc + 16, d1, ws0 + 512 + 64, xsb);
+    pf_scale16<EXACT>(acc + 16, d1, ws0 + 512 + 64, xsb);
 }
 
-// MODE: 0 = fast drain (what q3_prefill runs): the same exact int32 group dots, folded with packed f32x2 FMAs.
-//       1 = EXACT: every output is the reference's left fold of unfused (dot * ws) * xs terms -- bit-identical to `matmul`
-//           (the operator-level proof).
-//       2 = dense ceiling (timing experiment only: the group structure is ignored, all of K is accumulated in ONE TMEM
-//           buffer and drained once per tile -- what this tiling / pipeline reaches as a plain int8 GEMM; the output is the raw
-//           integer dot converted to f32).
-//       3 / 4 / 5 = timing experiments on the grouped pipeline (outputs are garbage): 3 = every group accumulator is read out
-//           of TMEM but not scaled; 4 = the accumulator hand-shake alone, no TMEM read; 5 = the scaling arithmetic without TMEM reads.
+// EXACT = false: the fast drain (what q3_prefill runs): the exact int32 group dots, folded with packed f32x2 FMAs.
+// EXACT = true: every output is the reference's left fold of unfused (dot * ws) * xs terms -- bit-identical to `matmul`
+//               (the operator-level proof).
 // K / GS must be even (checked by the host): the unit of hand-over between the MMA warp and the epilogue is a PAIR of group
 // accumulators (2 x 128 TMEM columns; two pair slots fill the 512 columns), and a scale-ring slot holds the rows of one pair.
 // PERSISTENT: grid = min(tiles, SMs); a CTA walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... (token tile fastest, so the
 // CTAs running together share weight tiles in L2).  The TMA and MMA warps run straight on into the next tile (stage ring,
 // accumulator pairs and scale ring keep their running indices), so a tile's output store and the pipeline refill overlap
 // and TMEM is allocated once per SM instead of once per tile.
-template <int GS, int EPI, int MODE>
+template <int GS, int EPI, bool EXACT>
 __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedulers host 5 warps (16384 / (5 x 32) = 102; 112 does not launch)
     k_gemm_q8(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_xs,
               const __grid_constant__ CUtensorMap map_ws, const PrefillGemmArgs a) {
@@ -264,8 +218,7 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
     const int nkb = a.K / PF_BK;
     constexpr int GPS = PF_BK / GS; // groups per stage
     constexpr int KPG = GS / 32;    // MMA K-steps per group
-    const int ng = a.K / GS, npair = ng >> 1;
-    constexpr bool DENSE = MODE == 2;
+    const int npair = (a.K / GS) >> 1; // accumulator pairs per tile
     static_assert(PF_NACC == 4 && PF_SG == 2 && (PF_SRING & (PF_SRING - 1)) == 0, "pairs");
 
     if (threadIdx.x == 0) {
@@ -318,21 +271,19 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
         // across tile boundaries), independent of the tile producer.  History: as eight 512-byte bulk copies per stage issued by the
         // tile producer from a divergent single-lane branch, the scale traffic -- not the tensor pipe, not the epilogue -- set the
         // pace of the whole kernel (8B gate/up: 650 us; the same kernel with the scale traffic switched off: 457 us).
-        if (!DENSE) {
-            int sc = 0; // running pair count
-            for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x) {
-                const int m0 = (tile % mt) * PF_BM, n0 = (tile / mt) * PF_BN;
-                for (int c = 0; c < npair; c++, sc++) {
-                    const int sl = sc & (PF_SRING - 1);
-                    pf_wait(sb + PF_BAR_SEMPTY + 8 * sl, ((sc / PF_SRING) & 1) ^ 1);
-                    if (pf_elect()) {
-                        uint64_t *bar = reinterpret_cast<uint64_t *>(smem + PF_BAR_SFULL) + sl;
-                        mbar_expect_tx(bar, 2048);
-                        tma_load_2d(smem + PF_OFF_SCALE + sl * 2048, &map_ws, n0, 2 * c, bar);
-                        tma_load_2d(smem + PF_OFF_SCALE + sl * 2048 + 1024, &map_xs, m0, 2 * c, bar);
-                    }
-                    __syncwarp();
+        int sc = 0; // running pair count
+        for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x) {
+            const int m0 = (tile % mt) * PF_BM, n0 = (tile / mt) * PF_BN;
+            for (int c = 0; c < npair; c++, sc++) {
+                const int sl = sc & (PF_SRING - 1);
+                pf_wait(sb + PF_BAR_SEMPTY + 8 * sl, ((sc / PF_SRING) & 1) ^ 1);
+                if (pf_elect()) {
+                    uint64_t *bar = reinterpret_cast<uint64_t *>(smem + PF_BAR_SFULL) + sl;
+                    mbar_expect_tx(bar, 2048);
+                    tma_load_2d(smem + PF_OFF_SCALE + sl * 2048, &map_ws, n0, 2 * c, bar);
+                    tma_load_2d(smem + PF_OFF_SCALE + sl * 2048 + 1024, &map_xs, m0, 2 * c, bar);
                 }
+                __syncwarp();
             }
         }
     } else if (warp == PF_MMA_WARP) {
@@ -340,9 +291,9 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
         // instruction descriptor: D = S32, A = B = signed int8, both K-major, N = 128, M = 128
         constexpr uint32_t IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((PF_BN >> 3) << 17) | ((PF_BM >> 4) << 24);
         uint64_t *tfull = reinterpret_cast<uint64_t *>(smem + PF_BAR_TFULL), *empty = reinterpret_cast<uint64_t *>(smem + PF_BAR_EMPTY);
-        int kbt = 0, pt = 0, titer = 0; // running stage uses, accumulator-pair uses, tiles
+        int kbt = 0, pt = 0; // running stage uses, accumulator-pair uses
         const uint64_t desc_a0 = umma_desc_k_sw128(sb + PF_OFF_A), desc_b0 = umma_desc_k_sw128(sb + PF_OFF_B);
-        for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x, titer++) {
+        for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x) {
             int gi = 0;
             for (int kb = 0; kb < nkb; kb++, kbt++) {
                 const int s = kbt % PF_STAGES;
@@ -353,45 +304,28 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
 #pragma unroll
                 for (int gg = 0; gg < GPS; gg++, gi++) {
                     const int ps = pt & 1;
-                    uint32_t col;
-                    if (DENSE) {
-                        col = 0;
-                        if (gi == 0) { // the previous tile's accumulator has been read out
-                            pf_wait(sb + PF_BAR_TEMPTY, (titer & 1) ^ 1);
-                            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        }
-                    } else { // each group accumulator of a pair is handed back on its own: the first one two scaling blocks earlier
-                        col = ps * 2 * PF_BN + (gi & 1) * PF_BN;
-                        pf_wait(sb + PF_BAR_TEMPTY + 8 * (2 * ps + (gi & 1)), ((pt >> 1) & 1) ^ 1);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        if (lane == 0 && (gi & 1) == 0) PF_STAMP(0, pt);
-                    }
+                    // each group accumulator of a pair is handed back on its own: the first one two scaling blocks earlier
+                    const uint32_t col = ps * 2 * PF_BN + (gi & 1) * PF_BN;
+                    pf_wait(sb + PF_BAR_TEMPTY + 8 * (2 * ps + (gi & 1)), ((pt >> 1) & 1) ^ 1);
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     if (pf_elect()) {
 #pragma unroll
                         for (int kk = 0; kk < KPG; kk++) {
                             const uint32_t koff = (gg * GS + kk * 32) >> 4; // along K inside the 128 B swizzle span, in 16-byte units
-                            umma_i8(tmem_base + col, da + koff, db + koff, IDESC, kk > 0 || (DENSE && gi > 0));
+                            umma_i8(tmem_base + col, da + koff, db + koff, IDESC, kk > 0);
                         }
-                        if (DENSE) {
-                            if (gi == ng - 1) umma_commit(&tfull[0]);
-                        } else if (gi & 1) { // pair complete -> epilogue
-                            umma_commit(&tfull[ps]);
-                        }
+                        if (gi & 1) umma_commit(&tfull[ps]); // pair complete -> epilogue
                     }
                     __syncwarp();
-                    if (!DENSE && (gi & 1)) {
-                        if (lane == 0) PF_STAMP(1, pt);
-                        pt++;
-                    }
+                    if (gi & 1) pt++;
                 }
                 if (pf_elect()) umma_commit(&empty[s]); // all MMAs reading this stage retired -> TMA may refill it
                 __syncwarp();
             }
         }
-        if (!DENSE) { // one empty pair: the epilogue's last look-ahead waits for it (and reads an accumulator nobody uses)
-            if (pf_elect()) umma_commit(&tfull[pt & 1]);
-            __syncwarp();
-        }
+        // one empty pair: the epilogue's last look-ahead waits for it (and reads an accumulator nobody uses)
+        if (pf_elect()) umma_commit(&tfull[pt & 1]);
+        __syncwarp();
     } else if (warp < PF_EPI_WARPS) {
         // ------------------------------- epilogue -------------------------------
         const int quad = warp & 3;  // TMEM lanes [32*quad, 32*quad+32) are the only ones this warp may read
@@ -399,48 +333,27 @@ __global__ void __launch_bounds__(PF_THREADS, 1) // 96 registers: three schedule
         const uint32_t tq = tmem_base + ((uint32_t)(quad * 32) << 16) + part * PF_COLS;
         const uint32_t wsx = sb + PF_OFF_SCALE + part * (PF_COLS * 4);                 // this thread's weight scales in scale slot 0, row 0
         const uint32_t xsx = sb + PF_OFF_SCALE + 1024 + (quad * 32 + lane) * 4;        // its token scale (slot: ws g0 | ws g1 | xs g0 | xs g1)
-        int pt = 0, titer = 0;      // running pair count (pair slot = pt & 1, scale slot = pt & (PF_SRING - 1)), tiles
+        int pt = 0;                 // running pair count (pair slot = pt & 1, scale slot = pt & (PF_SRING - 1))
         uint32_t d0[16], d1[16];    // the two chunk buffers of the TMEM read stream (live across pairs and tiles)
-        if (MODE == 5) {
-#pragma unroll
-            for (int j = 0; j < 16; j++) d0[j] = d1[j] = threadIdx.x + j;
-        }
         uint32_t s_ok = 0;          // the scale rows of the pair about to start are known to have landed (asked ahead of time)
-        if (!DENSE) {               // the very first pair of this CTA: nobody has requested its first chunk yet
-            pf_wait(sb + PF_BAR_TFULL, 0);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if (MODE < 4) PF_LD16(d0, tq);
-        }
-        for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x, titer++) {
+        // the very first pair of this CTA: nobody has requested its first chunk yet
+        pf_wait(sb + PF_BAR_TFULL, 0);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        PF_LD16(d0, tq);
+        for (int tile = blockIdx.x; tile < ntile; tile += gridDim.x) {
             float acc[PF_COLS];
 #pragma unroll
             for (int j = 0; j < PF_COLS; j++) acc[j] = 0.0f;
-            if (DENSE) {
-                pf_wait(sb + PF_BAR_TFULL, titer & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                PF_LD16(d0, tq);
-                PF_LD16(d1, tq + 16);
-                pf_wait_ld();
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                __syncwarp();
-                if (lane == 0) pf_arrive(sb + PF_BAR_TEMPTY);
-#pragma unroll
-                for (int j = 0; j < 16; j++) {
-                    acc[j] = (float)(int)d0[j];
-                    acc[16 + j] = (float)(int)d1[j];
-                }
-            } else {
 #pragma unroll 1
-                for (int c = 0; c < npair; c++, pt++) {
-                    const uint32_t ps = pt & 1, sl = pt & (PF_SRING - 1);
-                    if (!s_ok) pf_wait(sb + PF_BAR_SFULL + 8 * sl, (pt / PF_SRING) & 1); // the pair's scale rows landed
-                    // the next pair's scale rows: asked for here, looked at when they are needed (never, after the very last pair)
-                    s_ok = pf_try(sb + PF_BAR_SFULL + 8 * ((pt + 1) & (PF_SRING - 1)), ((pt + 1) / PF_SRING) & 1);
-                    pf_drain_pair<MODE>(acc, d0, d1, tq + ps * (2 * PF_BN), wsx + sl * 2048, xsx + sl * 2048, sb + PF_BAR_TEMPTY + 16 * ps, lane,
-                                        tq + (ps ^ 1) * (2 * PF_BN), sb + PF_BAR_TFULL + 8 * (ps ^ 1), ((pt + 1) >> 1) & 1);
-                    __syncwarp();
-                    if (lane == 0) pf_arrive(sb + PF_BAR_SEMPTY + 8 * sl); // scale rows consumed
-                }
+            for (int c = 0; c < npair; c++, pt++) {
+                const uint32_t ps = pt & 1, sl = pt & (PF_SRING - 1);
+                if (!s_ok) pf_wait(sb + PF_BAR_SFULL + 8 * sl, (pt / PF_SRING) & 1); // the pair's scale rows landed
+                // the next pair's scale rows: asked for here, looked at when they are needed (never, after the very last pair)
+                s_ok = pf_try(sb + PF_BAR_SFULL + 8 * ((pt + 1) & (PF_SRING - 1)), ((pt + 1) / PF_SRING) & 1);
+                pf_drain_pair<EXACT>(acc, d0, d1, tq + ps * (2 * PF_BN), wsx + sl * 2048, xsx + sl * 2048, sb + PF_BAR_TEMPTY + 16 * ps, lane,
+                                     tq + (ps ^ 1) * (2 * PF_BN), sb + PF_BAR_TFULL + 8 * (ps ^ 1), ((pt + 1) >> 1) & 1);
+                __syncwarp();
+                if (lane == 0) pf_arrive(sb + PF_BAR_SEMPTY + 8 * sl); // scale rows consumed
             }
             // ---- write the tile out ----
             // A thread owns a token ROW (TMEM lane) and 32 consecutive columns, so direct stores would touch 32 different cache

@@ -420,7 +420,7 @@ def op_prefill_attention(q, k, v, pos0: int, n_heads: int, n_kv: int, device: in
 
 
 def bench_gemm_q8(T: int, N: int, K: int, gs: int = 64, mode: int = 0, reps: int = 5, device: int = 0) -> float:
-    """Milliseconds per launch of the tcgen05 GEMM alone (mode 0 fast drain, 1 exact drain, 2 dense int8 ceiling)."""
+    """Milliseconds per launch of the tcgen05 GEMM alone (mode 0 fast drain, 1 exact drain)."""
     ms = C.c_float(0)
     _check(load_library().q3_bench_gemm_q8(device, T, N, K, gs, mode, reps, C.byref(ms)))
     return ms.value

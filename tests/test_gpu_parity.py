@@ -536,6 +536,20 @@ def test_tensor_core_gemm_bit_identical_to_reference_matmul(T, N, K, gs):
     assert np.abs(fast - ref).max() <= 2e-6 * scale * np.sqrt(K / gs)
 
 
+def test_tensor_core_gemm_rejects_unknown_modes():
+    """The GEMM has two drains, fast (0) and exact (1); any other mode is an argument error, not a different computation."""
+    T, N, K, gs = 128, 128, 128, 64
+    xq, wq = np.zeros((T, K), np.int8), np.zeros(N * K, np.int8)
+    xs, ws = np.ones((T, K // gs), np.float32), np.ones(N * K // gs, np.float32)
+    for mode in (2, 5, -1):
+        with pytest.raises(T_mod.Q3Error) as e:
+            T_mod.op_gemm_q8(xq, xs, wq, ws, T, N, K, gs, exact=mode)
+        assert e.value.code == -1  # Q3_EINVAL
+        with pytest.raises(T_mod.Q3Error) as e:
+            T_mod.bench_gemm_q8(T, N, K, gs, mode, 1)
+        assert e.value.code == -1
+
+
 @pytest.mark.parametrize("name,gs,seed,T", [("tiny-untied", 64, 1, 37), ("small", 128, 2, 130), ("tiny", 64, 0, 5)])
 def test_prefill_matches_sequential_forwards(models, name, gs, seed, T):
     """q3_prefill (batched tensor-core path) leaves the KV cache and the last-token logits as T sequential
