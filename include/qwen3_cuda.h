@@ -121,6 +121,20 @@ int q3_prefill(q3_handle *h, const int *tokens, int n, int pos0, float *last_log
  * launch stream, inputs resident; milliseconds. */
 int q3_bench_prefill(q3_handle *h, const int *tokens, int n, int pos0, float *ms_out);
 
+/* Extension: score n tokens at positions pos0..pos0+n-1 in one batched pass.
+ * Leaves the KV cache exactly as q3_prefill(h, tokens, n, pos0, NULL) does.
+ * For every i in [0, n), with logits_i = the logits after tokens[0..i] at position pos0+i:
+ *   logprobs_out[i] = log softmax(logits_i)[targets[i]]   (natural log, f32; targets: n ids, required iff logprobs_out)
+ *   argmax_out[i]   = argmax(logits_i), last index among equal maxima (sampler.rs:57-59, as q3_forward_argmax)
+ * At least one of logprobs_out / argmax_out must be non-NULL.  q3_logits_device() is unspecified afterwards.
+ * A target is scored at its own position, so a long text can be scored in pieces: the target of a piece's last position is
+ * the first token of the next piece.  Every argument is checked before any device work (Q3_EINVAL; Q3_ECOMM for an
+ * unconnected tensor-parallel handle): on an error nothing is written.  Fast mode runs the batched prefill, then the final
+ * norm, the lm_head on the tensor cores and the reduction on every row; exact mode (or a shape without the batched path)
+ * runs n q3_forward steps and reduces the reference's own logits.  Under tensor parallelism every rank runs the full lm_head
+ * and returns the full results; there the batched path is required (Q3_EUNSUPPORTED otherwise). */
+int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out);
+
 /* Zero the KV cache (a freshly built reference transformer, qwen3.rs:439-440). */
 int q3_reset(q3_handle *h);
 
@@ -217,6 +231,8 @@ int q3_bench_gemm_q8(int device, int T, int N, int K, int gs, int mode, int reps
  * *rng_state is Sampler::rng_state before the call and after it. */
 int q3_op_sample(int device, const float *logits, int n, float temperature, float topp, unsigned long long *rng_state,
                  int *token_out);
+/* The reduction q3_score runs, on host-supplied logits [rows][n] (operator-level parity tests). */
+int q3_op_logprobs(int device, const float *logits, int rows, int n, const int *targets, float *logprobs_out, int *argmax_out);
 /* layers.rs:109-119 RMSNorm::forward */
 int q3_op_rmsnorm(int device, const float *x, const float *w, int n, float *out);
 /* qwen3-export model_exporter.rs:104-161 quantize_q80 on the device (SURVEY.md §8f-3). */

@@ -17,7 +17,7 @@
 //   tokenizer.rs          Tokenizer (byte-level BPE)         qwen3::Tokenizer (same results; vocabulary lookups hashed)
 //   generation.rs:188-195 render_prompt                      qwen3::render_prompt
 //
-// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill.
+// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill, score.
 //
 // Errors: construction failures throw qwen3::Error (the reference returns anyhow::Error with the same
 // message text); forward() with an out-of-range token / pos throws (the reference panics on the slice
@@ -38,6 +38,7 @@
 #include <stdexcept>
 #include <string>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "qwen3_cuda.h"
@@ -116,6 +117,16 @@ public:
     const std::vector<float> &prefill(const std::vector<int> &tokens, size_t pos0) {
         detail::check(q3_prefill(h_, tokens.data(), (int)tokens.size(), (int)pos0, logits_.data()));
         return logits_;
+    }
+    // q3_score: tokens at positions pos0.. in one batched pass -> (log-probability of targets[i] after tokens[0..i], greedy
+    // argmax there).  Empty targets: no log-probabilities (first vector empty).  Cache as after prefill(tokens, pos0).
+    std::pair<std::vector<float>, std::vector<int>> score(const std::vector<int> &tokens, const std::vector<int> &targets, size_t pos0) {
+        if (!targets.empty() && targets.size() != tokens.size()) throw std::invalid_argument("score: targets and tokens differ in length");
+        std::vector<float> lp(targets.size());
+        std::vector<int> am(tokens.size());
+        detail::check(q3_score(h_, tokens.data(), (int)tokens.size(), (int)pos0, targets.empty() ? nullptr : targets.data(),
+                               targets.empty() ? nullptr : lp.data(), am.data()));
+        return {std::move(lp), std::move(am)};
     }
     void reset() { detail::check(q3_reset(h_)); } // zero the KV cache
     q3_handle *handle() { return h_; }

@@ -134,6 +134,12 @@ struct q3_handle {
     float *pf_x = nullptr, *pf_q = nullptr, *pf_att = nullptr, *pf_hb = nullptr, *pf_xsT = nullptr, *pf_hsT = nullptr;
     int8_t *pf_xq = nullptr, *pf_hq = nullptr;
     int *pf_tokens = nullptr;
+    // q3_score, allocated on its first call: per-position targets / results [seq_len], the lm_head rows of one chunk
+    // [sc_cap][vocab] f32 (grow-only, freed in q3_destroy)
+    int *sc_targets = nullptr, *sc_argmax = nullptr;
+    float *sc_lp = nullptr, *sc_logits = nullptr;
+    int sc_cap = 0;
+    bool sc_want_lp = false; // this call asked for log-probabilities (targets uploaded)
     // device sampler (sampler.rs on the device, q3_sampler.cuh)
     float samp_temperature = 0.0f, samp_topp = 0.9f;
     unsigned long long *d_rng = nullptr, *d_keys = nullptr;
@@ -936,11 +942,15 @@ static int prefill_tp_rowparallel(q3_handle *h, int which, const CUtensorMap &mx
 }
 
 static int prefill_run(q3_handle *h, const int *tokens_host, int T, int pos0);
-// prompts longer than the tensor-parallel partial blocks go through in chunks (causal attention reads the earlier chunks' cache rows)
-static int prefill_chunks(q3_handle *h, const int *tokens_host, int n, int pos0) {
+static int score_rows(q3_handle *h, int T, int out0);
+// prompts longer than the tensor-parallel partial blocks go through in chunks (causal attention reads the earlier chunks' cache rows).
+// score: q3_score's head stage on each chunk's rows of pf_x, before the next chunk overwrites them.
+static int prefill_chunks(q3_handle *h, const int *tokens_host, int n, int pos0, bool score = false) {
     const int cap = h->tp_size > 1 ? h->pf_tp_cap : n;
     for (int off = 0; off < n; off += cap) {
-        int rc = prefill_run(h, tokens_host + off, n - off < cap ? n - off : cap, pos0 + off);
+        const int T = n - off < cap ? n - off : cap;
+        int rc = prefill_run(h, tokens_host + off, T, pos0 + off);
+        if (!rc && score) rc = score_rows(h, T, off);
         if (rc) return rc;
     }
     return 0;
@@ -1023,6 +1033,73 @@ static int prefill_run(q3_handle *h, const int *tokens_host, int T, int pos0) {
         } else if ((rc = prefill_tp_rowparallel(h, 1, mx_h, W.w2.map, dn, T))) return rc;
     }
     CK(cudaMemcpyAsync(h->x, h->pf_x + (size_t)(T - 1) * dim, (size_t)dim * 4, cudaMemcpyDeviceToDevice, s));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------
+// q3_score: final norm + lm_head + log-softmax / argmax on every row of the batched prefill
+// ------------------------------------------------------------------------------------------
+// lm_head rows per GEMM: a [T][vocab] f32 block would be 1.24 GB at T 2048 (151936 entries), so the head runs in row chunks
+constexpr int SCORE_ROWS = 512;
+
+// the per-position buffers [seq_len]; with lm_head: also the lm_head's group-major scales / TMA map and room for `rows` logits
+// rows.  Grow-only; nothing is allocated before the first q3_score.
+static int score_reserve(q3_handle *h, bool lm_head, int rows) {
+    const q3_config &c = h->cfg;
+    int rc;
+    if (!h->sc_targets) { // one allocation: a failure leaves all three unset
+        int *p = nullptr;
+        if ((rc = dmalloc(h, (void **)&p, (size_t)c.seq_len * 12))) return rc;
+        h->sc_targets = p;
+        h->sc_argmax = p + c.seq_len;
+        h->sc_lp = (float *)(p + 2 * (size_t)c.seq_len);
+    }
+    if (!lm_head) return 0;
+    if ((rc = prefill_prepare_tensor(h, h->wcls))) return rc; // tied: sets sT / map on the copy in wcls only, freed once with allocs
+    rows = (rows + 127) / 128 * 128;
+    if (rows > SCORE_ROWS) rows = SCORE_ROWS;
+    if (rows <= h->sc_cap) return 0;
+    if (h->sc_logits) cudaFree(h->sc_logits);
+    h->sc_logits = nullptr;
+    h->sc_cap = 0;
+    cudaError_t e = cudaMalloc((void **)&h->sc_logits, (size_t)rows * c.vocab_size * 4);
+    if (e != cudaSuccess) {
+        h->sc_logits = nullptr;
+        cudaGetLastError();
+        return fail(Q3_ECUDA, "score logits buffer for %d rows: %s", rows, cudaGetErrorString(e));
+    }
+    h->sc_cap = rows;
+    return 0;
+}
+
+static void launch_logprobs(q3_handle *h, const float *logits, int rows, int out0) {
+    k_logprobs<<<rows, LP_THREADS, 0, h->stream>>>(logits, h->cfg.vocab_size, (size_t)h->cfg.vocab_size, h->sc_targets + out0,
+                                                  h->sc_want_lp ? h->sc_lp + out0 : nullptr, h->sc_argmax + out0);
+}
+
+// rows [0, T) of pf_x (positions out0 .. out0 + T - 1 of the q3_score call): final RMSNorm + quantise into rows [0, Tc) of
+// pf_xq / pf_xsT (pf_x is read only), the lm_head on the fast-drain tensor-core GEMM, then k_logprobs -- SCORE_ROWS rows at a time
+static int score_rows(q3_handle *h, int T, int out0) {
+    const q3_config &c = h->cfg;
+    const int gs = c.group_size, dim = c.dim;
+    cudaStream_t s = h->stream;
+    int rc;
+    for (int r0 = 0; r0 < T; r0 += SCORE_ROWS) {
+        const int Tc = T - r0 < SCORE_ROWS ? T - r0 : SCORE_ROWS, Tcpad = (Tc + 127) / 128 * 128;
+        float *x = h->pf_x + (size_t)r0 * dim;
+        if (dim <= 4096) {
+            GS_DISPATCH(gs, (k_pf_norm_quant<GS, 4><<<Tc, 256, 0, s>>>(x, h->rms_final, h->pf_xq, h->pf_xsT, dim, Tcpad, nullptr, nullptr, nullptr, 0)));
+        } else {
+            GS_DISPATCH(gs, (k_pf_norm_quant<GS><<<Tc, 256, 0, s>>>(x, h->rms_final, h->pf_xq, h->pf_xsT, dim, Tcpad, nullptr, nullptr, nullptr, 0)));
+        }
+        CUtensorMap mx;
+        if ((rc = make_map_i8(&mx, h->pf_xq, Tcpad, dim))) return rc;
+        PrefillGemmArgs g{};
+        g.T = Tc; g.Tpad = Tcpad; g.K = dim; g.N = c.vocab_size; g.wsT = h->wcls.sT; g.xsT = h->pf_xsT; g.out = h->sc_logits; g.ld_out = c.vocab_size;
+        if ((rc = launch_gemm_q8<PF_EPI_STORE>(gs, mx, h->wcls.map, g, s))) return rc;
+        launch_logprobs(h, h->sc_logits, Tc, out0 + r0);
+    }
     CK(cudaGetLastError());
     return 0;
 }
@@ -1288,6 +1365,7 @@ extern "C" void q3_destroy(q3_handle *h) {
         if (h->g_greedy[e]) cudaGraphExecDestroy(h->g_greedy[e]);
     }
     prefill_release(h);
+    if (h->sc_logits) cudaFree(h->sc_logits);
     for (void *p : h->peer_maps) cudaIpcCloseMemHandle(p);
     for (void *p : h->allocs) cudaFree(p);
     if (h->h_logits) cudaFreeHost(h->h_logits);
@@ -1666,6 +1744,42 @@ extern "C" int q3_bench_prefill(q3_handle *h, const int *tokens, int n, int pos0
     return h->tp_size > 1 ? mega_check(h) : Q3_OK;
 }
 
+extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out) {
+    if (!h || !tokens || n <= 0) return fail(Q3_EINVAL, "bad score arguments");
+    if (pos0 < 0 || (long long)pos0 + n > h->cfg.seq_len)
+        return fail(Q3_EINVAL, "index out of bounds: pos0 + n = %lld > seq_len %d", (long long)pos0 + n, h->cfg.seq_len);
+    if (!logprobs_out && !argmax_out) return fail(Q3_EINVAL, "q3_score needs logprobs_out or argmax_out");
+    if (logprobs_out && !targets) return fail(Q3_EINVAL, "logprobs_out needs targets");
+    const int V = h->cfg.vocab_size;
+    for (int i = 0; i < n; i++) {
+        if (tokens[i] < 0 || tokens[i] >= V) return fail(Q3_EINVAL, "index out of bounds: token %d", tokens[i]);
+        if (logprobs_out && (targets[i] < 0 || targets[i] >= V)) return fail(Q3_EINVAL, "index out of bounds: target %d", targets[i]);
+    }
+    if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
+    const bool batched = h->pf_ok && !h->exact && V % 128 == 0;
+    // Under TP, q3_forward leaves only this rank's vocabulary shard in h->logits (all of it only on the logits root, if one is set)
+    if (h->tp_size > 1 && !batched) return fail(Q3_EUNSUPPORTED, "q3_score under tensor parallelism needs the batched prefill path");
+    CK(cudaSetDevice(h->device));
+    int rc;
+    if ((rc = score_reserve(h, batched, n))) return rc;
+    h->sc_want_lp = logprobs_out != nullptr;
+    if (logprobs_out) CK(cudaMemcpyAsync(h->sc_targets, targets, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+    if (batched) {
+        if ((rc = prefill_chunks(h, tokens, n, pos0, true))) return rc;
+    } else {
+        // sequential decode steps (exact mode: the logits are the reference's bit for bit), reduced one at a time
+        for (int i = 0; i < n; i++) {
+            if ((rc = q3_forward(h, tokens[i], pos0 + i, nullptr))) return rc;
+            launch_logprobs(h, h->logits, 1, i);
+        }
+    }
+    if (logprobs_out) CK(cudaMemcpyAsync(logprobs_out, h->sc_lp, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (argmax_out) CK(cudaMemcpyAsync(argmax_out, h->sc_argmax, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaGetLastError());
+    return mega_check(h);
+}
+
 extern "C" int q3_reset(q3_handle *h) {
     if (!h) return fail(Q3_EINVAL, "null handle");
     CK(cudaSetDevice(h->device));
@@ -1869,6 +1983,29 @@ extern "C" int q3_op_sample(int device, const float *logits, int n, float temper
     CK(cudaGetLastError());
     CK(cudaMemcpy(rng_state, dr.p, 8, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(token_out, dt.p, 4, cudaMemcpyDeviceToHost));
+    return Q3_OK;
+}
+
+// q3_score's reduction on host-supplied logits [rows][n]: log-softmax at targets[r] and the last argmax of every row
+extern "C" int q3_op_logprobs(int device, const float *logits, int rows, int n, const int *targets, float *logprobs_out, int *argmax_out) {
+    if (!logits || rows <= 0 || n <= 0) return fail(Q3_EINVAL, "bad logprobs arguments");
+    if (!logprobs_out && !argmax_out) return fail(Q3_EINVAL, "q3_op_logprobs needs logprobs_out or argmax_out");
+    if (logprobs_out && !targets) return fail(Q3_EINVAL, "logprobs_out needs targets");
+    if (logprobs_out)
+        for (int r = 0; r < rows; r++)
+            if (targets[r] < 0 || targets[r] >= n) return fail(Q3_EINVAL, "index out of bounds: target %d (n %d)", targets[r], n);
+    CK(cudaSetDevice(device));
+    DevBuf dl, dt, dlp, dam;
+    int rc;
+    if ((rc = dl.alloc((size_t)rows * n * 4)) || (rc = dt.alloc((size_t)rows * 4)) || (rc = dlp.alloc((size_t)rows * 4)) ||
+        (rc = dam.alloc((size_t)rows * 4)))
+        return rc;
+    CK(cudaMemcpy(dl.p, logits, (size_t)rows * n * 4, cudaMemcpyHostToDevice));
+    if (logprobs_out) CK(cudaMemcpy(dt.p, targets, (size_t)rows * 4, cudaMemcpyHostToDevice));
+    k_logprobs<<<rows, LP_THREADS>>>(dl.as<float>(), n, (size_t)n, dt.as<int>(), logprobs_out ? dlp.as<float>() : nullptr, dam.as<int>());
+    CK(cudaGetLastError());
+    if (logprobs_out) CK(cudaMemcpy(logprobs_out, dlp.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
+    if (argmax_out) CK(cudaMemcpy(argmax_out, dam.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
     return Q3_OK;
 }
 

@@ -705,6 +705,82 @@ __global__ void __launch_bounds__(1024) k_argmax(const float *__restrict__ logit
 }
 
 // ------------------------------------------------------------------------------------------
+// Per-row log-softmax at a target index + greedy argmax (q3_score, q3_op_logprobs).  One CTA per row of `logits`
+// (row pitch ld floats), one streaming pass: each thread keeps the running max m (the value of its argmax key),
+// sum s of expf(x - m) rescaled when m grows, and the key of its last maximum -- the total-order key of k_argmax, so
+// the index is the reference's (sampler.rs:57-59: last index among equal maxima).  The per-thread partials are
+// combined over a fixed shuffle / shared-memory tree, so the result depends on the row's values and LP_THREADS only:
+// the same logits give the same bits however many rows are launched.  lp = (x[target] - m) - logf(s).
+// ------------------------------------------------------------------------------------------
+constexpr int LP_THREADS = 512;
+constexpr int LP_BATCH = 8; // loads issued per thread before they are folded (in index order)
+
+struct LpPart {
+    long long key; // (total_key(max) << 32) | index
+    float m, s;
+};
+// (a, b) -> a; commutative, so both lanes of a shuffle pair hold the same value
+__device__ __forceinline__ void lp_combine(LpPart &a, const LpPart &b) {
+    if (b.key > a.key) {
+        a.s = b.s + (a.s == 0.0f ? 0.0f : a.s * expf(a.m - b.m));
+        a.m = b.m;
+        a.key = b.key;
+    } else {
+        a.s = a.s + (b.s == 0.0f ? 0.0f : b.s * expf(b.m - a.m));
+    }
+}
+__device__ __forceinline__ LpPart lp_shfl(const LpPart &p, int o) {
+    LpPart q;
+    q.key = __shfl_xor_sync(0xffffffffu, p.key, o);
+    q.m = __shfl_xor_sync(0xffffffffu, p.m, o);
+    q.s = __shfl_xor_sync(0xffffffffu, p.s, o);
+    return q;
+}
+
+__global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict__ logits, int n, size_t ld,
+                                                         const int *__restrict__ targets, float *lp_out, int *argmax_out) {
+    __shared__ LpPart red[LP_THREADS / 32];
+    const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *x = logits + (size_t)row * ld;
+    LpPart p{(long long)0x8000000000000000LL, -INFINITY, 0.0f};
+    for (int base = tid; base < n; base += LP_BATCH * LP_THREADS) {
+        float v[LP_BATCH];
+#pragma unroll
+        for (int k = 0; k < LP_BATCH; k++) {
+            const int i = base + k * LP_THREADS;
+            v[k] = i < n ? x[i] : 0.0f;
+        }
+#pragma unroll
+        for (int k = 0; k < LP_BATCH; k++) {
+            const int i = base + k * LP_THREADS;
+            if (i < n) {
+                const long long key = ((long long)total_key(v[k]) << 32) | (unsigned)i;
+                if (key > p.key) { // new maximum (or an equal value at a later index: expf(0) = 1 either way)
+                    p.s = (p.s == 0.0f ? 0.0f : p.s * expf(p.m - v[k])) + 1.0f;
+                    p.m = v[k];
+                    p.key = key;
+                } else {
+                    p.s += expf(v[k] - p.m);
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lp_combine(p, lp_shfl(p, o));
+    if (lane == 0) red[warp] = p;
+    __syncthreads();
+    if (warp == 0) {
+        p = lane < LP_THREADS / 32 ? red[lane] : LpPart{(long long)0x8000000000000000LL, -INFINITY, 0.0f};
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) lp_combine(p, lp_shfl(p, o));
+        if (lane == 0) {
+            if (lp_out) lp_out[row] = __fsub_rn(__fsub_rn(x[targets[row]], p.m), logf(p.s));
+            if (argmax_out) argmax_out[row] = (int)(p.key & 0xffffffffLL);
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // Exporter quantiser on the device (qwen3-export model_exporter.rs:104-161, SURVEY §8f-3):
 // scale = max|w|/127 (1.0 for an all-zero group), q = clamp(rint(w/scale), -127, 127).
 // rintf is round-half-to-even == round_half_to_even() (:321-338).

@@ -6,7 +6,10 @@ The tokenizer / chat templates are out of scope (SURVEY.md §2 #8); callers pass
 (q3_decode_greedy), only token ids cross PCIe."""
 from __future__ import annotations
 
-from typing import List, Optional, Sequence
+import math
+from typing import List, Optional, Sequence, Tuple
+
+import numpy as np
 
 from .sampler import Sampler
 
@@ -46,6 +49,19 @@ def generate_fast(transformer, prompt_tokens: Sequence[int], max_new: int) -> Li
     pos0 = len(prompt_tokens) - 1
     n = max(0, min(max_new, seq_len - pos0))
     return transformer.decode_greedy(int(prompt_tokens[-1]), pos0, n)
+
+
+def perplexity(transformer, tokens: Sequence[int], pos0: int = 0) -> Tuple[float, float]:
+    """Perplexity of `tokens` placed at positions pos0.. -> (exp(-mean log p), sum log p) over the len(tokens) - 1 predictions
+    tokens[1:], each conditioned on the tokens before it.  One q3_score pass; the KV cache then holds tokens[:-1]."""
+    if len(tokens) < 2:
+        raise ValueError("perplexity needs at least two tokens")
+    seq_len = transformer.get_config().seq_len
+    if pos0 < 0 or len(tokens) - 1 + pos0 > seq_len:
+        raise ValueError(f"{len(tokens) - 1} scored positions from pos0 {pos0} exceed seq_len {seq_len}")
+    lp, _ = transformer.score(list(tokens[:-1]), targets=list(tokens[1:]), pos0=pos0, want_argmax=False)
+    total = float(np.sum(np.asarray(lp, np.float64)))
+    return math.exp(-total / (len(tokens) - 1)), total
 
 
 # ---------------------------------------------------------------------------------------------

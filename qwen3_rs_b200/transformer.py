@@ -75,6 +75,7 @@ ABI = {
     "q3_decode_sample": (_i, [_vp, _i, _i, _i, _vp]),
     "q3_prefill": (_i, [_vp, _vp, _i, _i, _vp]),
     "q3_bench_prefill": (_i, [_vp, _vp, _i, _i, C.POINTER(_f)]),
+    "q3_score": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
     "q3_reset": (_i, [_vp]),
     "q3_logits_device": (_vp, [_vp]),
     "q3_logits_host": (_vp, [_vp]),
@@ -97,6 +98,7 @@ ABI = {
     "q3_op_sample": (_i, [_i, _vp, _i, _f, _f, C.POINTER(C.c_ulonglong), C.POINTER(_i)]),
     "q3_bench_gemm_q8": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(_f)]),
     "q3_op_prefill_attention": (_i, [_i, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    "q3_op_logprobs": (_i, [_i, _vp, _i, _i, _vp, _vp, _vp]),
     "q3_op_rmsnorm": (_i, [_i, _vp, _vp, _i, _vp]),
     "q3_op_quantize_q80": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
     "q3_op_quantize_q80_dev": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
@@ -207,6 +209,19 @@ class Transformer:
         ms = C.c_float(0)
         _check(load_library().q3_bench_prefill(self._h, _ptr(t), t.size, int(pos0), C.byref(ms)))
         return ms.value
+
+    def score(self, tokens: Sequence[int], targets: Optional[Sequence[int]] = None, pos0: int = 0, want_argmax: bool = True):
+        """q3_score: run `tokens` at positions pos0.. in one batched pass -> (logprobs, argmax).  logprobs[i] is the natural-log
+        probability of targets[i] after tokens[:i + 1] (None without targets); argmax[i] the greedy token there (None unless
+        want_argmax).  Leaves the KV cache as prefill(tokens, pos0) does."""
+        t = np.ascontiguousarray(tokens, np.int32).reshape(-1)
+        tg = None if targets is None else np.ascontiguousarray(targets, np.int32).reshape(-1)
+        if tg is not None and tg.size != t.size:
+            raise ValueError(f"score: {tg.size} targets for {t.size} tokens")
+        lp = None if tg is None else np.empty(t.size, np.float32)
+        am = np.empty(t.size, np.int32) if want_argmax else None
+        _check(load_library().q3_score(self._h, _ptr(t), t.size, int(pos0), _ptr(tg), _ptr(lp), _ptr(am)))
+        return lp, am
 
     def reset(self) -> None:
         _check(load_library().q3_reset(self._h))
@@ -424,6 +439,20 @@ def bench_gemm_q8(T: int, N: int, K: int, gs: int = 64, mode: int = 0, reps: int
     ms = C.c_float(0)
     _check(load_library().q3_bench_gemm_q8(device, T, N, K, gs, mode, reps, C.byref(ms)))
     return ms.value
+
+
+def op_logprobs(logits, targets=None, want_argmax: bool = True, device: int = 0):
+    """q3_score's reduction on logits [rows][n] -> (log softmax(row)[targets[r]] or None, last argmax of each row or None)."""
+    a = np.ascontiguousarray(logits, np.float32)
+    a = a.reshape(1, -1) if a.ndim == 1 else a
+    rows, n = a.shape
+    tg = None if targets is None else np.ascontiguousarray(targets, np.int32).reshape(-1)
+    if tg is not None and tg.size != rows:
+        raise ValueError(f"op_logprobs: {tg.size} targets for {rows} rows")
+    lp = None if tg is None else np.empty(rows, np.float32)
+    am = np.empty(rows, np.int32) if want_argmax else None
+    _check(load_library().q3_op_logprobs(device, _ptr(a), rows, n, _ptr(tg), _ptr(lp), _ptr(am)))
+    return lp, am
 
 
 def op_rmsnorm(x, w, device: int = 0):

@@ -25,6 +25,8 @@ extern "C" {
     fn q3_forward_argmax(h: *mut Q3Handle, token: c_int, pos: c_int, next_token: *mut c_int) -> c_int;
     fn q3_decode_greedy(h: *mut Q3Handle, first_token: c_int, pos0: c_int, n: c_int, tokens_out: *mut c_int) -> c_int;
     fn q3_prefill(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, last_logits_host: *mut c_float) -> c_int;
+    fn q3_score(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, targets: *const c_int, logprobs_out: *mut c_float,
+                argmax_out: *mut c_int) -> c_int;
     fn q3_reset(h: *mut Q3Handle) -> c_int;
     fn q3_logits_host(h: *mut Q3Handle) -> *mut c_float;
 }
@@ -93,6 +95,23 @@ impl CudaTransformer {
             panic!("{}", last_error());
         }
         unsafe { std::slice::from_raw_parts(self.logits, self.config.vocab_size) }
+    }
+
+    /// Score `tokens` at positions pos0.. in one batched pass: (natural-log probability of `targets[i]` after tokens[..=i],
+    /// greedy argmax there).  Perplexity of a text = exp(-mean) of `score(&text[..n - 1], &text[1..], 0).0`.
+    pub fn score(&mut self, tokens: &[usize], targets: &[usize], pos0: usize) -> (Vec<f32>, Vec<usize>) {
+        assert_eq!(tokens.len(), targets.len());
+        let ids: Vec<c_int> = tokens.iter().map(|&t| t as c_int).collect();
+        let tg: Vec<c_int> = targets.iter().map(|&t| t as c_int).collect();
+        let mut lp = vec![0.0f32; ids.len()];
+        let mut am = vec![0 as c_int; ids.len()];
+        let rc = unsafe {
+            q3_score(self.handle, ids.as_ptr(), ids.len() as c_int, pos0 as c_int, tg.as_ptr(), lp.as_mut_ptr(), am.as_mut_ptr())
+        };
+        if rc != 0 {
+            panic!("{}", last_error());
+        }
+        (lp, am.into_iter().map(|a| a as usize).collect())
     }
 
     /// Zero the KV cache (a fresh `TransformerBlockBuffers`, qwen3.rs:439-440).
