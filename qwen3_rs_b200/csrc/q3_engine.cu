@@ -47,7 +47,31 @@ static int fail(int code, const char *fmt, ...) {
     } while (0)
 
 extern "C" const char *q3_last_error(void) { return g_err; }
+
 extern "C" const char *q3_version(void) { return "qwen3cuda 0.1 (sm_100a)"; }
+
+// Milliseconds of GPU time from an event recorded on `s` before work() to one recorded after it, once the stream's earlier work
+// has finished.  The events are destroyed on every path.
+template <class F>
+static int time_events(cudaStream_t s, float *ms, F &&work) {
+    struct Events {
+        cudaEvent_t e[2] = {nullptr, nullptr};
+        ~Events() {
+            for (cudaEvent_t x : e)
+                if (x) cudaEventDestroy(x);
+        }
+    } ev;
+    CK(cudaEventCreate(&ev.e[0]));
+    CK(cudaEventCreate(&ev.e[1]));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaEventRecord(ev.e[0], s));
+    if (int rc = work()) return rc;
+    CK(cudaEventRecord(ev.e[1], s));
+    CK(cudaEventSynchronize(ev.e[1]));
+    CK(cudaGetLastError());
+    CK(cudaEventElapsedTime(ms, ev.e[0], ev.e[1]));
+    return 0;
+}
 
 // ------------------------------------------------------------------------------------------
 // handle
@@ -335,17 +359,26 @@ static int upload_f32(q3_handle *h, float **dst, const float *src, size_t n) {
     case 128: { constexpr int GS = 128; CALL; } break; \
     default: break;                          \
     }
+// GQA factor (query heads per kv head); create_impl admits only these four
+#define KV_DISPATCH(kv_mul, CALL)                          \
+    switch (kv_mul) {                                      \
+    case 1: { constexpr int KVM = 1; CALL; } break;        \
+    case 2: { constexpr int KVM = 2; CALL; } break;        \
+    case 4: { constexpr int KVM = 4; CALL; } break;        \
+    case 8: { constexpr int KVM = 8; CALL; } break;        \
+    default: break;                                        \
+    }
 
 template <int GS, int EPI>
-static void launch_gemv_t(const q3_handle *h, GemvArgs a, cudaStream_t s) {
+static void launch_gemv_t(int num_sms, int exact, GemvArgs a, cudaStream_t s) {
     int npairs = a.rows / 2;
     int grid = (npairs + 7) / 8;
-    int cap = h->num_sms * 8;
+    int cap = num_sms * 8;
     if (grid > cap) grid = cap;
     if (grid < 1) grid = 1;
     size_t smem = (size_t)a.K + (size_t)(a.K / GS) * 4;
-    const bool expref = EPI == EPI_SWIGLU && (h->exact & 16);
-    if (h->exact & 2) {
+    const bool expref = EPI == EPI_SWIGLU && (exact & 16);
+    if (exact & 2) {
         smem += (size_t)16 * (a.K / GS) * 4; // [8 warps][2 rows][ng] terms
         if (expref) k_gemv<GS, EPI, true, true><<<grid, 256, smem, s>>>(a);
         else k_gemv<GS, EPI, true, false><<<grid, 256, smem, s>>>(a);
@@ -354,25 +387,32 @@ static void launch_gemv_t(const q3_handle *h, GemvArgs a, cudaStream_t s) {
         else k_gemv<GS, EPI, false, false><<<grid, 256, smem, s>>>(a);
     }
 }
+// exact: the reference-order mask (q3_handle::exact)
 template <int EPI>
-static void launch_gemv(const q3_handle *h, const GemvArgs &a, cudaStream_t s) {
-    GS_DISPATCH(h->cfg.group_size, (launch_gemv_t<GS, EPI>(h, a, s)));
+static void launch_gemv(int gs, int num_sms, int exact, const GemvArgs &a, cudaStream_t s) {
+    GS_DISPATCH(gs, (launch_gemv_t<GS, EPI>(num_sms, exact, a, s)));
 }
 
-static int launch_norm_quant(const q3_handle *h, const NormQuantArgs &a, cudaStream_t s) {
-    if (h->exact & 1) {
-        GS_DISPATCH(h->cfg.group_size, (k_rmsnorm_quant<GS, true><<<1, 1024, (size_t)a.n * 4, s>>>(a)));
+static int launch_norm_quant(int gs, int exact, const NormQuantArgs &a, cudaStream_t s) {
+    if (exact & 1) {
+        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, true><<<1, 1024, (size_t)a.n * 4, s>>>(a)));
     } else {
-        GS_DISPATCH(h->cfg.group_size, (k_rmsnorm_quant<GS, false><<<1, 1024, 0, s>>>(a)));
+        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, false><<<1, 1024, 0, s>>>(a)));
     }
     return 1;
+}
+
+// split-K decode attention of one layer at position d_tokpos[1]: partials of ATTN_MAX_SPLITS CTAs per kv head into attn_part
+static void launch_attn_partial(const q3_handle *h, const float *kc_l, const float *vc_l, cudaStream_t s) {
+    dim3 ag(h->n_kv_l, ATTN_MAX_SPLITS);
+    KV_DISPATCH(h->kv_mul, (k_attn_partial<KVM><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l)));
 }
 
 // One transformer block.  Returns the number of kernel launches.
 static int launch_layer(q3_handle *h, int l, bool first_from_embed, cudaStream_t s) {
     const q3_config &c = h->cfg;
     const LayerDev &W = h->layers[l];
-    const int gs = c.group_size, dim = c.dim;
+    const int gs = c.group_size, dim = c.dim, ns = h->num_sms, ex = h->exact;
     const int *d_token = h->d_tokpos, *d_pos = h->d_tokpos + 1;
     float *kc_l = h->kc + (size_t)l * c.seq_len * h->KV_l;
     float *vc_l = h->vc + (size_t)l * c.seq_len * h->KV_l;
@@ -381,12 +421,12 @@ static int launch_layer(q3_handle *h, int l, bool first_from_embed, cudaStream_t
     NormQuantArgs na{};
     na.x = h->x; na.w = W.rms_att; na.q = h->xq; na.s = h->xs; na.n = dim;
     if (first_from_embed) { na.embed_q = h->embed.q; na.embed_s = h->embed.s; na.token = d_token; }
-    n += launch_norm_quant(h, na, s);
+    n += launch_norm_quant(gs, ex, na, s);
     // q, k, v projections (layers.rs:334-336)
     GemvArgs g{};
     g.wq = W.qkv.q; g.ws = W.qkv.s; g.xq = h->xq; g.xs = h->xs; g.K = dim; g.rows = W.qkv.rows;
     g.q = h->q; g.kc = kc_l; g.vc = vc_l; g.AH = h->AH_l; g.KV = h->KV_l; g.pos = d_pos;
-    launch_gemv<EPI_QKV>(h, g, s); n++;
+    launch_gemv<EPI_QKV>(gs, ns, ex, g, s); n++;
     // QK-norm + RoPE (layers.rs:339-340)
     int nh = h->n_heads_l + h->n_kv_l;
     if (h->exact & 4)
@@ -395,35 +435,28 @@ static int launch_layer(q3_handle *h, int l, bool first_from_embed, cudaStream_t
         k_qknorm_rope<false><<<(nh + 3) / 4, 128, 0, s>>>(h->q, kc_l, W.q_ln, W.k_ln, h->rope, d_pos, h->n_heads_l, h->n_kv_l, h->KV_l);
     n++;
     // attention (layers.rs:343) + quantize (qwen3.rs:152)
-    dim3 ag(h->n_kv_l, ATTN_MAX_SPLITS);
     if (h->exact & 8) {
         k_attn_ordered<<<h->n_heads_l, 128, 0, s>>>(h->q, kc_l, vc_l, h->att, h->xb, d_pos, h->KV_l, h->kv_mul, c.seq_len);
         int n4 = h->AH_l / 4, grid = (n4 + 255) / 256;
         GS_DISPATCH(gs, (k_quantize<GS><<<grid, 256, 0, s>>>(h->xb, h->AH_l, h->xq, h->xs)));
         n += 2;
     } else {
-    switch (h->kv_mul) {
-    case 1: k_attn_partial<1><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, d_pos, h->KV_l, h->n_heads_l); break;
-    case 2: k_attn_partial<2><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, d_pos, h->KV_l, h->n_heads_l); break;
-    case 4: k_attn_partial<4><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, d_pos, h->KV_l, h->n_heads_l); break;
-    case 8: k_attn_partial<8><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, d_pos, h->KV_l, h->n_heads_l); break;
-    }
-    n++;
-    GS_DISPATCH(gs, (k_attn_combine_quant<GS><<<h->n_heads_l, 128, 0, s>>>(h->attn_part, d_pos, h->xb, h->xq, h->xs)));
-    n++;
+        launch_attn_partial(h, kc_l, vc_l, s);
+        GS_DISPATCH(gs, (k_attn_combine_quant<GS><<<h->n_heads_l, 128, 0, s>>>(h->attn_part, d_pos, h->xb, h->xq, h->xs)));
+        n += 2;
     }
     // o_proj + residual (qwen3.rs:153-156)
     GemvArgs o{};
     o.wq = W.wo.q; o.ws = W.wo.s; o.xq = h->xq; o.xs = h->xs; o.K = h->AH_l; o.rows = dim; o.out = h->x;
-    launch_gemv<EPI_RESID>(h, o, s); n++;
+    launch_gemv<EPI_RESID>(gs, ns, ex, o, s); n++;
     // ffn_norm + quantize (qwen3.rs:159-161)
     NormQuantArgs nf{};
     nf.x = h->x; nf.w = W.rms_ffn; nf.q = h->xq; nf.s = h->xs; nf.n = dim;
-    n += launch_norm_quant(h, nf, s);
+    n += launch_norm_quant(gs, ex, nf, s);
     // gate/up + SwiGLU (layers.rs:468-475)
     GemvArgs gu{};
     gu.wq = W.w13.q; gu.ws = W.w13.s; gu.xq = h->xq; gu.xs = h->xs; gu.K = dim; gu.rows = W.w13.rows; gu.out = h->hb;
-    launch_gemv<EPI_SWIGLU>(h, gu, s); n++;
+    launch_gemv<EPI_SWIGLU>(gs, ns, ex, gu, s); n++;
     // quantize(hb) (layers.rs:478)
     {
         int n4 = h->H_l / 4, grid = (n4 + 255) / 256;
@@ -433,7 +466,7 @@ static int launch_layer(q3_handle *h, int l, bool first_from_embed, cudaStream_t
     // down + residual (layers.rs:479, qwen3.rs:175)
     GemvArgs dn{};
     dn.wq = W.w2.q; dn.ws = W.w2.s; dn.xq = h->hq; dn.xs = h->hs; dn.K = h->H_l; dn.rows = dim; dn.out = h->x;
-    launch_gemv<EPI_RESID>(h, dn, s); n++;
+    launch_gemv<EPI_RESID>(gs, ns, ex, dn, s); n++;
     return n;
 }
 
@@ -442,10 +475,10 @@ static int launch_head(q3_handle *h, cudaStream_t s) {
     const q3_config &c = h->cfg;
     NormQuantArgs na{};
     na.x = h->x; na.w = h->rms_final; na.q = h->xq; na.s = h->xs; na.n = c.dim; na.write_normed = 1;
-    int n = launch_norm_quant(h, na, s);
+    int n = launch_norm_quant(c.group_size, h->exact, na, s);
     GemvArgs g{};
     g.wq = h->wcls.q; g.ws = h->wcls.s; g.xq = h->xq; g.xs = h->xs; g.K = c.dim; g.rows = c.vocab_size; g.out = h->logits;
-    launch_gemv<EPI_STORE>(h, g, s); n++;
+    launch_gemv<EPI_STORE>(c.group_size, h->num_sms, h->exact, g, s); n++;
     return n;
 }
 
@@ -515,17 +548,6 @@ static int pick_n_kt(int K, int gs) {
     for (int n = (K + MEGA_MAX_KT - 1) / MEGA_MAX_KT; n <= 64; n++)
         if (K % (n * gs) == 0 && (K / n) % 16 == 0 && K / n <= MEGA_MAX_KT) return n;
     return 0;
-}
-
-template <int GS>
-static void *mega_kernel_for(int kvmul) {
-    switch (kvmul) {
-    case 1: return (void *)k_mega_decode<GS, 1>;
-    case 2: return (void *)k_mega_decode<GS, 2>;
-    case 4: return (void *)k_mega_decode<GS, 4>;
-    case 8: return (void *)k_mega_decode<GS, 8>;
-    }
-    return nullptr;
 }
 
 static int build_stream(q3_handle *h, MegaGemv &g, const std::vector<const DevQT *> &src, int units, int K, bool pair) {
@@ -644,7 +666,7 @@ static int build_mega(q3_handle *h, const float *rms_att_all, const float *rms_f
         a.part[0][r] = h->part_buf[0]; a.part[1][r] = h->part_buf[1];
         a.logits[r] = h->logits; a.best[r] = h->d_best; a.xbar[r] = (unsigned long long *)h->d_flags;
     }
-    GS_DISPATCH(gs, (h->mega_fn = mega_kernel_for<GS>(h->kv_mul)));
+    GS_DISPATCH(gs, KV_DISPATCH(h->kv_mul, (h->mega_fn = (void *)k_mega_decode<GS, KVM>)));
     if (!h->mega_fn) { h->mega_why = "no kernel for this GQA factor"; return 0; }
     const size_t slot = (size_t)MEGA_GW * (MEGA_MAX_KT + 4 * (MEGA_MAX_KT / gs));
     h->mega_smem = MEGA_NSTAGE * slot + MEGA_SCRATCH + 1024 + MEGA_MAX_KT * 4;
@@ -679,18 +701,14 @@ static int launch_mega(q3_handle *h, int l0, int l1, bool from_embed, bool run_h
 }
 
 static int check_tok_pos(const q3_handle *h, int token, int pos);
-// did any in-kernel wait time out?  The per-token entry points queue the 4-byte status read on the stream BEFORE their
-// one synchronize (mega_status_async) so that the check costs no extra round trip; the others read it here.
-static int mega_status_async(q3_handle *h) {
-    if (!h->d_status || h->decode_path != 1) return 0;
-    CK(cudaMemcpyAsync(h->h_small + 16, h->d_status, 4, cudaMemcpyDeviceToHost, h->stream));
-    return 0;
-}
-static int mega_check(q3_handle *h, bool queued = false) {
-    if (!h->d_status || h->decode_path != 1) return 0;
-    int code = 0;
-    if (queued) code = h->h_small[16];
-    else CK(cudaMemcpy(&code, h->d_status, 4, cudaMemcpyDeviceToHost));
+// The end of every entry point that waits for its work: one synchronize of the handle's stream, then -- did any in-kernel wait
+// time out?  The 4-byte status read is queued on the stream BEFORE the synchronize so that the check costs no extra round trip.
+static int finish_call(q3_handle *h) {
+    const bool mega = h->d_status && h->decode_path == 1;
+    if (mega) CK(cudaMemcpyAsync(h->h_small + 16, h->d_status, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (!mega) return 0;
+    const int code = h->h_small[16];
     if (code) {
         // Single GPU: all protocol state is local, reset it and the handle stays usable.  Tensor parallel: peers write into this
         // rank's flags and keep their own counters, so a rank-local reset would pair stale counters -- fail-stop instead.
@@ -730,13 +748,11 @@ extern "C" int q3_debug_profile(q3_handle *h, int token, int pos, unsigned long 
     h->margs.prof = d;
     int rc = launch_mega(h, 0, h->cfg.n_layers, true, true, false, false);
     h->margs.prof = nullptr;
-    if (!rc) {
-        cudaError_t e = cudaStreamSynchronize(h->stream);
-        if (e == cudaSuccess) e = cudaMemcpy(out, d, bytes, cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) rc = fail(Q3_ECUDA, "profile run failed: %s", cudaGetErrorString(e));
+    if (!rc) { // the stamps are copied out even when a wait timed out: they show where
+        cudaError_t e = cudaMemcpyAsync(out, d, bytes, cudaMemcpyDeviceToHost, h->stream);
+        rc = e == cudaSuccess ? finish_call(h) : fail(Q3_ECUDA, "profile copy failed: %s", cudaGetErrorString(e));
     }
     cudaFree(d);
-    if (!rc) rc = mega_check(h);
     return rc;
 }
 extern "C" int q3_num_sms(const q3_handle *h) { return h ? h->num_sms : 0; }
@@ -751,6 +767,27 @@ static inline bool use_mega(const q3_handle *h) { return h->decode_path == 1 && 
 static int tp_ready(const q3_handle *h) {
     if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
     if (h->tp_size > 1 && !use_mega(h)) return fail(Q3_EUNSUPPORTED, "under tensor parallelism only the persistent fast path is available");
+    return 0;
+}
+
+// what a caller needs from one decode step
+enum StepOut {
+    STEP_LOGITS,   // the logits
+    STEP_ARGMAX,   // + their argmax in d_tokpos[2]
+    STEP_FEEDBACK, // + the argmax fed back as the next token / position and appended to the history
+};
+// One decode step of the token / position in d_tokpos on the current path: the persistent kernel, or the CUDA graph of the
+// exact mask.  gather: see launch_mega.
+static int launch_decode_step(q3_handle *h, StepOut out, bool gather = false) {
+    if (use_mega(h)) return launch_mega(h, 0, h->cfg.n_layers, true, true, out == STEP_FEEDBACK, gather);
+    CK(cudaGraphLaunch(out == STEP_FEEDBACK ? h->g_greedy[h->exact] : h->g_fwd[h->exact], h->stream));
+    if (out == STEP_ARGMAX) launch_argmax(h, false, h->stream);
+    return 0;
+}
+// final norm + lm_head on h->x alone
+static int launch_head_only(q3_handle *h, bool gather) {
+    if (use_mega(h)) return launch_mega(h, 0, 0, false, true, false, gather);
+    launch_head(h, h->stream);
     return 0;
 }
 
@@ -847,6 +884,36 @@ static int prefill_prepare_tensor(q3_handle *h, DevQT &t) {
     return 0;
 }
 
+// k_pf_attention_h needs more than the default 48 KB of dynamic shared memory
+static int allow_pf_attention(int kv_mul) {
+    int rc = 0;
+    KV_DISPATCH(kv_mul, (rc = allow_smem(k_pf_attention_h<KVM>, PFH_SMEM)));
+    return rc;
+}
+
+// causal attention of T query rows (positions pos0 .. pos0+T-1) over K / V cache rows 0 .. pos0+T-1 on the tensor cores, FP16
+// hi / lo split: the K / V rows are split once into kvh ([4][plane] halves), then streamed
+static void launch_pf_attention(const float *q, const float *kc, const float *vc, __half *kvh, size_t plane, float *out, int T, int pos0,
+                                int n_kv, int kv_mul, int num_sms, cudaStream_t s) {
+    const int AH = n_kv * kv_mul * HEAD_DIM, KV = n_kv * HEAD_DIM;
+    k_pf_split_kv<<<num_sms * 4, 256, 0, s>>>(kc, vc, kvh, ((size_t)pos0 + T) * KV / 4, plane);
+    const int bq = PFH_R / kv_mul;
+    dim3 ag(n_kv, (T + bq - 1) / bq);
+    KV_DISPATCH(kv_mul, (k_pf_attention_h<KVM><<<ag, 128, PFH_SMEM, s>>>(q, kvh, plane, out, T, pos0, AH, KV)));
+}
+
+// RMSNorm + quantise of rows [0, T) of x (pitch dim) into pf_xq / pf_xsT (group-major, pitch Tpad); embed: the rows are first
+// gathered from the embedding table at pf_tokens
+static void launch_pf_norm_quant(const q3_handle *h, float *x, const float *w, int T, int Tpad, bool embed) {
+    const int dim = h->cfg.dim;
+    const int8_t *eq = embed ? h->embed.q : nullptr;
+    if (dim <= 4096) {
+        GS_DISPATCH(h->cfg.group_size, (k_pf_norm_quant<GS, 4><<<T, 256, 0, h->stream>>>(x, w, h->pf_xq, h->pf_xsT, dim, Tpad, eq, h->embed.s, h->pf_tokens, 0)));
+    } else {
+        GS_DISPATCH(h->cfg.group_size, (k_pf_norm_quant<GS><<<T, 256, 0, h->stream>>>(x, w, h->pf_xq, h->pf_xsT, dim, Tpad, eq, h->embed.s, h->pf_tokens, 0)));
+    }
+}
+
 static int prefill_init(q3_handle *h) {
     const q3_config &c = h->cfg;
     h->pf_ok = false;
@@ -859,11 +926,8 @@ static int prefill_init(q3_handle *h) {
         return 0;
     }
     if (!get_encode_fn()) { h->pf_why = "cuTensorMapEncodeTiled unavailable"; return 0; }
-    CK(cudaFuncSetAttribute(k_pf_attention_h<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
     int rc;
+    if ((rc = allow_pf_attention(h->kv_mul))) return rc;
     for (auto &W : h->layers) {
         if ((rc = prefill_prepare_tensor(h, W.qkv))) return rc;
         if ((rc = prefill_prepare_tensor(h, W.wo))) return rc;
@@ -987,41 +1051,21 @@ static int prefill_run(q3_handle *h, const int *tokens_host, int T, int pos0) {
         float *kc_l = h->kc + (size_t)l * c.seq_len * KV;
         float *vc_l = h->vc + (size_t)l * c.seq_len * KV;
         // attn_norm + quantize (qwen3.rs:134-136), embedding on layer 0
-        if (dim <= 4096) {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS, 4><<<T, 256, 0, s>>>(h->pf_x, W.rms_att, h->pf_xq, h->pf_xsT, dim, Tpad,
-                                                                     l == 0 ? h->embed.q : nullptr, h->embed.s, h->pf_tokens, 0)));
-        } else {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS><<<T, 256, 0, s>>>(h->pf_x, W.rms_att, h->pf_xq, h->pf_xsT, dim, Tpad,
-                                                                  l == 0 ? h->embed.q : nullptr, h->embed.s, h->pf_tokens, 0)));
-        }
+        launch_pf_norm_quant(h, h->pf_x, W.rms_att, T, Tpad, l == 0);
         PrefillGemmArgs g{};
         g.T = T; g.Tpad = Tpad; g.K = dim; g.N = W.qkv.rows; g.wsT = W.qkv.sT; g.xsT = h->pf_xsT;
         g.q = h->pf_q; g.kc = kc_l; g.vc = vc_l; g.AH = AH; g.KV = KV; g.pos0 = pos0;
         if ((rc = launch_gemm_q8<PF_EPI_QKV>(gs, mx_dim, W.qkv.map, g, s))) return rc;
         dim3 rg((h->n_heads_l + h->n_kv_l + 3) / 4, T);
         k_pf_qknorm_rope<<<rg, 128, 0, s>>>(h->pf_q, kc_l, W.q_ln, W.k_ln, h->rope, pos0, h->n_heads_l, h->n_kv_l, AH, KV);
-        // attention on the tensor cores, FP16 hi / lo split: K / V rows 0 .. pos0+T-1 of this layer split once, then streamed
-        const size_t rows = (size_t)pos0 + T, plane = h->pf_kvh_rows * KV;
-        k_pf_split_kv<<<h->num_sms * 4, 256, 0, s>>>(kc_l, vc_l, h->pf_kvh, rows * KV / 4, plane);
-        const int bq = PFH_R / h->kv_mul;
-        dim3 ag(h->n_kv_l, (T + bq - 1) / bq);
-        switch (h->kv_mul) {
-        case 1: k_pf_attention_h<1><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-        case 2: k_pf_attention_h<2><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-        case 4: k_pf_attention_h<4><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-        case 8: k_pf_attention_h<8><<<ag, 128, PFH_SMEM, s>>>(h->pf_q, h->pf_kvh, plane, h->pf_att, T, pos0, AH, KV); break;
-        }
+        launch_pf_attention(h->pf_q, kc_l, vc_l, h->pf_kvh, h->pf_kvh_rows * KV, h->pf_att, T, pos0, h->n_kv_l, h->kv_mul, h->num_sms, s);
         GS_DISPATCH(gs, (k_pf_quantize<GS><<<T, 256, 0, s>>>(h->pf_att, h->pf_xq, h->pf_xsT, AH, Tpad)));
         PrefillGemmArgs o{};
         o.T = T; o.Tpad = Tpad; o.K = AH; o.N = dim; o.wsT = W.wo.sT; o.xsT = h->pf_xsT; o.out = h->pf_x; o.ld_out = dim;
         if (h->tp_size == 1) {
             if ((rc = launch_gemm_q8<PF_EPI_RESID>(gs, mx_ah, W.wo.map, o, s))) return rc;
         } else if ((rc = prefill_tp_rowparallel(h, 0, mx_ah, W.wo.map, o, T))) return rc;
-        if (dim <= 4096) {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS, 4><<<T, 256, 0, s>>>(h->pf_x, W.rms_ffn, h->pf_xq, h->pf_xsT, dim, Tpad, nullptr, nullptr, nullptr, 0)));
-        } else {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS><<<T, 256, 0, s>>>(h->pf_x, W.rms_ffn, h->pf_xq, h->pf_xsT, dim, Tpad, nullptr, nullptr, nullptr, 0)));
-        }
+        launch_pf_norm_quant(h, h->pf_x, W.rms_ffn, T, Tpad, false);
         PrefillGemmArgs gu{};
         gu.T = T; gu.Tpad = Tpad; gu.K = dim; gu.N = W.w13.rows; gu.wsT = W.w13.sT; gu.xsT = h->pf_xsT; gu.out = h->pf_hb; gu.ld_out = H;
         if ((rc = launch_gemm_q8<PF_EPI_SWIGLU>(gs, mx_dim, W.w13.map, gu, s))) return rc;
@@ -1088,11 +1132,7 @@ static int score_rows(q3_handle *h, int T, int out0) {
     for (int r0 = 0; r0 < T; r0 += SCORE_ROWS) {
         const int Tc = T - r0 < SCORE_ROWS ? T - r0 : SCORE_ROWS, Tcpad = (Tc + 127) / 128 * 128;
         float *x = h->pf_x + (size_t)r0 * dim;
-        if (dim <= 4096) {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS, 4><<<Tc, 256, 0, s>>>(x, h->rms_final, h->pf_xq, h->pf_xsT, dim, Tcpad, nullptr, nullptr, nullptr, 0)));
-        } else {
-            GS_DISPATCH(gs, (k_pf_norm_quant<GS><<<Tc, 256, 0, s>>>(x, h->rms_final, h->pf_xq, h->pf_xsT, dim, Tcpad, nullptr, nullptr, nullptr, 0)));
-        }
+        launch_pf_norm_quant(h, x, h->rms_final, Tc, Tcpad, false);
         CUtensorMap mx;
         if ((rc = make_map_i8(&mx, h->pf_xq, Tcpad, dim))) return rc;
         PrefillGemmArgs g{};
@@ -1411,6 +1451,19 @@ static int check_tok_pos(const q3_handle *h, int token, int pos) {
     return 0;
 }
 
+// a prompt of n tokens at positions pos0 .. pos0+n-1 (q3_prefill, q3_bench_prefill, q3_score): the batched path gathers the
+// embedding rows of the tokens on the device unchecked
+static int check_prompt(const q3_handle *h, const int *tokens, int n, int pos0) {
+    if (!h || !tokens || n <= 0) return fail(Q3_EINVAL, "bad prompt arguments");
+    if (pos0 < 0 || (long long)pos0 + n > h->cfg.seq_len)
+        return fail(Q3_EINVAL, "index out of bounds: pos0 %d + n %d > seq_len %d", pos0, n, h->cfg.seq_len);
+    for (int i = 0; i < n; i++)
+        if (tokens[i] < 0 || tokens[i] >= h->cfg.vocab_size)
+            return fail(Q3_EINVAL, "index out of bounds: token %d >= vocab_size %d", tokens[i], h->cfg.vocab_size);
+    if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
+    return 0;
+}
+
 static int set_tok_pos(q3_handle *h, int token, int pos) {
     h->h_small[0] = token;
     h->h_small[1] = pos;
@@ -1427,20 +1480,11 @@ extern "C" int q3_forward(q3_handle *h, int token, int pos, float *logits_host) 
     if ((rc = set_tok_pos(h, token, pos))) return rc;
     if (logits_host && h->tp_size > 1 && h->logits_root >= 0 && h->logits_root != h->tp_rank)
         return fail(Q3_EINVAL, "rank %d asked for logits but the logits root is rank %d", h->tp_rank, h->logits_root);
-    if (use_mega(h)) {
-        if ((rc = launch_mega(h, 0, h->cfg.n_layers, true, true, false, logits_host != nullptr))) return rc;
-    } else {
-        CK(cudaGraphLaunch(h->g_fwd[h->exact], h->stream));
-    }
-    if ((rc = mega_status_async(h))) return rc;
-    if (logits_host) {
-        CK(cudaMemcpyAsync(h->h_logits, h->logits, (size_t)h->cfg.vocab_size * 4, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        if (logits_host != h->h_logits) memcpy(logits_host, h->h_logits, (size_t)h->cfg.vocab_size * 4);
-    } else {
-        CK(cudaStreamSynchronize(h->stream));
-    }
-    return mega_check(h, true);
+    if ((rc = launch_decode_step(h, STEP_LOGITS, logits_host != nullptr))) return rc;
+    if (logits_host) CK(cudaMemcpyAsync(h->h_logits, h->logits, (size_t)h->cfg.vocab_size * 4, cudaMemcpyDeviceToHost, h->stream));
+    if ((rc = finish_call(h))) return rc;
+    if (logits_host && logits_host != h->h_logits) memcpy(logits_host, h->h_logits, (size_t)h->cfg.vocab_size * 4);
+    return Q3_OK;
 }
 
 extern "C" int q3_forward_argmax(q3_handle *h, int token, int pos, int *next_token) {
@@ -1449,16 +1493,11 @@ extern "C" int q3_forward_argmax(q3_handle *h, int token, int pos, int *next_tok
     if (!next_token) return fail(Q3_EINVAL, "null next_token");
     CK(cudaSetDevice(h->device));
     if ((rc = set_tok_pos(h, token, pos))) return rc;
-    if (use_mega(h)) {
-        if ((rc = launch_mega(h, 0, h->cfg.n_layers, true, true, true, false))) return rc;
-    } else {
-        CK(cudaGraphLaunch(h->g_greedy[h->exact], h->stream));
-    }
+    if ((rc = launch_decode_step(h, STEP_FEEDBACK))) return rc;
     CK(cudaMemcpyAsync(h->h_small + 8, h->d_tokpos + 2, 4, cudaMemcpyDeviceToHost, h->stream));
-    if ((rc = mega_status_async(h))) return rc;
-    CK(cudaStreamSynchronize(h->stream));
+    if ((rc = finish_call(h))) return rc;
     *next_token = h->h_small[8];
-    return mega_check(h, true);
+    return Q3_OK;
 }
 
 extern "C" int q3_decode_greedy(q3_handle *h, int first_token, int pos0, int n, int *tokens_out) {
@@ -1468,18 +1507,10 @@ extern "C" int q3_decode_greedy(q3_handle *h, int first_token, int pos0, int n, 
     if (n > h->history_cap) return fail(Q3_EINVAL, "n too large");
     CK(cudaSetDevice(h->device));
     if ((rc = set_tok_pos(h, first_token, pos0))) return rc;
-    for (int i = 0; i < n; i++) {
-        if (use_mega(h)) {
-            if ((rc = launch_mega(h, 0, h->cfg.n_layers, true, true, true, false))) return rc;
-        } else {
-            CK(cudaGraphLaunch(h->g_greedy[h->exact], h->stream));
-        }
-    }
-    if (tokens_out && n > 0) {
-        CK(cudaMemcpyAsync(tokens_out, h->d_history, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
-    }
-    CK(cudaStreamSynchronize(h->stream));
-    return mega_check(h);
+    for (int i = 0; i < n; i++)
+        if ((rc = launch_decode_step(h, STEP_FEEDBACK))) return rc;
+    if (tokens_out && n > 0) CK(cudaMemcpyAsync(tokens_out, h->d_history, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    return finish_call(h);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1527,17 +1558,8 @@ extern "C" int q3_sampler_skip(q3_handle *h, int n_draws) {
 static int launch_sampled_step(q3_handle *h, bool feedback) {
     int rc;
     const bool greedy = h->samp_temperature == 0.0f;
-    if (use_mega(h)) {
-        if ((rc = launch_mega(h, 0, h->cfg.n_layers, true, true, greedy && feedback, !greedy))) return rc;
-    } else if (greedy) {
-        if (feedback) CK(cudaGraphLaunch(h->g_greedy[h->exact], h->stream));
-        else {
-            CK(cudaGraphLaunch(h->g_fwd[h->exact], h->stream));
-            launch_argmax(h, false, h->stream);
-        }
-    } else {
-        CK(cudaGraphLaunch(h->g_fwd[h->exact], h->stream));
-    }
+    // greedy: the step's own argmax; otherwise k_sample draws from the full logits
+    if ((rc = launch_decode_step(h, !greedy ? STEP_LOGITS : feedback ? STEP_FEEDBACK : STEP_ARGMAX, !greedy))) return rc;
     if (!greedy) {
         SampleArgs a{};
         a.logits = h->logits; a.n = h->cfg.vocab_size; a.temperature = h->samp_temperature; a.topp = h->samp_topp;
@@ -1557,10 +1579,9 @@ extern "C" int q3_forward_sample(q3_handle *h, int token, int pos, int *next_tok
     if ((rc = set_tok_pos(h, token, pos))) return rc;
     if ((rc = launch_sampled_step(h, false))) return rc;
     CK(cudaMemcpyAsync(h->h_small + 8, h->d_tokpos + 2, 4, cudaMemcpyDeviceToHost, h->stream));
-    if ((rc = mega_status_async(h))) return rc;
-    CK(cudaStreamSynchronize(h->stream));
+    if ((rc = finish_call(h))) return rc;
     *next_token = h->h_small[8];
-    return mega_check(h, true);
+    return Q3_OK;
 }
 extern "C" int q3_decode_sample(q3_handle *h, int first_token, int pos0, int n, int *tokens_out) {
     int rc = check_tok_pos(h, first_token, pos0);
@@ -1573,8 +1594,7 @@ extern "C" int q3_decode_sample(q3_handle *h, int first_token, int pos0, int n, 
     for (int i = 0; i < n; i++)
         if ((rc = launch_sampled_step(h, true))) return rc;
     if (tokens_out && n > 0) CK(cudaMemcpyAsync(tokens_out, h->d_history, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    return mega_check(h);
+    return finish_call(h);
 }
 
 extern "C" int q3_bench_decode(q3_handle *h, int first_token, int pos0, int steps, float *ms_out) {
@@ -1583,26 +1603,15 @@ extern "C" int q3_bench_decode(q3_handle *h, int first_token, int pos0, int step
     if (steps < 1 || pos0 + steps > h->cfg.seq_len) return fail(Q3_EINVAL, "pos0 + steps exceeds seq_len");
     CK(cudaSetDevice(h->device));
     if ((rc = set_tok_pos(h, first_token, pos0))) return rc;
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventRecord(e0, h->stream));
-    for (int i = 0; i < steps; i++) {
-        if (use_mega(h)) {
-            if ((rc = launch_mega(h, 0, h->cfg.n_layers, true, true, true, false))) return rc;
-        } else {
-            CK(cudaGraphLaunch(h->g_greedy[h->exact], h->stream));
-        }
-    }
-    CK(cudaEventRecord(e1, h->stream));
-    CK(cudaEventSynchronize(e1));
     float ms = 0;
-    CK(cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
+    rc = time_events(h->stream, &ms, [&] {
+        for (int i = 0; i < steps; i++)
+            if (int rc1 = launch_decode_step(h, STEP_FEEDBACK)) return rc1;
+        return 0;
+    });
+    if (rc) return rc;
     if (ms_out) *ms_out = ms;
-    return mega_check(h);
+    return finish_call(h);
 }
 
 extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float *ms_out, int *launches_out,
@@ -1613,7 +1622,7 @@ extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float 
     int rc;
     if ((rc = set_tok_pos(h, 0, pos))) return rc;
     const q3_config &c = h->cfg;
-    const int gs = c.group_size, dim = c.dim, L = c.n_layers;
+    const int gs = c.group_size, ns = h->num_sms, ex = h->exact, dim = c.dim, L = c.n_layers;
     auto one = [&](int l) {
         const LayerDev &W = h->layers[l];
         float *kc_l = h->kc + (size_t)l * c.seq_len * h->KV_l;
@@ -1624,33 +1633,27 @@ extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float 
         case 0:
             g.wq = W.qkv.q; g.ws = W.qkv.s; g.K = dim; g.rows = W.qkv.rows; g.q = h->q; g.kc = kc_l; g.vc = vc_l;
             g.AH = h->AH_l; g.KV = h->KV_l;
-            launch_gemv<EPI_QKV>(h, g, h->stream);
+            launch_gemv<EPI_QKV>(gs, ns, ex, g, h->stream);
             break;
         case 1:
             g.wq = W.wo.q; g.ws = W.wo.s; g.K = h->AH_l; g.rows = dim; g.out = h->xb;
-            launch_gemv<EPI_STORE>(h, g, h->stream);
+            launch_gemv<EPI_STORE>(gs, ns, ex, g, h->stream);
             break;
         case 2:
             g.wq = W.w13.q; g.ws = W.w13.s; g.K = dim; g.rows = W.w13.rows; g.out = h->hb;
-            launch_gemv<EPI_SWIGLU>(h, g, h->stream);
+            launch_gemv<EPI_SWIGLU>(gs, ns, ex, g, h->stream);
             break;
         case 3:
             g.wq = W.w2.q; g.ws = W.w2.s; g.xq = h->hq; g.xs = h->hs; g.K = h->H_l; g.rows = dim; g.out = h->xb;
-            launch_gemv<EPI_STORE>(h, g, h->stream);
+            launch_gemv<EPI_STORE>(gs, ns, ex, g, h->stream);
             break;
         case 4:
             g.wq = h->wcls.q; g.ws = h->wcls.s; g.K = dim; g.rows = c.vocab_size; g.out = h->logits;
-            launch_gemv<EPI_STORE>(h, g, h->stream);
+            launch_gemv<EPI_STORE>(gs, ns, ex, g, h->stream);
             break;
-        case 5: {
-            dim3 ag(h->n_kv_l, ATTN_MAX_SPLITS);
-            switch (h->kv_mul) {
-            case 1: k_attn_partial<1><<<ag, 128, 0, h->stream>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l); break;
-            case 2: k_attn_partial<2><<<ag, 128, 0, h->stream>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l); break;
-            case 4: k_attn_partial<4><<<ag, 128, 0, h->stream>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l); break;
-            case 8: k_attn_partial<8><<<ag, 128, 0, h->stream>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l); break;
-            }
-        } break;
+        case 5:
+            launch_attn_partial(h, kc_l, vc_l, h->stream);
+            break;
         }
     };
     double bytes = 0;
@@ -1664,20 +1667,13 @@ extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float 
     case 5: bytes = 2.0 * (pos + 1) * h->KV_l * 4; break;
     }
     for (int l = 0; l < L; l++) one(l); // warm-up pass
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventRecord(e0, h->stream));
-    for (int r = 0; r < reps; r++)
-        for (int l = 0; l < L; l++) one(l);
-    CK(cudaEventRecord(e1, h->stream));
-    CK(cudaEventSynchronize(e1));
-    CK(cudaGetLastError());
     float ms = 0;
-    CK(cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
+    rc = time_events(h->stream, &ms, [&] {
+        for (int r = 0; r < reps; r++)
+            for (int l = 0; l < L; l++) one(l);
+        return 0;
+    });
+    if (rc) return rc;
     if (ms_out) *ms_out = ms;
     if (launches_out) *launches_out = reps * L;
     if (bytes_out) *bytes_out = bytes;
@@ -1685,10 +1681,7 @@ extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float 
 }
 
 extern "C" int q3_prefill(q3_handle *h, const int *tokens, int n, int pos0, float *last_logits_host) {
-    if (!h || !tokens || n <= 0) return fail(Q3_EINVAL, "bad prefill arguments");
-    if (pos0 < 0 || pos0 + n > h->cfg.seq_len) return fail(Q3_EINVAL, "index out of bounds: pos0 + n = %d > seq_len %d", pos0 + n, h->cfg.seq_len);
-    for (int i = 0; i < n; i++)
-        if (tokens[i] < 0 || tokens[i] >= h->cfg.vocab_size) return fail(Q3_EINVAL, "index out of bounds: token %d", tokens[i]);
+    if (int rc = check_prompt(h, tokens, n, pos0)) return rc;
     CK(cudaSetDevice(h->device));
     if (!h->pf_ok || h->exact) {
         // sequential decode steps: same results as n forwards by construction (exact mode, TP, odd shapes)
@@ -1699,68 +1692,42 @@ extern "C" int q3_prefill(q3_handle *h, const int *tokens, int n, int pos0, floa
         return Q3_OK;
     }
     int rc;
-    if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
     if ((rc = prefill_chunks(h, tokens, n, pos0))) return rc;
     // final norm + quantize + lm_head on the last token only (qwen3.rs:72-76)
     if ((rc = set_tok_pos(h, tokens[n - 1], pos0 + n - 1))) return rc;
-    if (use_mega(h)) {
-        if ((rc = launch_mega(h, 0, 0, false, true, false, last_logits_host != nullptr))) return rc;
-    } else {
-        launch_head(h, h->stream);
-    }
-    if (last_logits_host) {
-        CK(cudaMemcpyAsync(h->h_logits, h->logits, (size_t)h->cfg.vocab_size * 4, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        if (last_logits_host != h->h_logits) memcpy(last_logits_host, h->h_logits, (size_t)h->cfg.vocab_size * 4);
-    } else {
-        CK(cudaStreamSynchronize(h->stream));
-    }
+    if ((rc = launch_head_only(h, last_logits_host != nullptr))) return rc;
+    if (last_logits_host) CK(cudaMemcpyAsync(h->h_logits, h->logits, (size_t)h->cfg.vocab_size * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaGetLastError());
-    return mega_check(h);
+    if ((rc = finish_call(h))) return rc;
+    if (last_logits_host && last_logits_host != h->h_logits) memcpy(last_logits_host, h->h_logits, (size_t)h->cfg.vocab_size * 4);
+    return Q3_OK;
 }
 
 extern "C" int q3_bench_prefill(q3_handle *h, const int *tokens, int n, int pos0, float *ms_out) {
-    if (!h || !tokens || n <= 0) return fail(Q3_EINVAL, "bad prefill arguments");
+    int rc = check_prompt(h, tokens, n, pos0);
+    if (rc) return rc;
     if (!h->pf_ok) return fail(Q3_EUNSUPPORTED, "batched prefill unavailable: %s", h->pf_why.c_str());
-    if (pos0 < 0 || pos0 + n > h->cfg.seq_len) return fail(Q3_EINVAL, "index out of bounds");
     CK(cudaSetDevice(h->device));
-    int rc;
-    if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
     if ((rc = prefill_chunks(h, tokens, n, pos0))) return rc; // warm-up (also sizes the buffers)
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventRecord(e0, h->stream));
-    if ((rc = prefill_chunks(h, tokens, n, pos0))) return rc;
-    CK(cudaEventRecord(e1, h->stream));
-    CK(cudaEventSynchronize(e1));
-    CK(cudaGetLastError());
     float ms = 0;
-    CK(cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
+    if ((rc = time_events(h->stream, &ms, [&] { return prefill_chunks(h, tokens, n, pos0); }))) return rc;
     if (ms_out) *ms_out = ms;
-    return h->tp_size > 1 ? mega_check(h) : Q3_OK;
+    return finish_call(h);
 }
 
 extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out) {
-    if (!h || !tokens || n <= 0) return fail(Q3_EINVAL, "bad score arguments");
-    if (pos0 < 0 || (long long)pos0 + n > h->cfg.seq_len)
-        return fail(Q3_EINVAL, "index out of bounds: pos0 + n = %lld > seq_len %d", (long long)pos0 + n, h->cfg.seq_len);
+    int rc = check_prompt(h, tokens, n, pos0);
+    if (rc) return rc;
     if (!logprobs_out && !argmax_out) return fail(Q3_EINVAL, "q3_score needs logprobs_out or argmax_out");
     if (logprobs_out && !targets) return fail(Q3_EINVAL, "logprobs_out needs targets");
     const int V = h->cfg.vocab_size;
-    for (int i = 0; i < n; i++) {
-        if (tokens[i] < 0 || tokens[i] >= V) return fail(Q3_EINVAL, "index out of bounds: token %d", tokens[i]);
-        if (logprobs_out && (targets[i] < 0 || targets[i] >= V)) return fail(Q3_EINVAL, "index out of bounds: target %d", targets[i]);
-    }
-    if (h->tp_size > 1 && !h->tp_connected) return fail(Q3_ECOMM, "tensor-parallel handle used before q3_tp_connect");
+    if (logprobs_out)
+        for (int i = 0; i < n; i++)
+            if (targets[i] < 0 || targets[i] >= V) return fail(Q3_EINVAL, "index out of bounds: target %d", targets[i]);
     const bool batched = h->pf_ok && !h->exact && V % 128 == 0;
     // Under TP, q3_forward leaves only this rank's vocabulary shard in h->logits (all of it only on the logits root, if one is set)
     if (h->tp_size > 1 && !batched) return fail(Q3_EUNSUPPORTED, "q3_score under tensor parallelism needs the batched prefill path");
     CK(cudaSetDevice(h->device));
-    int rc;
     if ((rc = score_reserve(h, batched, n))) return rc;
     h->sc_want_lp = logprobs_out != nullptr;
     if (logprobs_out) CK(cudaMemcpyAsync(h->sc_targets, targets, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
@@ -1775,9 +1742,8 @@ extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const 
     }
     if (logprobs_out) CK(cudaMemcpyAsync(logprobs_out, h->sc_lp, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
     if (argmax_out) CK(cudaMemcpyAsync(argmax_out, h->sc_argmax, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
-    return mega_check(h);
+    return finish_call(h);
 }
 
 extern "C" int q3_reset(q3_handle *h) {
@@ -1826,16 +1792,12 @@ extern "C" int q3_forward_layers(q3_handle *h, int pos, int layer0, int layer1, 
     }
     CK(cudaMemcpyAsync(x_host, h->x, (size_t)h->cfg.dim * 4, cudaMemcpyDeviceToHost, h->stream));
     if (run_head) {
-        if (use_mega(h)) {
-            if ((rc = launch_mega(h, 0, 0, false, true, false, true))) return rc;
-        } else
-        launch_head(h, h->stream);
+        if ((rc = launch_head_only(h, true))) return rc;
         if (logits_host)
             CK(cudaMemcpyAsync(logits_host, h->logits, (size_t)h->cfg.vocab_size * 4, cudaMemcpyDeviceToHost, h->stream));
     }
-    CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
-    return mega_check(h);
+    return finish_call(h);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1907,14 +1869,10 @@ extern "C" int q3_op_matmul(int device, const int8_t *xq, const float *xs, const
     GemvArgs a{};
     a.wq = dwq.as<int8_t>(); a.ws = dws.as<float>(); a.xq = dxq.as<int8_t>(); a.xs = dxs.as<float>();
     a.K = n; a.rows = d; a.out = dout.as<float>(); a.dots = group_dots_out ? ddots.as<int32_t>() : nullptr;
-    q3_handle fake;
-    cudaDeviceProp prop;
-    cudaGetDeviceProperties(&prop, device);
-    fake.num_sms = prop.multiProcessorCount;
-    fake.cfg.group_size = gs;
-    fake.exact = exact ? 31 : 0;
+    int num_sms = 0;
+    CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
     if ((rc = prepare_exact_kernels())) return rc;
-    launch_gemv<EPI_STORE>(&fake, a, 0);
+    launch_gemv<EPI_STORE>(gs, num_sms, exact ? 31 : 0, a, 0);
     CK(cudaGetLastError());
     CK(cudaMemcpy(out, dout.p, (size_t)d * 4, cudaMemcpyDeviceToHost));
     if (group_dots_out) CK(cudaMemcpy(group_dots_out, ddots.p, (size_t)d * ng * 4, cudaMemcpyDeviceToHost));
@@ -2011,7 +1969,7 @@ extern "C" int q3_op_logprobs(int device, const float *logits, int rows, int n, 
 
 // Causal prefill attention alone (layers.rs:374-419 for T query tokens at positions pos0 .. pos0+T-1 over a cache of pos0+T rows):
 // q [T][n_heads*128] (already normalised + rotated), k / v [pos0+T][n_kv*128], out [T][n_heads*128].
-// The kernel is the one q3_prefill runs (k_pf_attention_h over a hi / lo split of K / V).
+// The launch is the one q3_prefill runs (launch_pf_attention: k_pf_attention_h over a hi / lo split of K / V).
 extern "C" int q3_op_prefill_attention(int device, const float *q, const float *k, const float *v, int T, int pos0, int n_heads, int n_kv,
                                        float *out) {
     CK(cudaSetDevice(device));
@@ -2027,20 +1985,11 @@ extern "C" int q3_op_prefill_attention(int device, const float *q, const float *
     CK(cudaMemcpy(dq.p, q, (size_t)T * AH * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dk.p, k, (size_t)nk * KV * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dv.p, v, (size_t)nk * KV * 4, cudaMemcpyHostToDevice));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    CK(cudaFuncSetAttribute(k_pf_attention_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFH_SMEM));
-    const size_t plane = (size_t)nk * KV;
-    k_pf_split_kv<<<296, 256>>>(dk.as<float>(), dv.as<float>(), dkvh.as<__half>(), plane / 4, plane);
-    const int bq = PFH_R / kv_mul;
-    dim3 ag(n_kv, (T + bq - 1) / bq);
-    switch (kv_mul) {
-    case 1: k_pf_attention_h<1><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
-    case 2: k_pf_attention_h<2><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
-    case 4: k_pf_attention_h<4><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
-    case 8: k_pf_attention_h<8><<<ag, 128, PFH_SMEM>>>(dq.as<float>(), dkvh.as<__half>(), plane, dout.as<float>(), T, pos0, AH, KV); break;
-    }
+    int num_sms = 0;
+    CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
+    if ((rc = allow_pf_attention(kv_mul))) return rc;
+    launch_pf_attention(dq.as<float>(), dk.as<float>(), dv.as<float>(), dkvh.as<__half>(), (size_t)nk * KV, dout.as<float>(), T, pos0, n_kv,
+                        kv_mul, num_sms, 0);
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy(out, dout.p, (size_t)T * AH * 4, cudaMemcpyDeviceToHost));
@@ -2078,22 +2027,12 @@ extern "C" int q3_bench_gemm_q8(int device, int T, int N, int K, int gs, int mod
     a.T = T; a.Tpad = Tpad; a.N = N; a.K = K; a.wsT = dwsT.as<float>(); a.xsT = dxsT.as<float>(); a.out = dout.as<float>(); a.ld_out = N;
     if ((rc = launch_gemm_q8<PF_EPI_STORE>(gs, mx, mw, a, 0, mode))) return rc; // warm-up
     CK(cudaDeviceSynchronize());
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
     float best = 1e30f;
     for (int r = 0; r < reps; r++) {
-        CK(cudaEventRecord(e0, 0));
-        if ((rc = launch_gemm_q8<PF_EPI_STORE>(gs, mx, mw, a, 0, mode))) return rc;
-        CK(cudaEventRecord(e1, 0));
-        CK(cudaEventSynchronize(e1));
         float ms = 0;
-        CK(cudaEventElapsedTime(&ms, e0, e1));
+        if ((rc = time_events(0, &ms, [&] { return launch_gemm_q8<PF_EPI_STORE>(gs, mx, mw, a, 0, mode); }))) return rc;
         best = ms < best ? ms : best;
     }
-    CK(cudaGetLastError());
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
     if (ms_out) *ms_out = best;
     return Q3_OK;
 }

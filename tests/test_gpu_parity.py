@@ -373,6 +373,13 @@ def test_bounds_are_errors_not_ub(models):
         with pytest.raises(T.Q3Error) as e:
             m.forward(tok, pos)
         assert e.value.code == -1 and "index out of bounds" in e.value.message
+    # prompts: a token id outside the vocabulary, and positions pos0 .. pos0+n-1 running past the context
+    for toks, pos0 in [([1, c.vocab_size], 0), ([-1, 1], 0), ([1, 2], c.seq_len - 1)]:
+        for run in (m.prefill, m.bench_prefill, m.score):
+            with pytest.raises(T.Q3Error) as e:
+                run(toks, pos0=pos0)
+            assert e.value.code == -1 and "index out of bounds" in e.value.message, run.__name__
+    m.forward(1, 0)
 
 
 def test_ctx_length_override(models):
