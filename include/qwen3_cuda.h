@@ -135,6 +135,18 @@ int q3_bench_prefill(q3_handle *h, const int *tokens, int n, int pos0, float *ms
  * and returns the full results; there the batched path is required (Q3_EUNSUPPORTED otherwise). */
 int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out);
 
+/* Extension: q3_score plus the k most likely tokens at every position, 1 <= k <= min(Q3_TOPK_MAX, vocab_size).
+ *   topk_ids_out[i*k + j]      = the j-th largest entry of logits_i: descending value, among equal values the larger index
+ *                                first (so topk_ids_out[i*k] == argmax_out[i])
+ *   topk_logprobs_out[i*k + j] = log softmax(logits_i)[topk_ids_out[i*k + j]]; bit-identical to q3_score's logprobs_out[i]
+ *                                where that id is targets[i]
+ * Both are required; targets / logprobs_out / argmax_out are optional, as in q3_score, and bit-identical to its outputs.
+ * Same checks, cache effect, paths and tensor-parallel behaviour as q3_score.  The [seq_len][k] result buffers are allocated
+ * on the first call and grow with k. */
+#define Q3_TOPK_MAX 64
+int q3_score_topk(q3_handle *h, const int *tokens, int n, int pos0, int k, int *topk_ids_out, float *topk_logprobs_out,
+                  const int *targets, float *logprobs_out, int *argmax_out);
+
 /* Zero the KV cache (a freshly built reference transformer, qwen3.rs:439-440). */
 int q3_reset(q3_handle *h);
 
@@ -233,6 +245,10 @@ int q3_op_sample(int device, const float *logits, int n, float temperature, floa
                  int *token_out);
 /* The reduction q3_score runs, on host-supplied logits [rows][n] (operator-level parity tests). */
 int q3_op_logprobs(int device, const float *logits, int rows, int n, const int *targets, float *logprobs_out, int *argmax_out);
+/* The reduction q3_score_topk runs, on host-supplied logits [rows][n]: ids_out / lps_out [rows][k] (required), 1 <= k <=
+ * min(Q3_TOPK_MAX, n); logprobs_out (needs targets) and argmax_out optional, as in q3_op_logprobs. */
+int q3_op_topk_logprobs(int device, const float *logits, int rows, int n, int k, const int *targets, int *ids_out, float *lps_out,
+                        float *logprobs_out, int *argmax_out);
 /* layers.rs:109-119 RMSNorm::forward */
 int q3_op_rmsnorm(int device, const float *x, const float *w, int n, float *out);
 /* qwen3-export model_exporter.rs:104-161 quantize_q80 on the device (SURVEY.md §8f-3). */

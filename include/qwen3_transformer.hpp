@@ -17,7 +17,7 @@
 //   tokenizer.rs          Tokenizer (byte-level BPE)         qwen3::Tokenizer (same results; vocabulary lookups hashed)
 //   generation.rs:188-195 render_prompt                      qwen3::render_prompt
 //
-// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill, score.
+// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill, score, score_topk.
 //
 // Errors: construction failures throw qwen3::Error (the reference returns anyhow::Error with the same
 // message text); forward() with an out-of-range token / pos throws (the reference panics on the slice
@@ -127,6 +127,27 @@ public:
         detail::check(q3_score(h_, tokens.data(), (int)tokens.size(), (int)pos0, targets.empty() ? nullptr : targets.data(),
                                targets.empty() ? nullptr : lp.data(), am.data()));
         return {std::move(lp), std::move(am)};
+    }
+    // q3_score_topk: the k most likely tokens at every position, row-major [n][k] (most likely first, equal values with the
+    // larger id first) and their log-probabilities; then score()'s two results (first empty without targets).
+    struct TopK {
+        std::vector<int> ids;
+        std::vector<float> logprobs;
+        std::vector<float> target_logprobs;
+        std::vector<int> argmax;
+    };
+    TopK score_topk(const std::vector<int> &tokens, int k, const std::vector<int> &targets, size_t pos0) {
+        if (!targets.empty() && targets.size() != tokens.size()) throw std::invalid_argument("score_topk: targets and tokens differ in length");
+        if (k < 1 || k > Q3_TOPK_MAX) throw std::invalid_argument("score_topk: k outside 1 .. Q3_TOPK_MAX");
+        TopK r;
+        r.ids.resize(tokens.size() * (size_t)k);
+        r.logprobs.resize(tokens.size() * (size_t)k);
+        r.target_logprobs.resize(targets.size());
+        r.argmax.resize(tokens.size());
+        detail::check(q3_score_topk(h_, tokens.data(), (int)tokens.size(), (int)pos0, k, r.ids.data(), r.logprobs.data(),
+                                    targets.empty() ? nullptr : targets.data(), targets.empty() ? nullptr : r.target_logprobs.data(),
+                                    r.argmax.data()));
+        return r;
     }
     void reset() { detail::check(q3_reset(h_)); } // zero the KV cache
     q3_handle *handle() { return h_; }

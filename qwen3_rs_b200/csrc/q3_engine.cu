@@ -164,6 +164,11 @@ struct q3_handle {
     float *sc_lp = nullptr, *sc_logits = nullptr;
     int sc_cap = 0;
     bool sc_want_lp = false; // this call asked for log-probabilities (targets uploaded)
+    // q3_score_topk, allocated on its first call: ids / log-probabilities [seq_len][tk_cap] (grow-only in k, freed in q3_destroy)
+    int *tk_ids = nullptr;
+    float *tk_lps = nullptr;
+    int tk_cap = 0;
+    int tk_k = 0; // k of this call; 0 in q3_score
     // device sampler (sampler.rs on the device, q3_sampler.cuh)
     float samp_temperature = 0.0f, samp_topp = 0.9f;
     unsigned long long *d_rng = nullptr, *d_keys = nullptr;
@@ -1117,9 +1122,33 @@ static int score_reserve(q3_handle *h, bool lm_head, int rows) {
     return 0;
 }
 
+// the [seq_len][k] results of q3_score_topk, sized for the largest k asked for so far (one allocation: ids, then lps)
+static int topk_reserve(q3_handle *h, int k) {
+    if (k <= h->tk_cap) return 0;
+    if (h->tk_ids) cudaFree(h->tk_ids);
+    h->tk_ids = nullptr;
+    h->tk_lps = nullptr;
+    h->tk_cap = 0;
+    const size_t n = (size_t)h->cfg.seq_len * k;
+    cudaError_t e = cudaMalloc((void **)&h->tk_ids, n * 8);
+    if (e != cudaSuccess) {
+        h->tk_ids = nullptr;
+        cudaGetLastError();
+        return fail(Q3_ECUDA, "top-k buffers for k %d: %s", k, cudaGetErrorString(e));
+    }
+    h->tk_lps = (float *)(h->tk_ids + n);
+    h->tk_cap = k;
+    return 0;
+}
+
 static void launch_logprobs(q3_handle *h, const float *logits, int rows, int out0) {
-    k_logprobs<<<rows, LP_THREADS, 0, h->stream>>>(logits, h->cfg.vocab_size, (size_t)h->cfg.vocab_size, h->sc_targets + out0,
-                                                  h->sc_want_lp ? h->sc_lp + out0 : nullptr, h->sc_argmax + out0);
+    const int V = h->cfg.vocab_size, k = h->tk_k;
+    float *lp = h->sc_want_lp ? h->sc_lp + out0 : nullptr;
+    if (k)
+        k_topk_logprobs<<<rows, LP_THREADS, 0, h->stream>>>(logits, V, (size_t)V, k, h->tk_ids + (size_t)out0 * k,
+                                                            h->tk_lps + (size_t)out0 * k, h->sc_targets + out0, lp, h->sc_argmax + out0);
+    else
+        k_logprobs<<<rows, LP_THREADS, 0, h->stream>>>(logits, V, (size_t)V, h->sc_targets + out0, lp, h->sc_argmax + out0);
 }
 
 // rows [0, T) of pf_x (positions out0 .. out0 + T - 1 of the q3_score call): final RMSNorm + quantise into rows [0, Tc) of
@@ -1328,6 +1357,7 @@ struct TpBlob {
     cudaIpcMemHandle_t ipc;
 };
 static_assert(sizeof(TpBlob) <= 256, "blob too large");
+static_assert(TOPK_MAX == Q3_TOPK_MAX, "k_topk_logprobs is built for Q3_TOPK_MAX");
 extern "C" size_t q3_tp_blob_size(void) { return 256; }
 
 extern "C" int q3_tp_export(q3_handle *h, void *blob_out) {
@@ -1406,6 +1436,7 @@ extern "C" void q3_destroy(q3_handle *h) {
     }
     prefill_release(h);
     if (h->sc_logits) cudaFree(h->sc_logits);
+    if (h->tk_ids) cudaFree(h->tk_ids);
     for (void *p : h->peer_maps) cudaIpcCloseMemHandle(p);
     for (void *p : h->allocs) cudaFree(p);
     if (h->h_logits) cudaFreeHost(h->h_logits);
@@ -1715,10 +1746,18 @@ extern "C" int q3_bench_prefill(q3_handle *h, const int *tokens, int n, int pos0
     return finish_call(h);
 }
 
-extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out) {
+// q3_score (k 0) and q3_score_topk (k 1 .. Q3_TOPK_MAX, ids / lps required)
+static int score_impl(q3_handle *h, const int *tokens, int n, int pos0, int k, int *ids_out, float *lps_out, const int *targets,
+                      float *logprobs_out, int *argmax_out) {
     int rc = check_prompt(h, tokens, n, pos0);
     if (rc) return rc;
-    if (!logprobs_out && !argmax_out) return fail(Q3_EINVAL, "q3_score needs logprobs_out or argmax_out");
+    if (k) {
+        if (k < 1 || k > Q3_TOPK_MAX || k > h->cfg.vocab_size)
+            return fail(Q3_EINVAL, "k %d outside 1 .. min(%d, vocab %d)", k, Q3_TOPK_MAX, h->cfg.vocab_size);
+        if (!ids_out || !lps_out) return fail(Q3_EINVAL, "q3_score_topk needs topk_ids_out and topk_logprobs_out");
+    } else if (!logprobs_out && !argmax_out) {
+        return fail(Q3_EINVAL, "q3_score needs logprobs_out or argmax_out");
+    }
     if (logprobs_out && !targets) return fail(Q3_EINVAL, "logprobs_out needs targets");
     const int V = h->cfg.vocab_size;
     if (logprobs_out)
@@ -1729,7 +1768,9 @@ extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const 
     if (h->tp_size > 1 && !batched) return fail(Q3_EUNSUPPORTED, "q3_score under tensor parallelism needs the batched prefill path");
     CK(cudaSetDevice(h->device));
     if ((rc = score_reserve(h, batched, n))) return rc;
+    if (k && (rc = topk_reserve(h, k))) return rc;
     h->sc_want_lp = logprobs_out != nullptr;
+    h->tk_k = k;
     if (logprobs_out) CK(cudaMemcpyAsync(h->sc_targets, targets, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
     if (batched) {
         if ((rc = prefill_chunks(h, tokens, n, pos0, true))) return rc;
@@ -1742,8 +1783,22 @@ extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const 
     }
     if (logprobs_out) CK(cudaMemcpyAsync(logprobs_out, h->sc_lp, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
     if (argmax_out) CK(cudaMemcpyAsync(argmax_out, h->sc_argmax, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (k) {
+        CK(cudaMemcpyAsync(ids_out, h->tk_ids, (size_t)n * k * 4, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(lps_out, h->tk_lps, (size_t)n * k * 4, cudaMemcpyDeviceToHost, h->stream));
+    }
     CK(cudaGetLastError());
     return finish_call(h);
+}
+
+extern "C" int q3_score(q3_handle *h, const int *tokens, int n, int pos0, const int *targets, float *logprobs_out, int *argmax_out) {
+    return score_impl(h, tokens, n, pos0, 0, nullptr, nullptr, targets, logprobs_out, argmax_out);
+}
+
+extern "C" int q3_score_topk(q3_handle *h, const int *tokens, int n, int pos0, int k, int *topk_ids_out, float *topk_logprobs_out,
+                             const int *targets, float *logprobs_out, int *argmax_out) {
+    if (k == 0) return fail(Q3_EINVAL, "k must be at least 1"); // k 0 selects q3_score's path in score_impl
+    return score_impl(h, tokens, n, pos0, k, topk_ids_out, topk_logprobs_out, targets, logprobs_out, argmax_out);
 }
 
 extern "C" int q3_reset(q3_handle *h) {
@@ -1962,6 +2017,36 @@ extern "C" int q3_op_logprobs(int device, const float *logits, int rows, int n, 
     if (logprobs_out) CK(cudaMemcpy(dt.p, targets, (size_t)rows * 4, cudaMemcpyHostToDevice));
     k_logprobs<<<rows, LP_THREADS>>>(dl.as<float>(), n, (size_t)n, dt.as<int>(), logprobs_out ? dlp.as<float>() : nullptr, dam.as<int>());
     CK(cudaGetLastError());
+    if (logprobs_out) CK(cudaMemcpy(logprobs_out, dlp.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
+    if (argmax_out) CK(cudaMemcpy(argmax_out, dam.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
+    return Q3_OK;
+}
+
+// q3_score_topk's reduction on host-supplied logits [rows][n]: the k largest entries of every row (descending value, ties to
+// the larger index) with their log-softmax, and optionally q3_op_logprobs' two outputs from the same pass
+extern "C" int q3_op_topk_logprobs(int device, const float *logits, int rows, int n, int k, const int *targets, int *ids_out,
+                                   float *lps_out, float *logprobs_out, int *argmax_out) {
+    if (!logits || rows <= 0 || n <= 0) return fail(Q3_EINVAL, "bad top-k arguments");
+    if (k < 1 || k > Q3_TOPK_MAX || k > n) return fail(Q3_EINVAL, "k %d outside 1 .. min(%d, n %d)", k, Q3_TOPK_MAX, n);
+    if (!ids_out || !lps_out) return fail(Q3_EINVAL, "q3_op_topk_logprobs needs ids_out and lps_out");
+    if (logprobs_out && !targets) return fail(Q3_EINVAL, "logprobs_out needs targets");
+    if (logprobs_out)
+        for (int r = 0; r < rows; r++)
+            if (targets[r] < 0 || targets[r] >= n) return fail(Q3_EINVAL, "index out of bounds: target %d (n %d)", targets[r], n);
+    CK(cudaSetDevice(device));
+    DevBuf dl, dt, dlp, dam, di, dv;
+    int rc;
+    const size_t rk = (size_t)rows * k;
+    if ((rc = dl.alloc((size_t)rows * n * 4)) || (rc = dt.alloc((size_t)rows * 4)) || (rc = dlp.alloc((size_t)rows * 4)) ||
+        (rc = dam.alloc((size_t)rows * 4)) || (rc = di.alloc(rk * 4)) || (rc = dv.alloc(rk * 4)))
+        return rc;
+    CK(cudaMemcpy(dl.p, logits, (size_t)rows * n * 4, cudaMemcpyHostToDevice));
+    if (logprobs_out) CK(cudaMemcpy(dt.p, targets, (size_t)rows * 4, cudaMemcpyHostToDevice));
+    k_topk_logprobs<<<rows, LP_THREADS>>>(dl.as<float>(), n, (size_t)n, k, di.as<int>(), dv.as<float>(), dt.as<int>(),
+                                          logprobs_out ? dlp.as<float>() : nullptr, argmax_out ? dam.as<int>() : nullptr);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(ids_out, di.p, rk * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(lps_out, dv.p, rk * 4, cudaMemcpyDeviceToHost));
     if (logprobs_out) CK(cudaMemcpy(logprobs_out, dlp.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
     if (argmax_out) CK(cudaMemcpy(argmax_out, dam.p, (size_t)rows * 4, cudaMemcpyDeviceToHost));
     return Q3_OK;

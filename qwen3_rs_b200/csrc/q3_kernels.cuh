@@ -737,12 +737,11 @@ __device__ __forceinline__ LpPart lp_shfl(const LpPart &p, int o) {
     return q;
 }
 
-__global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict__ logits, int n, size_t ld,
-                                                         const int *__restrict__ targets, float *lp_out, int *argmax_out) {
-    __shared__ LpPart red[LP_THREADS / 32];
-    const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const float *x = logits + (size_t)row * ld;
-    LpPart p{(long long)0x8000000000000000LL, -INFINITY, 0.0f};
+// One thread's streaming pass over its elements x[tid], x[tid + LP_THREADS], ... of a row of n: the running max, the
+// rescaled sum and the key of the last maximum.  each(i, v) sees every element the thread folds (k_topk_logprobs' histogram).
+template <class F>
+__device__ __forceinline__ void lp_accumulate(LpPart &p, const float *__restrict__ x, int n, int tid, F each) {
+    p = LpPart{(long long)0x8000000000000000LL, -INFINITY, 0.0f};
     for (int base = tid; base < n; base += LP_BATCH * LP_THREADS) {
         float v[LP_BATCH];
 #pragma unroll
@@ -754,6 +753,7 @@ __global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict
         for (int k = 0; k < LP_BATCH; k++) {
             const int i = base + k * LP_THREADS;
             if (i < n) {
+                each(i, v[k]);
                 const long long key = ((long long)total_key(v[k]) << 32) | (unsigned)i;
                 if (key > p.key) { // new maximum (or an equal value at a later index: expf(0) = 1 either way)
                     p.s = (p.s == 0.0f ? 0.0f : p.s * expf(p.m - v[k])) + 1.0f;
@@ -765,6 +765,14 @@ __global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict
             }
         }
     }
+}
+__global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict__ logits, int n, size_t ld,
+                                                         const int *__restrict__ targets, float *lp_out, int *argmax_out) {
+    __shared__ LpPart red[LP_THREADS / 32];
+    const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *x = logits + (size_t)row * ld;
+    LpPart p;
+    lp_accumulate(p, x, n, tid, [](int, float) {});
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) lp_combine(p, lp_shfl(p, o));
     if (lane == 0) red[warp] = p;
@@ -777,6 +785,172 @@ __global__ void __launch_bounds__(LP_THREADS) k_logprobs(const float *__restrict
             if (lp_out) lp_out[row] = __fsub_rn(__fsub_rn(x[targets[row]], p.m), logf(p.s));
             if (argmax_out) argmax_out[row] = (int)(p.key & 0xffffffffLL);
         }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// Per-row top-k log-probabilities (q3_score_topk, q3_op_topk_logprobs).  One CTA per row, k <= TOPK_MAX.  The k entries
+// are the k largest 64-bit keys (total_key(x) << 32) | index -- descending value, ties to the larger index -- so ids[0] is
+// k_logprobs' argmax and the selection is a function of the row alone.  lps[j] = (x[ids[j]] - m) - logf(s) with m, s from
+// k_logprobs' own accumulation (lp_accumulate) and combine tree: at ids[j] == target it is q3_score's value bit for bit.
+// Selection is a radix select on the key as an unsigned number, 11 bits per digit from the top:
+//   1. the (m, s) pass also counts the top digit of every key into a shared histogram;
+//   2. a scan finds the bin of the k-th largest key; all keys above that bin are in the top k;
+//   3. if those keys plus the bin's hold at most TOPK_CAP, a second read gathers them and a bitonic sort orders them;
+//   4. otherwise the next digit is counted over the bin's keys (another read of the row), down into the index bits.
+// Keys are unique, so the bin of the last digit holds one key and the loop ends: an all-equal row takes 5 counting reads.
+// ------------------------------------------------------------------------------------------
+constexpr int TOPK_MAX = 64;
+constexpr int TOPK_DIGIT = 11;                // bits per radix digit (the last one, bits 8..0, has 9)
+constexpr int TOPK_BINS = 1 << TOPK_DIGIT;
+constexpr int TOPK_CAP = 2048;                // candidates sorted in shared memory (16 KB)
+static_assert(TOPK_BINS == 4 * LP_THREADS, "the bin scan gives each thread 4 bins");
+
+// the key of k_argmax / k_logprobs as an unsigned number (same order)
+__device__ __forceinline__ unsigned long long topk_key(float v, int i) {
+    return ((unsigned long long)((unsigned)total_key(v) ^ 0x80000000u) << 32) | (unsigned)i;
+}
+
+__global__ void __launch_bounds__(LP_THREADS) k_topk_logprobs(const float *__restrict__ logits, int n, size_t ld, int k,
+                                                              int *ids, float *lps, const int *__restrict__ targets,
+                                                              float *lp_out, int *argmax_out) {
+    __shared__ LpPart red[LP_THREADS / 32];
+    __shared__ unsigned hist[TOPK_BINS];
+    __shared__ unsigned long long cand[TOPK_CAP];
+    __shared__ unsigned wsum[LP_THREADS / 32];
+    __shared__ float s_m, s_s;
+    __shared__ unsigned s_bin, s_gt, s_count;
+    const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *x = logits + (size_t)row * ld;
+    for (int b = tid; b < TOPK_BINS; b += LP_THREADS) hist[b] = 0;
+    if (tid == 0) s_count = 0;
+    __syncthreads();
+    LpPart p;
+    lp_accumulate(p, x, n, tid, [&](int, float v) {
+        atomicAdd(&hist[((unsigned)total_key(v) ^ 0x80000000u) >> (32 - TOPK_DIGIT)], 1u);
+    });
+    // k_logprobs' combine tree, step for step (its __syncthreads also completes the histogram)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lp_combine(p, lp_shfl(p, o));
+    if (lane == 0) red[warp] = p;
+    __syncthreads();
+    if (warp == 0) {
+        p = lane < LP_THREADS / 32 ? red[lane] : LpPart{(long long)0x8000000000000000LL, -INFINITY, 0.0f};
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) lp_combine(p, lp_shfl(p, o));
+        if (lane == 0) {
+            s_m = p.m;
+            s_s = p.s;
+            if (lp_out) lp_out[row] = __fsub_rn(__fsub_rn(x[targets[row]], p.m), logf(p.s));
+            if (argmax_out) argmax_out[row] = (int)(p.key & 0xffffffffLL);
+        }
+    }
+    unsigned long long sel = 0; // the key's digits chosen so far: every key in the top k is >= sel << shift
+    int shift = 64;             // key bits below the chosen digits
+    unsigned above = 0;         // keys above the chosen prefix: all in the top k
+    unsigned need = (unsigned)k; // how many of the top k are still to be found under the chosen prefix
+    for (;;) {
+        const int width = shift >= TOPK_DIGIT ? TOPK_DIGIT : shift;
+        // the bin holding the need-th largest key of this digit: each thread owns 4 bins, thread 0 the top ones
+        unsigned h[4], c = 0;
+#pragma unroll
+        for (int j = 0; j < 4; j++) c += h[j] = hist[TOPK_BINS - 1 - 4 * tid - j];
+        unsigned incl = c;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += t;
+        }
+        if (lane == 31) wsum[warp] = incl;
+        __syncthreads();
+        unsigned acc = incl - c;
+        for (int w = 0; w < warp; w++) acc += wsum[w];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (acc < need && acc + h[j] >= need) {
+                s_bin = TOPK_BINS - 1 - 4 * tid - j;
+                s_gt = acc;
+            }
+            acc += h[j];
+        }
+        __syncthreads();
+        const unsigned bin = s_bin, gt = s_gt;
+        shift -= width;
+        sel = (sel << width) | bin;
+        above += gt;
+        if (above + hist[bin] <= TOPK_CAP) break;
+        need -= gt;
+        // the next digit, counted over the keys under the chosen prefix (one more read of the row)
+        const int nw = shift >= TOPK_DIGIT ? TOPK_DIGIT : shift;
+        __syncthreads(); // every thread has read hist[bin]
+        for (int b = tid; b < TOPK_BINS; b += LP_THREADS) hist[b] = 0;
+        __syncthreads();
+        for (int base = tid; base < n; base += LP_BATCH * LP_THREADS) {
+            float v[LP_BATCH];
+#pragma unroll
+            for (int j = 0; j < LP_BATCH; j++) {
+                const int i = base + j * LP_THREADS;
+                v[j] = i < n ? x[i] : 0.0f;
+            }
+#pragma unroll
+            for (int j = 0; j < LP_BATCH; j++) {
+                const int i = base + j * LP_THREADS;
+                const unsigned long long key = topk_key(v[j], i);
+                if (i < n && (key >> shift) == sel) atomicAdd(&hist[(unsigned)(key >> (shift - nw)) & ((1u << nw) - 1)], 1u);
+            }
+        }
+        __syncthreads();
+    }
+    // gather every key >= lo (above + hist[bin] of them, at least k) into shared memory, warp by warp
+    const unsigned long long lo = sel << shift;
+    for (int base0 = 0; base0 < n; base0 += LP_BATCH * LP_THREADS) { // uniform trip count: the ballots see full warps
+        float v[LP_BATCH];
+#pragma unroll
+        for (int j = 0; j < LP_BATCH; j++) {
+            const int i = base0 + tid + j * LP_THREADS;
+            v[j] = i < n ? x[i] : 0.0f;
+        }
+#pragma unroll
+        for (int j = 0; j < LP_BATCH; j++) {
+            const int i = base0 + tid + j * LP_THREADS;
+            const unsigned long long key = topk_key(v[j], i);
+            const bool take = i < n && key >= lo;
+            const unsigned mask = __ballot_sync(0xffffffffu, take);
+            if (mask) {
+                unsigned off = 0;
+                if (lane == 0) off = atomicAdd(&s_count, (unsigned)__popc(mask));
+                off = __shfl_sync(0xffffffffu, off, 0) + __popc(mask & ((1u << lane) - 1));
+                if (take && off < TOPK_CAP) cand[off] = key;
+            }
+        }
+    }
+    __syncthreads();
+    const int cnt = (int)min(s_count, (unsigned)TOPK_CAP);
+    int npad = 1;
+    while (npad < cnt) npad <<= 1;
+    for (int i = cnt + tid; i < npad; i += LP_THREADS) cand[i] = 0; // below every key that can be among the top k
+    __syncthreads();
+    // bitonic sort, descending
+    for (int kk = 2; kk <= npad; kk <<= 1) {
+        for (int j = kk >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < npad; i += LP_THREADS) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const unsigned long long a = cand[i], b = cand[ixj];
+                    if ((a < b) == ((i & kk) == 0)) {
+                        cand[i] = b;
+                        cand[ixj] = a;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    const float m = s_m, ls = logf(s_s);
+    for (int j = tid; j < k; j += LP_THREADS) {
+        const int id = (int)(cand[j] & 0xffffffffu);
+        ids[(size_t)row * k + j] = id;
+        lps[(size_t)row * k + j] = __fsub_rn(__fsub_rn(x[id], m), ls);
     }
 }
 

@@ -76,6 +76,7 @@ ABI = {
     "q3_prefill": (_i, [_vp, _vp, _i, _i, _vp]),
     "q3_bench_prefill": (_i, [_vp, _vp, _i, _i, C.POINTER(_f)]),
     "q3_score": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "q3_score_topk": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "q3_reset": (_i, [_vp]),
     "q3_logits_device": (_vp, [_vp]),
     "q3_logits_host": (_vp, [_vp]),
@@ -99,6 +100,7 @@ ABI = {
     "q3_bench_gemm_q8": (_i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(_f)]),
     "q3_op_prefill_attention": (_i, [_i, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "q3_op_logprobs": (_i, [_i, _vp, _i, _i, _vp, _vp, _vp]),
+    "q3_op_topk_logprobs": (_i, [_i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "q3_op_rmsnorm": (_i, [_i, _vp, _vp, _i, _vp]),
     "q3_op_quantize_q80": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
     "q3_op_quantize_q80_dev": (_i, [_i, _vp, _sz, _i, _vp, _vp]),
@@ -222,6 +224,24 @@ class Transformer:
         am = np.empty(t.size, np.int32) if want_argmax else None
         _check(load_library().q3_score(self._h, _ptr(t), t.size, int(pos0), _ptr(tg), _ptr(lp), _ptr(am)))
         return lp, am
+
+    def score_topk(self, tokens: Sequence[int], k: int, targets: Optional[Sequence[int]] = None, pos0: int = 0,
+                   want_argmax: bool = True):
+        """q3_score_topk: score() plus the k most likely tokens at every position -> (ids [n, k], lps [n, k], logprobs,
+        argmax).  Row i of ids is in descending probability, equal values with the larger id first (ids[:, 0] is the argmax);
+        lps holds their natural-log probabilities.  logprobs / argmax as in score() and bit-identical to its results."""
+        t = np.ascontiguousarray(tokens, np.int32).reshape(-1)
+        tg = None if targets is None else np.ascontiguousarray(targets, np.int32).reshape(-1)
+        if tg is not None and tg.size != t.size:
+            raise ValueError(f"score_topk: {tg.size} targets for {t.size} tokens")
+        k = _topk_k(k)
+        ids = np.empty((t.size, k), np.int32)
+        lps = np.empty((t.size, k), np.float32)
+        lp = None if tg is None else np.empty(t.size, np.float32)
+        am = np.empty(t.size, np.int32) if want_argmax else None
+        _check(load_library().q3_score_topk(self._h, _ptr(t), t.size, int(pos0), k, _ptr(ids), _ptr(lps), _ptr(tg), _ptr(lp),
+                                            _ptr(am)))
+        return ids, lps, lp, am
 
     def reset(self) -> None:
         _check(load_library().q3_reset(self._h))
@@ -453,6 +473,33 @@ def op_logprobs(logits, targets=None, want_argmax: bool = True, device: int = 0)
     am = np.empty(rows, np.int32) if want_argmax else None
     _check(load_library().q3_op_logprobs(device, _ptr(a), rows, n, _ptr(tg), _ptr(lp), _ptr(am)))
     return lp, am
+
+
+TOPK_MAX = 64  # Q3_TOPK_MAX in include/qwen3_cuda.h
+
+
+def _topk_k(k) -> int:
+    if isinstance(k, bool) or int(k) != k or not 1 <= k <= TOPK_MAX:
+        raise ValueError(f"k must be an integer in 1 .. {TOPK_MAX}, got {k!r}")
+    return int(k)
+
+
+def op_topk_logprobs(logits, k: int, targets=None, want_argmax: bool = True, device: int = 0):
+    """q3_score_topk's reduction on logits [rows][n] -> (ids [rows, k], lps [rows, k], log softmax(row)[targets[r]] or None,
+    last argmax of each row or None)."""
+    a = np.ascontiguousarray(logits, np.float32)
+    a = a.reshape(1, -1) if a.ndim == 1 else a
+    rows, n = a.shape
+    tg = None if targets is None else np.ascontiguousarray(targets, np.int32).reshape(-1)
+    if tg is not None and tg.size != rows:
+        raise ValueError(f"op_topk_logprobs: {tg.size} targets for {rows} rows")
+    k = _topk_k(k)
+    ids = np.empty((rows, k), np.int32)
+    lps = np.empty((rows, k), np.float32)
+    lp = None if tg is None else np.empty(rows, np.float32)
+    am = np.empty(rows, np.int32) if want_argmax else None
+    _check(load_library().q3_op_topk_logprobs(device, _ptr(a), rows, n, k, _ptr(tg), _ptr(ids), _ptr(lps), _ptr(lp), _ptr(am)))
+    return ids, lps, lp, am
 
 
 def op_rmsnorm(x, w, device: int = 0):

@@ -27,6 +27,9 @@ extern "C" {
     fn q3_prefill(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, last_logits_host: *mut c_float) -> c_int;
     fn q3_score(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, targets: *const c_int, logprobs_out: *mut c_float,
                 argmax_out: *mut c_int) -> c_int;
+    fn q3_score_topk(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, k: c_int, topk_ids_out: *mut c_int,
+                     topk_logprobs_out: *mut c_float, targets: *const c_int, logprobs_out: *mut c_float, argmax_out: *mut c_int)
+                     -> c_int;
     fn q3_reset(h: *mut Q3Handle) -> c_int;
     fn q3_logits_host(h: *mut Q3Handle) -> *mut c_float;
 }
@@ -112,6 +115,25 @@ impl CudaTransformer {
             panic!("{}", last_error());
         }
         (lp, am.into_iter().map(|a| a as usize).collect())
+    }
+
+    /// The `k` most likely tokens at every position of `tokens` (positions pos0..), in one batched pass: for each position
+    /// `k` (token, natural-log probability) pairs, most likely first, equal values with the larger token id first
+    /// (1 <= k <= min(64, vocab_size)).  The cache is left as by `score`.
+    pub fn score_topk(&mut self, tokens: &[usize], k: usize, pos0: usize) -> Vec<Vec<(usize, f32)>> {
+        let ids: Vec<c_int> = tokens.iter().map(|&t| t as c_int).collect();
+        let mut top = vec![0 as c_int; ids.len() * k];
+        let mut lps = vec![0.0f32; ids.len() * k];
+        let rc = unsafe {
+            q3_score_topk(self.handle, ids.as_ptr(), ids.len() as c_int, pos0 as c_int, k as c_int, top.as_mut_ptr(),
+                          lps.as_mut_ptr(), std::ptr::null(), std::ptr::null_mut(), std::ptr::null_mut())
+        };
+        if rc != 0 {
+            panic!("{}", last_error());
+        }
+        top.chunks(k.max(1)).zip(lps.chunks(k.max(1)))
+            .map(|(t, l)| t.iter().zip(l).map(|(&i, &v)| (i as usize, v)).collect())
+            .collect()
     }
 
     /// Zero the KV cache (a fresh `TransformerBlockBuffers`, qwen3.rs:439-440).

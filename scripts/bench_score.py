@@ -9,9 +9,11 @@ Per model, one JSON line:
   lm_head_gemm_ms   the lm_head GEMM alone in the same row chunks (q3_bench_gemm_q8, best of reps), for the split of head_ms
   scored_tok_s      T / score_ms
   forward_ms_per_token  256 sequential q3_forward calls with host logits (the way to get the same numbers without q3_score)
+With --topk K1,K2,..: q3_score_topk with targets at each k, timed like score_ms with the calls of every k and q3_score's
+alternated rep by rep (topk_ms, median; topk_extra_ms = topk_ms - the alternated q3_score's median).
 The card's name, power limit and max SM clock are read in the same run.
 
-usage: python scripts/bench_score.py [--models qwen3-4b,qwen3-8b] [--T 2048] [--reps 7]"""
+usage: python scripts/bench_score.py [--models qwen3-4b,qwen3-8b] [--T 2048] [--reps 7] [--topk 1,20,64]"""
 import argparse
 import os
 import subprocess
@@ -39,7 +41,29 @@ def card():
         return {"gpu": torch.cuda.get_device_name(0), "power_limit": f"unavailable ({e!r})"}
 
 
-def run(model, Tn, reps):
+def timed(fn):
+    t0 = time.perf_counter()
+    out = fn()
+    return (time.perf_counter() - t0) * 1e3, out
+
+
+def run_topk(m, t, tg, ks, reps):
+    """q3_score and q3_score_topk at every k, alternated rep by rep after one warm-up call each."""
+    fns = {0: lambda: m.score(t, targets=tg)}
+    for k in ks:
+        fns[k] = lambda k=k: m.score_topk(t, k, targets=tg)
+    for f in fns.values():
+        f()
+    ms = {k: [] for k in fns}
+    for _ in range(reps):
+        for k, f in fns.items():
+            ms[k].append(timed(f)[0])
+    base = float(np.median(ms[0]))
+    return {"topk_score_ms": base, "topk_ms": {k: float(np.median(ms[k])) for k in ks},
+            "topk_extra_ms": {k: float(np.median(ms[k])) - base for k in ks}, "topk_ms_all": {k: ms[k] for k in ks}}
+
+
+def run(model, Tn, reps, ks=()):
     shape = synth.SHAPES[model]
     m = T.TransformerBuilder.new(bench.bench_checkpoint(model, 64)).with_ctx_length(Tn + 8).build()
     try:
@@ -58,6 +82,7 @@ def run(model, Tn, reps):
         gemm_ms = 0.0
         for r0 in range(0, Tn, SCORE_ROWS):
             gemm_ms += T.bench_gemm_q8(min(SCORE_ROWS, Tn - r0), shape.vocab_size, shape.dim, 64, 0, reps)
+        topk = run_topk(m, t, tg, ks, reps) if ks else {}
         m.reset()
         lg = np.empty(shape.vocab_size, np.float32)
         m.forward(t[0], 0)
@@ -68,7 +93,7 @@ def run(model, Tn, reps):
         return {"model": model, "group_size": 64, "T": Tn, "prefill_ms": pf_ms, "score_ms": sc_ms, "score_ms_all": sc,
                 "head_ms": head_ms, "head_int8_TOPS": ops / head_ms / 1e9, "lm_head_gemm_ms": gemm_ms,
                 "lm_head_gemm_int8_TOPS": ops / gemm_ms / 1e9, "scored_tok_s": Tn / sc_ms * 1e3,
-                "forward_ms_per_token": fwd_ms, "mean_logprob": float(np.mean(lp)), "finite": bool(np.isfinite(lp).all() and np.isfinite(lg).all())}
+                "forward_ms_per_token": fwd_ms, "mean_logprob": float(np.mean(lp)), "finite": bool(np.isfinite(lp).all() and np.isfinite(lg).all()), **topk}
     finally:
         m.close()
 
@@ -78,10 +103,12 @@ def main():
     ap.add_argument("--models", default="qwen3-4b,qwen3-8b")
     ap.add_argument("--T", type=int, default=2048)
     ap.add_argument("--reps", type=int, default=7)
+    ap.add_argument("--topk", default="", help="comma-separated k values for q3_score_topk, e.g. 1,20,64")
     a = ap.parse_args()
+    ks = [int(k) for k in a.topk.split(",") if k]
     info = card()
     for model in a.models.split(","):
-        bench.emit({**run(model, a.T, a.reps), **info})
+        bench.emit({**run(model, a.T, a.reps, ks), **info})
 
 
 if __name__ == "__main__":
