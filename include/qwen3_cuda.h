@@ -97,6 +97,36 @@ int q3_forward_argmax(q3_handle *h, int token, int pos, int *next_token);
  * (first_token, pos0). */
 int q3_decode_greedy(q3_handle *h, int first_token, int pos0, int n, int *tokens_out);
 
+/* Extension: n decode steps in one pass over the weights (the verification step of speculative decoding).
+ * Runs tokens[i] at position pos0+i for i in [0, n), 1 <= n <= Q3_MULTI_MAX, in one pass over the weights.
+ * argmax_out[i] (required) = last index of the maximum of the logits after tokens[0..i]; logits_host (optional) = those
+ * logits, [n][vocab_size].  Fast mode: every row (logits, argmax, the K/V cache row pos0+i) is bit-identical to what
+ * q3_forward on the multi-kernel path (q3_set_decode_path(h, 0)) computes for the same token, position and cache,
+ * whatever path q3_forward is set to.  Exact mode, or any non-zero exact mask: the n single-token steps of that mode
+ * are run one after another (same results).  Tensor-parallel handle: Q3_EUNSUPPORTED.  Arguments are checked before
+ * any device work, as in q3_prefill.  q3_logits_device() is unspecified afterwards.  The per-token buffers are allocated
+ * on the first call; the graph of each n is captured on its first use. */
+#define Q3_MULTI_MAX 8
+int q3_forward_multi(q3_handle *h, const int *tokens, int n, int pos0, int *argmax_out, float *logits_host);
+
+/* Timing helper: reps q3_forward_multi steps of n tokens (all token id 0) at pos0 .. pos0+n-1, after an untimed warm-up, CUDA
+ * events on the launch stream; total milliseconds.  Writes the K/V rows of those positions. */
+int q3_bench_multi(q3_handle *h, int n, int pos0, int reps, float *ms_out);
+
+/* Extension: greedy decoding with a draft model.  n greedy tokens of `target` after first_token at pos0, drafting k tokens per
+ * round with `draft` (a second handle on the same device, same vocab_size, e.g. Qwen3-0.6B for Qwen3-8B) and verifying them with
+ * q3_forward_multi.  Each round: kk = min(k, n - produced - 1); the draft proposes d[0..kk) with q3_decode_greedy on whichever
+ * path it is set to; the target computes a[0..kk] for [tok, d...] at pos; the longest prefix j with d[i] == a[i] is accepted
+ * and d[0..j), a[j] are emitted; when all kk were accepted the draft runs one more step to write its cache row for d[kk-1].
+ * tokens_out: bit-identical to q3_decode_greedy(target, first_token, pos0, n) on the multi-kernel path, for ANY draft
+ * (its weights and its cache contents only change how many tokens are accepted).  The target's KV rows [pos0, pos0+n) end
+ * up bit-identical to what that call leaves; no target row at or after pos0+n is written.  1 <= k <= Q3_MULTI_MAX - 1.
+ * rounds_out / drafted_out / accepted_out: optional statistics.  Both handles: tp_size 1; distinct; on the same device;
+ * pos0+n <= both seq_len.
+ * Every argument is checked before any device work (Q3_EINVAL; Q3_EUNSUPPORTED for a tensor-parallel handle). */
+int q3_decode_speculative(q3_handle *target, q3_handle *draft, int first_token, int pos0, int n, int k, int *tokens_out,
+                          int *rounds_out, int *drafted_out, int *accepted_out);
+
 /* Extension (SURVEY.md §8f-1, second half): the reference's Sampler (sampler.rs) on the device.
  * q3_sampler_set = Sampler::new(vocab, temperature, topp, rng_seed) (:30-41; the same argument checks, Q3_EINVAL instead
  * of the asserts).  q3_forward_sample = forward + Sampler::sample (:116-136): temperature 0 -> argmax; otherwise

@@ -17,7 +17,8 @@
 //   tokenizer.rs          Tokenizer (byte-level BPE)         qwen3::Tokenizer (same results; vocabulary lookups hashed)
 //   generation.rs:188-195 render_prompt                      qwen3::render_prompt
 //
-// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill, score, score_topk.
+// Extensions of the drop-in (SURVEY section 8f): forward_argmax, decode_greedy, prefill, score, score_topk, forward_multi,
+// decode_speculative.
 //
 // Errors: construction failures throw qwen3::Error (the reference returns anyhow::Error with the same
 // message text); forward() with an out-of-range token / pos throws (the reference panics on the slice
@@ -148,6 +149,35 @@ public:
                                     targets.empty() ? nullptr : targets.data(), targets.empty() ? nullptr : r.target_logprobs.data(),
                                     r.argmax.data()));
         return r;
+    }
+    // q3_forward_multi: tokens[i] at position pos0 + i (1 <= n <= Q3_MULTI_MAX) in one pass over the weights; the greedy token
+    // after each prefix, and with want_logits the logits rows [n][vocab_size] (else empty).
+    struct Multi {
+        std::vector<int> argmax;
+        std::vector<float> logits;
+    };
+    Multi forward_multi(const std::vector<int> &tokens, size_t pos0, bool want_logits = false) {
+        if (tokens.empty() || tokens.size() > Q3_MULTI_MAX) throw std::invalid_argument("forward_multi: 1 .. Q3_MULTI_MAX tokens");
+        Multi r;
+        r.argmax.resize(tokens.size());
+        if (want_logits) r.logits.resize(tokens.size() * (size_t)cfg_.vocab_size);
+        detail::check(q3_forward_multi(h_, tokens.data(), (int)tokens.size(), (int)pos0, r.argmax.data(),
+                                       want_logits ? r.logits.data() : nullptr));
+        return r;
+    }
+    // q3_decode_speculative: n greedy tokens after first_token at pos0, k (1 .. Q3_MULTI_MAX - 1) drafted per round by `draft`;
+    // the tokens of decode_greedy on the multi-kernel path.  Statistics of the rounds in the optional outputs.
+    struct SpecStats {
+        int rounds = 0, drafted = 0, accepted = 0;
+    };
+    std::vector<int> decode_speculative(Transformer &draft, int first_token, size_t pos0, size_t n, int k, SpecStats *stats = nullptr) {
+        if (k < 1 || k > Q3_MULTI_MAX - 1) throw std::invalid_argument("decode_speculative: k outside 1 .. Q3_MULTI_MAX - 1");
+        std::vector<int> out(n);
+        SpecStats st;
+        detail::check(q3_decode_speculative(h_, draft.h_, first_token, (int)pos0, (int)n, k, out.data(), &st.rounds, &st.drafted,
+                                            &st.accepted));
+        if (stats) *stats = st;
+        return out;
     }
     void reset() { detail::check(q3_reset(h_)); } // zero the KV cache
     q3_handle *handle() { return h_; }

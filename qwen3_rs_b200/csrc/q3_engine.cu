@@ -116,6 +116,14 @@ struct q3_handle {
     int *h_small = nullptr;    // pinned scratch
     cudaStream_t stream = nullptr;
     cudaGraphExec_t g_fwd[32] = {}, g_greedy[32] = {}; // [exact mask]
+    // q3_forward_multi, allocated on its first call: the graph step's per-token state for Q3_MULTI_MAX tokens (m_ctl: tokens,
+    // pos0, per-step (token, position) pairs of the exact-mode fallback, argmax), one graph per token count (fast mode only)
+    float *m_x = nullptr, *m_xb = nullptr, *m_q = nullptr, *m_hb = nullptr, *m_logits = nullptr, *m_part = nullptr;
+    int8_t *m_xq = nullptr, *m_hq = nullptr;
+    float *m_xs = nullptr, *m_hs = nullptr;
+    int *m_ctl = nullptr, *h_mctl = nullptr; // device / pinned host [MCTL_INTS]
+    float *h_mlogits = nullptr;              // pinned [Q3_MULTI_MAX][vocab], allocated when logits are first asked for
+    cudaGraphExec_t g_multi[Q3_MULTI_MAX + 1] = {};
     // Reference-order mask (bit-level parity mode; q3_set_exact = all bits, q3_set_exact_mask = per reduction, for the
     // attribution of int8 flips): 1 RMSNorm sum of squares, 2 GEMV group fold, 4 QK-norm sum of squares,
     // 8 attention (score dots, softmax with glibc expf, value mix), 16 glibc expf in SwiGLU
@@ -374,8 +382,70 @@ static int upload_f32(q3_handle *h, float **dst, const float *src, size_t n) {
     default: break;                                        \
     }
 
+// The buffers one graph decode step works on, [nt] rows each (token t = row t): the handle's single-token state (step_bufs) or
+// q3_forward_multi's Q3_MULTI_MAX-row blocks (multi_bufs).  tokens / pos / argmax are device words: tokens[nt], the position of
+// token 0, argmax[nt].
+struct StepBufs {
+    float *x, *xb, *q, *hb, *logits, *part;
+    int8_t *xq, *hq;
+    float *xs, *hs;
+    int *tokens, *pos, *argmax;
+};
+static StepBufs step_bufs(const q3_handle *h) {
+    return {h->x, h->xb, h->q, h->hb, h->logits, h->attn_part, h->xq, h->hq, h->xs, h->hs, h->d_tokpos, h->d_tokpos + 1, h->d_tokpos + 2};
+}
+// m_ctl layout (ints): [0, 8) tokens, [8] pos0, [16, 32) the exact-mode fallback's (token, position) of each step, [32, 40) argmax
+constexpr int MCTL_POS0 = Q3_MULTI_MAX, MCTL_STEPS = 16, MCTL_ARGMAX = 32, MCTL_INTS = 40;
+static StepBufs multi_bufs(const q3_handle *h) {
+    return {h->m_x, h->m_xb, h->m_q, h->m_hb, h->m_logits, h->m_part, h->m_xq, h->m_hq, h->m_xs, h->m_hs,
+            h->m_ctl, h->m_ctl + MCTL_POS0, h->m_ctl + MCTL_ARGMAX};
+}
+
+// Shared memory of k_gemv for NT tokens: [NT][K] int8 + [NT][K/GS] scales; at most GEMV_MULTI_SMEM (the opt-in maximum of a block)
+constexpr int GEMV_MULTI_SMEM = 227 * 1024;
+#define NT_DISPATCH(nt, CALL)                                 \
+    switch (nt) {                                             \
+    case 2: { constexpr int NT = 2; CALL; } break;            \
+    case 3: { constexpr int NT = 3; CALL; } break;            \
+    case 4: { constexpr int NT = 4; CALL; } break;            \
+    case 5: { constexpr int NT = 5; CALL; } break;            \
+    case 6: { constexpr int NT = 6; CALL; } break;            \
+    case 7: { constexpr int NT = 7; CALL; } break;            \
+    case 8: { constexpr int NT = 8; CALL; } break;            \
+    default: break;                                           \
+    }
+
+template <int GS, int EPI, int NT>
+static void launch_gemv_nt(int num_sms, const GemvArgs &a, size_t smem, cudaStream_t s) {
+    // one wave: each CTA stages the NT token vectors once, as many CTAs per SM as the shared memory admits
+    int occ = 1;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gemv<GS, EPI, false, false, NT>, 256, smem);
+    if (occ < 1) occ = 1;
+    int grid = (a.rows / 2 + 7) / 8;
+    if (grid > num_sms * occ) grid = num_sms * occ;
+    if (grid < 1) grid = 1;
+    k_gemv<GS, EPI, false, false, NT><<<grid, 256, smem, s>>>(a);
+}
+
 template <int GS, int EPI>
-static void launch_gemv_t(int num_sms, int exact, GemvArgs a, cudaStream_t s) {
+static void launch_gemv_t(int num_sms, int exact, GemvArgs a, cudaStream_t s, int nt) {
+    if (nt > 1) { // fast mode only: tokens in groups whose staged vectors fit in shared memory
+        const size_t per = (size_t)a.K + (size_t)(a.K / GS) * 4;
+        const int fit = (int)(GEMV_MULTI_SMEM / per);
+        for (int t0 = 0; t0 < nt;) {
+            const int c = nt - t0 < fit ? nt - t0 : fit;
+            GemvArgs b = a;
+            b.xq = a.xq + (size_t)t0 * a.K;
+            b.xs = a.xs + (size_t)t0 * (a.K / GS);
+            b.tok0 = t0;
+            if (EPI == EPI_QKV) b.q = a.q + (size_t)t0 * a.AH;
+            else b.out = a.out + (size_t)t0 * (EPI == EPI_SWIGLU ? a.rows / 2 : a.rows);
+            if (c == 1) launch_gemv_t<GS, EPI>(num_sms, 0, b, s, 1);
+            else NT_DISPATCH(c, (launch_gemv_nt<GS, EPI, NT>(num_sms, b, (size_t)c * per, s)));
+            t0 += c;
+        }
+        return;
+    }
     int npairs = a.rows / 2;
     int grid = (npairs + 7) / 8;
     int cap = num_sms * 8;
@@ -392,113 +462,115 @@ static void launch_gemv_t(int num_sms, int exact, GemvArgs a, cudaStream_t s) {
         else k_gemv<GS, EPI, false, false><<<grid, 256, smem, s>>>(a);
     }
 }
-// exact: the reference-order mask (q3_handle::exact)
+// exact: the reference-order mask (q3_handle::exact); nt tokens (token-major rows of xq / xs / out / q), nt > 1 in fast mode only
 template <int EPI>
-static void launch_gemv(int gs, int num_sms, int exact, const GemvArgs &a, cudaStream_t s) {
-    GS_DISPATCH(gs, (launch_gemv_t<GS, EPI>(num_sms, exact, a, s)));
+static void launch_gemv(int gs, int num_sms, int exact, const GemvArgs &a, cudaStream_t s, int nt = 1) {
+    GS_DISPATCH(gs, (launch_gemv_t<GS, EPI>(num_sms, exact, a, s, nt)));
 }
 
-static int launch_norm_quant(int gs, int exact, const NormQuantArgs &a, cudaStream_t s) {
+static int launch_norm_quant(int gs, int exact, const NormQuantArgs &a, cudaStream_t s, int nt = 1) {
     if (exact & 1) {
-        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, true><<<1, 1024, (size_t)a.n * 4, s>>>(a)));
+        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, true><<<nt, 1024, (size_t)a.n * 4, s>>>(a)));
     } else {
-        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, false><<<1, 1024, 0, s>>>(a)));
+        GS_DISPATCH(gs, (k_rmsnorm_quant<GS, false><<<nt, 1024, 0, s>>>(a)));
     }
     return 1;
 }
 
-// split-K decode attention of one layer at position d_tokpos[1]: partials of ATTN_MAX_SPLITS CTAs per kv head into attn_part
-static void launch_attn_partial(const q3_handle *h, const float *kc_l, const float *vc_l, cudaStream_t s) {
-    dim3 ag(h->n_kv_l, ATTN_MAX_SPLITS);
-    KV_DISPATCH(h->kv_mul, (k_attn_partial<KVM><<<ag, 128, 0, s>>>(h->q, kc_l, vc_l, h->attn_part, h->d_tokpos + 1, h->KV_l, h->n_heads_l)));
+// split-K decode attention of one layer for nt tokens at positions *pos ..: partials of ATTN_MAX_SPLITS CTAs per (kv head, token)
+static void launch_attn_partial(const q3_handle *h, const StepBufs &b, int nt, const float *kc_l, const float *vc_l, cudaStream_t s) {
+    dim3 ag(h->n_kv_l * nt, ATTN_MAX_SPLITS);
+    KV_DISPATCH(h->kv_mul, (k_attn_partial<KVM><<<ag, 128, 0, s>>>(b.q, kc_l, vc_l, b.part, b.pos, h->KV_l, h->n_heads_l, nt)));
 }
 
-// One transformer block.  Returns the number of kernel launches.
-static int launch_layer(q3_handle *h, int l, bool first_from_embed, cudaStream_t s) {
+// One transformer block for the nt tokens of b.  Returns the number of kernel launches.
+static int launch_layer(q3_handle *h, const StepBufs &b, int nt, int l, bool first_from_embed, cudaStream_t s) {
     const q3_config &c = h->cfg;
     const LayerDev &W = h->layers[l];
     const int gs = c.group_size, dim = c.dim, ns = h->num_sms, ex = h->exact;
-    const int *d_token = h->d_tokpos, *d_pos = h->d_tokpos + 1;
+    const int *d_token = b.tokens, *d_pos = b.pos;
     float *kc_l = h->kc + (size_t)l * c.seq_len * h->KV_l;
     float *vc_l = h->vc + (size_t)l * c.seq_len * h->KV_l;
     int n = 0;
     // attn_norm + quantize (qwen3.rs:134-136); layer 0 also gathers the embedding row (qwen3.rs:64)
     NormQuantArgs na{};
-    na.x = h->x; na.w = W.rms_att; na.q = h->xq; na.s = h->xs; na.n = dim;
+    na.x = b.x; na.w = W.rms_att; na.q = b.xq; na.s = b.xs; na.n = dim;
     if (first_from_embed) { na.embed_q = h->embed.q; na.embed_s = h->embed.s; na.token = d_token; }
-    n += launch_norm_quant(gs, ex, na, s);
+    n += launch_norm_quant(gs, ex, na, s, nt);
     // q, k, v projections (layers.rs:334-336)
     GemvArgs g{};
-    g.wq = W.qkv.q; g.ws = W.qkv.s; g.xq = h->xq; g.xs = h->xs; g.K = dim; g.rows = W.qkv.rows;
-    g.q = h->q; g.kc = kc_l; g.vc = vc_l; g.AH = h->AH_l; g.KV = h->KV_l; g.pos = d_pos;
-    launch_gemv<EPI_QKV>(gs, ns, ex, g, s); n++;
+    g.wq = W.qkv.q; g.ws = W.qkv.s; g.xq = b.xq; g.xs = b.xs; g.K = dim; g.rows = W.qkv.rows;
+    g.q = b.q; g.kc = kc_l; g.vc = vc_l; g.AH = h->AH_l; g.KV = h->KV_l; g.pos = d_pos;
+    launch_gemv<EPI_QKV>(gs, ns, ex, g, s, nt); n++;
     // QK-norm + RoPE (layers.rs:339-340)
     int nh = h->n_heads_l + h->n_kv_l;
+    dim3 rg((nh + 3) / 4, nt);
     if (h->exact & 4)
-        k_qknorm_rope<true><<<(nh + 3) / 4, 128, 0, s>>>(h->q, kc_l, W.q_ln, W.k_ln, h->rope, d_pos, h->n_heads_l, h->n_kv_l, h->KV_l);
+        k_qknorm_rope<true><<<rg, 128, 0, s>>>(b.q, kc_l, W.q_ln, W.k_ln, h->rope, d_pos, h->n_heads_l, h->n_kv_l, h->KV_l);
     else
-        k_qknorm_rope<false><<<(nh + 3) / 4, 128, 0, s>>>(h->q, kc_l, W.q_ln, W.k_ln, h->rope, d_pos, h->n_heads_l, h->n_kv_l, h->KV_l);
+        k_qknorm_rope<false><<<rg, 128, 0, s>>>(b.q, kc_l, W.q_ln, W.k_ln, h->rope, d_pos, h->n_heads_l, h->n_kv_l, h->KV_l);
     n++;
     // attention (layers.rs:343) + quantize (qwen3.rs:152)
-    if (h->exact & 8) {
-        k_attn_ordered<<<h->n_heads_l, 128, 0, s>>>(h->q, kc_l, vc_l, h->att, h->xb, d_pos, h->KV_l, h->kv_mul, c.seq_len);
+    if (h->exact & 8) { // single-token
+        k_attn_ordered<<<h->n_heads_l, 128, 0, s>>>(b.q, kc_l, vc_l, h->att, b.xb, d_pos, h->KV_l, h->kv_mul, c.seq_len);
         int n4 = h->AH_l / 4, grid = (n4 + 255) / 256;
-        GS_DISPATCH(gs, (k_quantize<GS><<<grid, 256, 0, s>>>(h->xb, h->AH_l, h->xq, h->xs)));
+        GS_DISPATCH(gs, (k_quantize<GS><<<grid, 256, 0, s>>>(b.xb, h->AH_l, b.xq, b.xs)));
         n += 2;
     } else {
-        launch_attn_partial(h, kc_l, vc_l, s);
-        GS_DISPATCH(gs, (k_attn_combine_quant<GS><<<h->n_heads_l, 128, 0, s>>>(h->attn_part, d_pos, h->xb, h->xq, h->xs)));
+        launch_attn_partial(h, b, nt, kc_l, vc_l, s);
+        GS_DISPATCH(gs, (k_attn_combine_quant<GS><<<dim3(h->n_heads_l, nt), 128, 0, s>>>(b.part, d_pos, b.xb, b.xq, b.xs)));
         n += 2;
     }
     // o_proj + residual (qwen3.rs:153-156)
     GemvArgs o{};
-    o.wq = W.wo.q; o.ws = W.wo.s; o.xq = h->xq; o.xs = h->xs; o.K = h->AH_l; o.rows = dim; o.out = h->x;
-    launch_gemv<EPI_RESID>(gs, ns, ex, o, s); n++;
+    o.wq = W.wo.q; o.ws = W.wo.s; o.xq = b.xq; o.xs = b.xs; o.K = h->AH_l; o.rows = dim; o.out = b.x;
+    launch_gemv<EPI_RESID>(gs, ns, ex, o, s, nt); n++;
     // ffn_norm + quantize (qwen3.rs:159-161)
     NormQuantArgs nf{};
-    nf.x = h->x; nf.w = W.rms_ffn; nf.q = h->xq; nf.s = h->xs; nf.n = dim;
-    n += launch_norm_quant(gs, ex, nf, s);
+    nf.x = b.x; nf.w = W.rms_ffn; nf.q = b.xq; nf.s = b.xs; nf.n = dim;
+    n += launch_norm_quant(gs, ex, nf, s, nt);
     // gate/up + SwiGLU (layers.rs:468-475)
     GemvArgs gu{};
-    gu.wq = W.w13.q; gu.ws = W.w13.s; gu.xq = h->xq; gu.xs = h->xs; gu.K = dim; gu.rows = W.w13.rows; gu.out = h->hb;
-    launch_gemv<EPI_SWIGLU>(gs, ns, ex, gu, s); n++;
+    gu.wq = W.w13.q; gu.ws = W.w13.s; gu.xq = b.xq; gu.xs = b.xs; gu.K = dim; gu.rows = W.w13.rows; gu.out = b.hb;
+    launch_gemv<EPI_SWIGLU>(gs, ns, ex, gu, s, nt); n++;
     // quantize(hb) (layers.rs:478)
     {
         int n4 = h->H_l / 4, grid = (n4 + 255) / 256;
-        GS_DISPATCH(gs, (k_quantize<GS><<<grid, 256, 0, s>>>(h->hb, h->H_l, h->hq, h->hs)));
+        GS_DISPATCH(gs, (k_quantize<GS><<<dim3(grid, nt), 256, 0, s>>>(b.hb, h->H_l, b.hq, b.hs)));
         n++;
     }
     // down + residual (layers.rs:479, qwen3.rs:175)
     GemvArgs dn{};
-    dn.wq = W.w2.q; dn.ws = W.w2.s; dn.xq = h->hq; dn.xs = h->hs; dn.K = h->H_l; dn.rows = dim; dn.out = h->x;
-    launch_gemv<EPI_RESID>(gs, ns, ex, dn, s); n++;
+    dn.wq = W.w2.q; dn.ws = W.w2.s; dn.xq = b.hq; dn.xs = b.hs; dn.K = h->H_l; dn.rows = dim; dn.out = b.x;
+    launch_gemv<EPI_RESID>(gs, ns, ex, dn, s, nt); n++;
     return n;
 }
 
 // final norm (in place) + quantize + lm_head (qwen3.rs:72-76)
-static int launch_head(q3_handle *h, cudaStream_t s) {
+static int launch_head(q3_handle *h, const StepBufs &b, int nt, cudaStream_t s) {
     const q3_config &c = h->cfg;
     NormQuantArgs na{};
-    na.x = h->x; na.w = h->rms_final; na.q = h->xq; na.s = h->xs; na.n = c.dim; na.write_normed = 1;
-    int n = launch_norm_quant(c.group_size, h->exact, na, s);
+    na.x = b.x; na.w = h->rms_final; na.q = b.xq; na.s = b.xs; na.n = c.dim; na.write_normed = 1;
+    int n = launch_norm_quant(c.group_size, h->exact, na, s, nt);
     GemvArgs g{};
-    g.wq = h->wcls.q; g.ws = h->wcls.s; g.xq = h->xq; g.xs = h->xs; g.K = c.dim; g.rows = c.vocab_size; g.out = h->logits;
-    launch_gemv<EPI_STORE>(c.group_size, h->num_sms, h->exact, g, s); n++;
+    g.wq = h->wcls.q; g.ws = h->wcls.s; g.xq = b.xq; g.xs = b.xs; g.K = c.dim; g.rows = c.vocab_size; g.out = b.logits;
+    launch_gemv<EPI_STORE>(c.group_size, h->num_sms, h->exact, g, s, nt); n++;
     return n;
 }
 
-static int launch_argmax(q3_handle *h, bool feedback, cudaStream_t s) {
+// argmax of every logits row of b; feedback (single token only): fed back as the next token / position, appended to the history
+static int launch_argmax(q3_handle *h, const StepBufs &b, int nt, bool feedback, cudaStream_t s) {
     int *tp = h->d_tokpos;
-    k_argmax<<<1, 1024, 0, s>>>(h->logits, h->cfg.vocab_size, tp + 2, feedback ? tp : nullptr, feedback ? tp + 1 : nullptr,
-                                feedback ? h->d_history : nullptr, tp + 3);
+    k_argmax<<<nt, 1024, 0, s>>>(b.logits, h->cfg.vocab_size, b.argmax, feedback ? tp : nullptr, feedback ? tp + 1 : nullptr,
+                                 feedback ? h->d_history : nullptr, tp + 3);
     return 1;
 }
 
-static int launch_step(q3_handle *h, bool argmax, bool feedback, cudaStream_t s) {
+static int launch_step(q3_handle *h, const StepBufs &b, int nt, bool argmax, bool feedback, cudaStream_t s) {
     int n = 0;
-    for (int l = 0; l < h->cfg.n_layers; l++) n += launch_layer(h, l, l == 0, s);
-    n += launch_head(h, s);
-    if (argmax) n += launch_argmax(h, feedback, s);
+    for (int l = 0; l < h->cfg.n_layers; l++) n += launch_layer(h, b, nt, l, l == 0, s);
+    n += launch_head(h, b, nt, s);
+    if (argmax) n += launch_argmax(h, b, nt, feedback, s);
     return n;
 }
 
@@ -508,7 +580,7 @@ static int build_graphs(q3_handle *h) {
         cudaGraphExec_t *slot = which ? &h->g_greedy[ex] : &h->g_fwd[ex];
         cudaGraph_t g;
         CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-        int n = launch_step(h, which == 1, which == 1, h->stream);
+        int n = launch_step(h, step_bufs(h), 1, which == 1, which == 1, h->stream);
         cudaError_t e = cudaStreamEndCapture(h->stream, &g);
         if (e != cudaSuccess) return fail(Q3_ECUDA, "graph capture failed: %s", cudaGetErrorString(e));
         if (!*slot) CK(cudaGraphInstantiate(slot, g, 0));
@@ -786,13 +858,13 @@ enum StepOut {
 static int launch_decode_step(q3_handle *h, StepOut out, bool gather = false) {
     if (use_mega(h)) return launch_mega(h, 0, h->cfg.n_layers, true, true, out == STEP_FEEDBACK, gather);
     CK(cudaGraphLaunch(out == STEP_FEEDBACK ? h->g_greedy[h->exact] : h->g_fwd[h->exact], h->stream));
-    if (out == STEP_ARGMAX) launch_argmax(h, false, h->stream);
+    if (out == STEP_ARGMAX) launch_argmax(h, step_bufs(h), 1, false, h->stream);
     return 0;
 }
 // final norm + lm_head on h->x alone
 static int launch_head_only(q3_handle *h, bool gather) {
     if (use_mega(h)) return launch_mega(h, 0, 0, false, true, false, gather);
-    launch_head(h, h->stream);
+    launch_head(h, step_bufs(h), 1, h->stream);
     return 0;
 }
 
@@ -1434,6 +1506,10 @@ extern "C" void q3_destroy(q3_handle *h) {
         if (h->g_fwd[e]) cudaGraphExecDestroy(h->g_fwd[e]);
         if (h->g_greedy[e]) cudaGraphExecDestroy(h->g_greedy[e]);
     }
+    for (cudaGraphExec_t g : h->g_multi)
+        if (g) cudaGraphExecDestroy(g);
+    if (h->h_mctl) cudaFreeHost(h->h_mctl);
+    if (h->h_mlogits) cudaFreeHost(h->h_mlogits);
     prefill_release(h);
     if (h->sc_logits) cudaFree(h->sc_logits);
     if (h->tk_ids) cudaFree(h->tk_ids);
@@ -1542,6 +1618,171 @@ extern "C" int q3_decode_greedy(q3_handle *h, int first_token, int pos0, int n, 
         if ((rc = launch_decode_step(h, STEP_FEEDBACK))) return rc;
     if (tokens_out && n > 0) CK(cudaMemcpyAsync(tokens_out, h->d_history, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
     return finish_call(h);
+}
+
+// ------------------------------------------------------------------------------------------
+// q3_forward_multi: n graph decode steps of consecutive positions in one pass over the weights
+// ------------------------------------------------------------------------------------------
+// The Q3_MULTI_MAX-row state of the multi-token step (nothing is allocated before the first call) and the shared-memory opt-in
+// of the multi-token GEMV kernels of this handle's group size
+static int multi_reserve(q3_handle *h) {
+    if (h->m_ctl) return 0;
+    const q3_config &c = h->cfg;
+    const int gs = c.group_size, dim = c.dim, maxd = h->AH_l > dim ? h->AH_l : dim;
+    const size_t M = Q3_MULTI_MAX;
+    int rc;
+    struct { void **p; size_t bytes; } want[] = {
+        {(void **)&h->m_x, M * dim * 4},           {(void **)&h->m_xb, M * maxd * 4},
+        {(void **)&h->m_q, M * h->AH_l * 4},       {(void **)&h->m_hb, M * h->H_l * 4},
+        {(void **)&h->m_logits, M * c.vocab_size * 4},
+        {(void **)&h->m_part, M * h->n_heads_l * ATTN_MAX_SPLITS * ATTN_PART_STRIDE * 4},
+        {(void **)&h->m_xq, M * maxd},             {(void **)&h->m_hq, M * h->H_l},
+        {(void **)&h->m_xs, M * (maxd / gs) * 4},  {(void **)&h->m_hs, M * (h->H_l / gs) * 4}};
+    for (auto &w : want) // a buffer already allocated by an earlier, failed reserve is kept
+        if (!*w.p && (rc = dmalloc(h, w.p, w.bytes))) return rc;
+    if (!h->h_mctl) CK(cudaMallocHost((void **)&h->h_mctl, MCTL_INTS * 4));
+#define ALLOW_MULTI(GS)                                                                                       \
+    for (int nt = 2; nt <= Q3_MULTI_MAX; nt++) {                                                              \
+        NT_DISPATCH(nt, (rc = allow_smem(k_gemv<GS, EPI_STORE, false, false, NT>, GEMV_MULTI_SMEM)));          \
+        if (!rc) NT_DISPATCH(nt, (rc = allow_smem(k_gemv<GS, EPI_QKV, false, false, NT>, GEMV_MULTI_SMEM)));   \
+        if (!rc) NT_DISPATCH(nt, (rc = allow_smem(k_gemv<GS, EPI_RESID, false, false, NT>, GEMV_MULTI_SMEM))); \
+        if (!rc) NT_DISPATCH(nt, (rc = allow_smem(k_gemv<GS, EPI_SWIGLU, false, false, NT>, GEMV_MULTI_SMEM)));\
+        if (rc) return rc;                                                                                    \
+    }
+    GS_DISPATCH(gs, ALLOW_MULTI(GS));
+#undef ALLOW_MULTI
+    int *ctl = nullptr; // allocated last: m_ctl set means the reserve is complete; a failed one is resumed by the next call
+    if ((rc = dmalloc(h, (void **)&ctl, MCTL_INTS * 4))) return rc;
+    CK(cudaMemset(ctl, 0, MCTL_INTS * 4));
+    h->m_ctl = ctl;
+    return 0;
+}
+
+// Queue the n-token step of tokens at pos0 .. pos0+n-1 (checked): logits rows into m_logits, argmax into m_ctl.  Fast mode: the
+// graph of n; exact mode (any mask bit): the n single-token steps of that mode one after another.
+static int launch_multi(q3_handle *h, const int *tokens, int n, int pos0) {
+    int *c = h->h_mctl;
+    for (int i = 0; i < n; i++) {
+        c[i] = tokens[i];
+        c[MCTL_STEPS + 2 * i] = tokens[i];
+        c[MCTL_STEPS + 2 * i + 1] = pos0 + i;
+    }
+    c[MCTL_POS0] = pos0;
+    CK(cudaMemcpyAsync(h->m_ctl, c, MCTL_INTS * 4, cudaMemcpyHostToDevice, h->stream));
+    if (h->exact) {
+        const size_t V = h->cfg.vocab_size;
+        for (int i = 0; i < n; i++) {
+            CK(cudaMemcpyAsync(h->d_tokpos, h->m_ctl + MCTL_STEPS + 2 * i, 8, cudaMemcpyDeviceToDevice, h->stream));
+            CK(cudaGraphLaunch(h->g_fwd[h->exact], h->stream));
+            launch_argmax(h, step_bufs(h), 1, false, h->stream);
+            CK(cudaMemcpyAsync(h->m_ctl + MCTL_ARGMAX + i, h->d_tokpos + 2, 4, cudaMemcpyDeviceToDevice, h->stream));
+            CK(cudaMemcpyAsync(h->m_logits + i * V, h->logits, V * 4, cudaMemcpyDeviceToDevice, h->stream));
+        }
+        return 0;
+    }
+    if (!h->g_multi[n]) {
+        cudaGraph_t g;
+        CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
+        launch_step(h, multi_bufs(h), n, true, false, h->stream);
+        cudaError_t e = cudaStreamEndCapture(h->stream, &g);
+        if (e != cudaSuccess) return fail(Q3_ECUDA, "graph capture failed: %s", cudaGetErrorString(e));
+        e = cudaGraphInstantiate(&h->g_multi[n], g, 0);
+        cudaGraphDestroy(g);
+        if (e != cudaSuccess) {
+            h->g_multi[n] = nullptr;
+            return fail(Q3_ECUDA, "graph instantiation failed: %s", cudaGetErrorString(e));
+        }
+    }
+    CK(cudaGraphLaunch(h->g_multi[n], h->stream));
+    return 0;
+}
+
+// the checks of q3_forward_multi / q3_bench_multi, before any device work
+static int check_multi(const q3_handle *h, const int *tokens, int n, int pos0) {
+    if (!h) return fail(Q3_EINVAL, "null handle");
+    if (h->tp_size > 1) return fail(Q3_EUNSUPPORTED, "the multi-token step runs on the multi-kernel path, which has no tensor-parallel exchange");
+    if (n < 1 || n > Q3_MULTI_MAX) return fail(Q3_EINVAL, "n %d outside 1 .. %d", n, Q3_MULTI_MAX);
+    return check_prompt(h, tokens, n, pos0);
+}
+
+extern "C" int q3_forward_multi(q3_handle *h, const int *tokens, int n, int pos0, int *argmax_out, float *logits_host) {
+    int rc = check_multi(h, tokens, n, pos0);
+    if (rc) return rc;
+    if (!argmax_out) return fail(Q3_EINVAL, "null argmax_out");
+    CK(cudaSetDevice(h->device));
+    if ((rc = multi_reserve(h))) return rc;
+    const size_t V = h->cfg.vocab_size;
+    if (logits_host && !h->h_mlogits) CK(cudaMallocHost((void **)&h->h_mlogits, Q3_MULTI_MAX * V * 4));
+    if ((rc = launch_multi(h, tokens, n, pos0))) return rc;
+    CK(cudaMemcpyAsync(h->h_mctl + MCTL_ARGMAX, h->m_ctl + MCTL_ARGMAX, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (logits_host) CK(cudaMemcpyAsync(h->h_mlogits, h->m_logits, n * V * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaGetLastError());
+    if ((rc = finish_call(h))) return rc;
+    memcpy(argmax_out, h->h_mctl + MCTL_ARGMAX, (size_t)n * 4);
+    if (logits_host) memcpy(logits_host, h->h_mlogits, n * V * 4);
+    return Q3_OK;
+}
+
+extern "C" int q3_bench_multi(q3_handle *h, int n, int pos0, int reps, float *ms_out) {
+    const int zeros[Q3_MULTI_MAX] = {};
+    int rc = check_multi(h, zeros, n, pos0);
+    if (rc) return rc;
+    if (reps < 1) return fail(Q3_EINVAL, "reps must be positive");
+    CK(cudaSetDevice(h->device));
+    if ((rc = multi_reserve(h))) return rc;
+    if ((rc = launch_multi(h, zeros, n, pos0))) return rc; // warm-up (captures the graph)
+    float ms = 0;
+    rc = time_events(h->stream, &ms, [&] {
+        for (int r = 0; r < reps; r++)
+            if (int rc1 = launch_multi(h, zeros, n, pos0)) return rc1;
+        return 0;
+    });
+    if (rc) return rc;
+    if (ms_out) *ms_out = ms;
+    return finish_call(h);
+}
+
+extern "C" int q3_decode_speculative(q3_handle *target, q3_handle *draft, int first_token, int pos0, int n, int k, int *tokens_out,
+                                     int *rounds_out, int *drafted_out, int *accepted_out) {
+    if (!target || !draft) return fail(Q3_EINVAL, "null handle");
+    if (target == draft) return fail(Q3_EINVAL, "the target and the draft must be different handles");
+    if (target->device != draft->device)
+        return fail(Q3_EINVAL, "the target (device %d) and the draft (device %d) must be on the same device", target->device, draft->device);
+    if (target->tp_size > 1 || draft->tp_size > 1) return fail(Q3_EUNSUPPORTED, "speculative decoding is single-GPU");
+    if (target->cfg.vocab_size != draft->cfg.vocab_size)
+        return fail(Q3_EINVAL, "vocab_size differs: target %d, draft %d", target->cfg.vocab_size, draft->cfg.vocab_size);
+    if (k < 1 || k > Q3_MULTI_MAX - 1) return fail(Q3_EINVAL, "k %d outside 1 .. %d", k, Q3_MULTI_MAX - 1);
+    if (n < 0 || (n > 0 && !tokens_out)) return fail(Q3_EINVAL, "bad n %d / tokens_out", n);
+    if (first_token < 0 || first_token >= target->cfg.vocab_size)
+        return fail(Q3_EINVAL, "index out of bounds: token %d >= vocab_size %d", first_token, target->cfg.vocab_size);
+    const int cap = target->cfg.seq_len < draft->cfg.seq_len ? target->cfg.seq_len : draft->cfg.seq_len;
+    if (pos0 < 0 || (long long)pos0 + n > cap)
+        return fail(Q3_EINVAL, "index out of bounds: pos0 %d + n %d > seq_len %d", pos0, n, cap);
+    int rounds = 0, drafted = 0, accepted = 0, produced = 0, tok = first_token, pos = pos0, rc;
+    while (produced < n) {
+        const int kk = k < n - produced - 1 ? k : n - produced - 1;
+        int seq[Q3_MULTI_MAX], a[Q3_MULTI_MAX];
+        seq[0] = tok;
+        // the draft's greedy tokens d = seq[1 .. kk] (its cache rows pos .. pos+kk-1), then the target's greedy token after each
+        // prefix of seq in one pass (its rows pos .. pos+kk); both calls end with a synchronise, so the two never overlap
+        if (kk > 0 && (rc = q3_decode_greedy(draft, tok, pos, kk, seq + 1))) return rc;
+        if ((rc = q3_forward_multi(target, seq, kk + 1, pos, a, nullptr))) return rc;
+        int j = 0;
+        while (j < kk && seq[1 + j] == a[j]) j++;
+        for (int i = 0; i < j; i++) tokens_out[produced++] = seq[1 + i];
+        tokens_out[produced++] = a[j];
+        rounds++;
+        drafted += kk;
+        accepted += j;
+        tok = a[j];
+        pos += j + 1;
+        // every draft token was accepted: the draft has no cache row yet for the last of them (position pos - 1)
+        if (j == kk && kk > 0 && produced < n && (rc = q3_forward(draft, seq[kk], pos - 1, nullptr))) return rc;
+    }
+    if (rounds_out) *rounds_out = rounds;
+    if (drafted_out) *drafted_out = drafted;
+    if (accepted_out) *accepted_out = accepted;
+    return Q3_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1683,7 +1924,7 @@ extern "C" int q3_bench_kernel(q3_handle *h, int kind, int pos, int reps, float 
             launch_gemv<EPI_STORE>(gs, ns, ex, g, h->stream);
             break;
         case 5:
-            launch_attn_partial(h, kc_l, vc_l, h->stream);
+            launch_attn_partial(h, step_bufs(h), 1, kc_l, vc_l, h->stream);
             break;
         }
     };
@@ -1843,7 +2084,7 @@ extern "C" int q3_forward_layers(q3_handle *h, int pos, int layer0, int layer1, 
     if (use_mega(h)) {
         if (layer1 > layer0 && (rc = launch_mega(h, layer0, layer1, false, false, false, false))) return rc;
     } else {
-        for (int l = layer0; l < layer1; l++) launch_layer(h, l, false, h->stream);
+        for (int l = layer0; l < layer1; l++) launch_layer(h, step_bufs(h), 1, l, false, h->stream);
     }
     CK(cudaMemcpyAsync(x_host, h->x, (size_t)h->cfg.dim * 4, cudaMemcpyDeviceToHost, h->stream));
     if (run_head) {

@@ -145,20 +145,21 @@ __device__ __forceinline__ void quantize_group4(const float4 &y, uint32_t &packe
 }
 
 // ------------------------------------------------------------------------------------------
-// RMSNorm (+ optional embedding gather) + group quantise.        one CTA, 1024 threads
+// RMSNorm (+ optional embedding gather) + group quantise.        one CTA per token, 1024 threads
 //   layers.rs:72-76 (embedding row, dequantised on the fly: tensor.rs:72-80),
 //   layers.rs:109-130 (RMSNorm), tensor.rs:91-119 (quantize).
 // x_io: residual stream (read; written when gathering the embedding or when inplace_norm).
+// Token t = blockIdx.x works on row t of x / q / s and gathers token[t].
 // ------------------------------------------------------------------------------------------
 struct NormQuantArgs {
-    float *x;              // [n] residual stream
+    float *x;              // [tokens][n] residual stream
     const float *w;        // [n] norm weight
-    int8_t *q;             // [n]
-    float *s;              // [n/GS]
+    int8_t *q;             // [tokens][n]
+    float *s;              // [tokens][n/GS]
     int n;
-    const int8_t *embed_q; // non-null: x = dequant(embed row *token) first
+    const int8_t *embed_q; // non-null: x = dequant(embed row token[t]) first
     const float *embed_s;
-    const int *token;
+    const int *token;      // [tokens]
     int write_normed;      // 1: x <- normed value (final norm is in place, qwen3.rs:72)
 };
 
@@ -171,6 +172,9 @@ __global__ void __launch_bounds__(1024) k_rmsnorm_quant(NormQuantArgs a) {
     __shared__ float s_f;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int n4 = a.n >> 2;
+    float *x = a.x + (size_t)blockIdx.x * a.n;
+    int8_t *q = a.q + (size_t)blockIdx.x * a.n;
+    float *s = a.s + (size_t)blockIdx.x * (a.n / GS);
     constexpr int MAXV = 4; // up to 16384 elements
     float4 v[MAXV];
     float ss = 0.0f;
@@ -180,13 +184,13 @@ __global__ void __launch_bounds__(1024) k_rmsnorm_quant(NormQuantArgs a) {
         v[k] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (i4 < n4) {
             if (a.embed_q) {
-                size_t base = (size_t)(*a.token) * a.n + (size_t)i4 * 4;
+                size_t base = (size_t)a.token[blockIdx.x] * a.n + (size_t)i4 * 4;
                 char4 e = *reinterpret_cast<const char4 *>(a.embed_q + base);
                 float sc = a.embed_s[base / GS];
                 v[k] = make_float4((float)e.x * sc, (float)e.y * sc, (float)e.z * sc, (float)e.w * sc);
-                reinterpret_cast<float4 *>(a.x)[i4] = v[k];
+                reinterpret_cast<float4 *>(x)[i4] = v[k];
             } else {
-                v[k] = reinterpret_cast<const float4 *>(a.x)[i4];
+                v[k] = reinterpret_cast<const float4 *>(x)[i4];
             }
             if (ORDERED) reinterpret_cast<float4 *>(s_x)[i4] = v[k];
             ss += __fmul_rn(v[k].x, v[k].x);
@@ -231,9 +235,9 @@ __global__ void __launch_bounds__(1024) k_rmsnorm_quant(NormQuantArgs a) {
             float scale;
             quantize_group4<GS>(y, packed, scale);
             if (i4 < n4) {
-                reinterpret_cast<uint32_t *>(a.q)[i4] = packed;
-                if ((i4 % (GS / 4)) == 0) a.s[i4 / (GS / 4)] = scale;
-                if (a.write_normed) reinterpret_cast<float4 *>(a.x)[i4] = y;
+                reinterpret_cast<uint32_t *>(q)[i4] = packed;
+                if ((i4 % (GS / 4)) == 0) s[i4 / (GS / 4)] = scale;
+                if (a.write_normed) reinterpret_cast<float4 *>(x)[i4] = y;
             }
         }
     }
@@ -259,10 +263,14 @@ __global__ void __launch_bounds__(1024) k_rmsnorm(const float *x, const float *w
 }
 
 // ------------------------------------------------------------------------------------------
-// Group quantise of an f32 vector (tensor.rs:91-119).   grid-stride, any n % GS == 0
+// Group quantise of an f32 vector (tensor.rs:91-119).   grid-stride, any n % GS == 0; blockIdx.y = row
+// of [rows][n] x / q and [rows][n/GS] s
 // ------------------------------------------------------------------------------------------
 template <int GS>
 __global__ void __launch_bounds__(256) k_quantize(const float *__restrict__ x, int n, int8_t *q, float *s) {
+    x += (size_t)blockIdx.y * n;
+    q += (size_t)blockIdx.y * n;
+    s += (size_t)blockIdx.y * (n / GS);
     const int n4 = n >> 2;
     const int lane = threadIdx.x & 31;
     for (int base = (blockIdx.x * blockDim.x + threadIdx.x) - lane; base < n4; base += gridDim.x * blockDim.x) {
@@ -279,44 +287,48 @@ __global__ void __launch_bounds__(256) k_quantize(const float *__restrict__ x, i
 }
 
 // ------------------------------------------------------------------------------------------
-// Batch-1 int8 GEMV with per-group f32 scales (tensor.rs:23-62).
-//   out[r] = sum_g ( (f32)(sum_k xq[g,k]*wq[r,g,k]) * ws[r,g] ) * xs[g]
+// Int8 GEMV with per-group f32 scales (tensor.rs:23-62) for NT tokens at once.
+//   out[t][r] = sum_g ( (f32)(sum_k xq[t][g,k]*wq[r,g,k]) * ws[r,g] ) * xs[t][g]
 // Row-major weights [rows][K] + scales [rows][K/GS].  256 threads = 8 warps; each warp owns a
 // PAIR of rows per step (rows 2p, 2p+1) and streams them with 128-bit L1-bypassing loads;
 // GS/16 adjacent lanes share one group, the int32 group dot is completed with shuffles and is
-// exactly the reference's i32 sum.  x (int8 + scales) is staged once per CTA in shared memory.
+// exactly the reference's i32 sum.  x (int8 + scales) of the NT tokens is staged once per CTA in
+// shared memory ([NT][K] then [NT][K/GS]), and every weight load feeds the NT tokens' dots: token
+// t's row result is folded in the same order whatever NT is, so it is bit-identical to NT = 1.
 // ------------------------------------------------------------------------------------------
 enum GemvEpi { EPI_STORE = 0, EPI_QKV = 1, EPI_RESID = 2, EPI_SWIGLU = 3 };
 
 struct GemvArgs {
     const int8_t *wq;
     const float *ws;
-    const int8_t *xq;
-    const float *xs;
+    const int8_t *xq;  // [NT][K]
+    const float *xs;   // [NT][K/GS]
     int K, rows;
-    float *out;        // STORE: [rows]; RESID: x[rows] += ; SWIGLU: hb[rows/2]
-    // QKV epilogue: rows [0,AH) -> q, [AH,AH+KV) -> kcache row, [AH+KV, AH+2KV) -> vcache row
+    float *out;        // STORE: [NT][rows]; RESID: x[NT][rows] += ; SWIGLU: hb[NT][rows/2]
+    // QKV epilogue: rows [0,AH) -> q[NT][AH], [AH,AH+KV) -> kcache row, [AH+KV, AH+2KV) -> vcache row
     float *q;
     float *kc, *vc;    // layer base of the caches
     int AH, KV;
-    const int *pos;
-    int32_t *dots;     // optional [rows][K/GS] per-group integer dots (tests)
+    const int *pos;    // token t writes cache row *pos + tok0 + t
+    int tok0;
+    int32_t *dots;     // optional [rows][K/GS] per-group integer dots (tests; NT = 1)
 };
 
 // ORDERED: the per-group f32 terms are parked in shared memory and folded left to right by one
 // lane per row (tensor.rs:41-61 `.map(..).sum()`), making the row result bit-identical to the
 // reference; EXPREF: exp() in the SwiGLU epilogue uses the glibc restatement.
-template <int GS, int EPI, bool ORDERED = false, bool EXPREF = ORDERED>
+template <int GS, int EPI, bool ORDERED = false, bool EXPREF = ORDERED, int NT = 1>
 __global__ void __launch_bounds__(256) k_gemv(GemvArgs a) {
+    static_assert(NT == 1 || !ORDERED, "the reference-order fold is single-token");
     extern __shared__ __align__(16) unsigned char smem[];
     int4 *sx = reinterpret_cast<int4 *>(smem);
-    float *sxs = reinterpret_cast<float *>(smem + a.K);
+    float *sxs = reinterpret_cast<float *>(smem + NT * a.K);
     float *sterms = sxs + (a.K / GS) + (threadIdx.x >> 5) * 2 * (a.K / GS); // ORDERED: [warp][2][ng]
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int nchunk = a.K >> 4; // 16-byte chunks per row
     const int ng = a.K / GS;
-    for (int i = tid; i < nchunk; i += 256) sx[i] = reinterpret_cast<const int4 *>(a.xq)[i];
-    for (int i = tid; i < ng; i += 256) sxs[i] = a.xs[i];
+    for (int i = tid; i < NT * nchunk; i += 256) sx[i] = reinterpret_cast<const int4 *>(a.xq)[i];
+    for (int i = tid; i < NT * ng; i += 256) sxs[i] = a.xs[i];
     __syncthreads();
 
     constexpr int LPG = GS / 16; // lanes per group
@@ -327,7 +339,9 @@ __global__ void __launch_bounds__(256) k_gemv(GemvArgs a) {
         const int4 *w1 = reinterpret_cast<const int4 *>(a.wq + (r0 + 1) * a.K);
         const float *s0 = a.ws + r0 * ng;
         const float *s1 = s0 + ng;
-        float acc0 = 0.0f, acc1 = 0.0f;
+        float acc0[NT], acc1[NT];
+#pragma unroll
+        for (int t = 0; t < NT; t++) acc0[t] = acc1[t] = 0.0f;
         for (int c0 = 0; c0 < nchunk; c0 += 128) {
             int4 wa[4], wb[4];
 #pragma unroll
@@ -342,34 +356,46 @@ __global__ void __launch_bounds__(256) k_gemv(GemvArgs a) {
             for (int u = 0; u < 4; u++) {
                 int c = c0 + u * 32 + lane;
                 bool ok = c < nchunk;
-                int d0 = 0, d1 = 0;
+                int d0[NT], d1[NT];
+#pragma unroll
+                for (int t = 0; t < NT; t++) d0[t] = d1[t] = 0;
                 if (ok) {
-                    int4 xv = sx[c];
-                    d0 = dot16(wa[u], xv, 0);
-                    d1 = dot16(wb[u], xv, 0);
+#pragma unroll
+                    for (int t = 0; t < NT; t++) {
+                        int4 xv = sx[t * nchunk + c];
+                        d0[t] = dot16(wa[u], xv, 0);
+                        d1[t] = dot16(wb[u], xv, 0);
+                    }
                 }
                 if (c - lane < nchunk) { // warp-uniform: this step has at least one live lane
 #pragma unroll
                     for (int o = LPG / 2; o > 0; o >>= 1) {
-                        d0 += __shfl_xor_sync(0xffffffffu, d0, o);
-                        d1 += __shfl_xor_sync(0xffffffffu, d1, o);
+#pragma unroll
+                        for (int t = 0; t < NT; t++) {
+                            d0[t] += __shfl_xor_sync(0xffffffffu, d0[t], o);
+                            d1[t] += __shfl_xor_sync(0xffffffffu, d1[t], o);
+                        }
                     }
                     if (ok && (lane % LPG) == 0) {
                         int g = c / LPG;
-                        float xsg = sxs[g];
-                        // (dot as f32 * weight_scale) * input_scale   (tensor.rs:59)
-                        float t0 = __fmul_rn(__fmul_rn((float)d0, __ldg(s0 + g)), xsg);
-                        float t1 = __fmul_rn(__fmul_rn((float)d1, __ldg(s1 + g)), xsg);
-                        if (ORDERED) {
-                            sterms[g] = t0;
-                            sterms[ng + g] = t1;
-                        } else {
-                            acc0 = __fadd_rn(acc0, t0);
-                            acc1 = __fadd_rn(acc1, t1);
+                        const float ws0 = __ldg(s0 + g), ws1 = __ldg(s1 + g);
+#pragma unroll
+                        for (int t = 0; t < NT; t++) {
+                            float xsg = sxs[t * ng + g];
+                            // (dot as f32 * weight_scale) * input_scale   (tensor.rs:59)
+                            float t0 = __fmul_rn(__fmul_rn((float)d0[t], ws0), xsg);
+                            float t1 = __fmul_rn(__fmul_rn((float)d1[t], ws1), xsg);
+                            if (ORDERED) {
+                                sterms[g] = t0;
+                                sterms[ng + g] = t1;
+                            } else {
+                                acc0[t] = __fadd_rn(acc0[t], t0);
+                                acc1[t] = __fadd_rn(acc1[t], t1);
+                            }
                         }
-                        if (a.dots) {
-                            a.dots[r0 * ng + g] = d0;
-                            a.dots[(r0 + 1) * ng + g] = d1;
+                        if (NT == 1 && a.dots) {
+                            a.dots[r0 * ng + g] = d0[0];
+                            a.dots[(r0 + 1) * ng + g] = d1[0];
                         }
                     }
                 }
@@ -380,33 +406,41 @@ __global__ void __launch_bounds__(256) k_gemv(GemvArgs a) {
             float t = 0.0f;
             if (lane < 2)
                 for (int g = 0; g < ng; g++) t = __fadd_rn(t, sterms[lane * ng + g]);
-            acc0 = __shfl_sync(0xffffffffu, t, 0);
-            acc1 = __shfl_sync(0xffffffffu, t, 1);
+            acc0[0] = __shfl_sync(0xffffffffu, t, 0);
+            acc1[0] = __shfl_sync(0xffffffffu, t, 1);
             __syncwarp();
         } else {
-            acc0 = warp_sum(acc0);
-            acc1 = warp_sum(acc1);
+#pragma unroll
+            for (int t = 0; t < NT; t++) {
+                acc0[t] = warp_sum(acc0[t]);
+                acc1[t] = warp_sum(acc1[t]);
+            }
         }
         if (lane == 0) {
-            if (EPI == EPI_STORE) {
-                a.out[r0] = acc0;
-                a.out[r0 + 1] = acc1;
-            } else if (EPI == EPI_RESID) { // ResidualConnection::forward, layers.rs:249-259
-                a.out[r0] = __fadd_rn(a.out[r0], acc0);
-                a.out[r0 + 1] = __fadd_rn(a.out[r0 + 1], acc1);
-            } else if (EPI == EPI_SWIGLU) { // layers.rs:472-475: g * (1/(1+exp(-g))) * up
-                float g = acc0;
-                float sw = __fmul_rn(g, __fdiv_rn(1.0f, __fadd_rn(1.0f, exp_sel<EXPREF>(-g))));
-                a.out[p] = __fmul_rn(sw, acc1);
-            } else { // EPI_QKV, layers.rs:334-336: K and V go straight into the cache row of `pos`
-                const int pos = *a.pos;
-                int r = (int)r0;
-                float *dst;
-                if (r < a.AH) dst = a.q + r;
-                else if (r < a.AH + a.KV) dst = a.kc + (size_t)pos * a.KV + (r - a.AH);
-                else dst = a.vc + (size_t)pos * a.KV + (r - a.AH - a.KV);
-                dst[0] = acc0;
-                dst[1] = acc1;
+#pragma unroll
+            for (int t = 0; t < NT; t++) {
+                if (EPI == EPI_STORE) {
+                    float *out = a.out + (size_t)t * a.rows;
+                    out[r0] = acc0[t];
+                    out[r0 + 1] = acc1[t];
+                } else if (EPI == EPI_RESID) { // ResidualConnection::forward, layers.rs:249-259
+                    float *out = a.out + (size_t)t * a.rows;
+                    out[r0] = __fadd_rn(out[r0], acc0[t]);
+                    out[r0 + 1] = __fadd_rn(out[r0 + 1], acc1[t]);
+                } else if (EPI == EPI_SWIGLU) { // layers.rs:472-475: g * (1/(1+exp(-g))) * up
+                    float g = acc0[t];
+                    float sw = __fmul_rn(g, __fdiv_rn(1.0f, __fadd_rn(1.0f, exp_sel<EXPREF>(-g))));
+                    a.out[(size_t)t * npairs + p] = __fmul_rn(sw, acc1[t]);
+                } else { // EPI_QKV, layers.rs:334-336: K and V go straight into the cache row of `pos`
+                    const int pos = *a.pos + a.tok0 + t;
+                    int r = (int)r0;
+                    float *dst;
+                    if (r < a.AH) dst = a.q + (size_t)t * a.AH + r;
+                    else if (r < a.AH + a.KV) dst = a.kc + (size_t)pos * a.KV + (r - a.AH);
+                    else dst = a.vc + (size_t)pos * a.KV + (r - a.AH - a.KV);
+                    dst[0] = acc0[t];
+                    dst[1] = acc1[t];
+                }
             }
         }
     }
@@ -418,6 +452,7 @@ __global__ void __launch_bounds__(256) k_gemv(GemvArgs a) {
 //   layers.rs:173-185 (half-split pairs (i, i+64)); cos/sin come from the host-computed table
 //   (layers.rs:161-171 evaluated with glibc, bit-identical to the reference's libm calls).
 // One warp per head; lane holds 4 consecutive dims; the pair partner lives in lane^16.
+// blockIdx.y = token t: q row t ([tokens][n_heads*128]) and the cache row *pos_p + t.
 // ------------------------------------------------------------------------------------------
 template <bool ORDERED = false>
 __global__ void __launch_bounds__(128) k_qknorm_rope(float *q, float *kc_layer, const float *q_ln,
@@ -427,7 +462,8 @@ __global__ void __launch_bounds__(128) k_qknorm_rope(float *q, float *kc_layer, 
     const int lane = threadIdx.x & 31;
     const int head = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (head >= n_heads + n_kv) return;
-    const int pos = *pos_p;
+    const int pos = *pos_p + blockIdx.y;
+    q += (size_t)blockIdx.y * n_heads * HEAD_DIM;
     float *p = head < n_heads ? q + (size_t)head * HEAD_DIM
                               : kc_layer + (size_t)pos * KV + (size_t)(head - n_heads) * HEAD_DIM;
     const float *w = head < n_heads ? q_ln : k_ln;
@@ -480,9 +516,12 @@ __global__ void __launch_bounds__(128) k_qknorm_rope(float *q, float *kc_layer, 
 // ------------------------------------------------------------------------------------------
 // GQA decode attention, split-K over the sequence (flash-decoding).
 //   layers.rs:374-419: s_t = (q . k_t) / sqrt(128) for t in 0..=pos, softmax, out = sum a_t v_t.
-// grid = (n_kv_heads, ATTN_MAX_SPLITS); the CTA streams its slice of K and V ONCE for all
+// grid = (n_kv_heads * ntok, ATTN_MAX_SPLITS); the CTA streams its slice of K and V ONCE for all
 // KVMUL query heads that share the kv head and leaves an un-normalised partial
-// (m, l, acc[128]) per query head; k_attn_combine_quant merges the partials.
+// (m, l, acc[128]) per query head; k_attn_combine_quant merges the partials.  Token t (q row t,
+// partials block t) sits at position *pos_p + t and takes the splits of that position, so its
+// result is the single-token one; the ntok CTAs of one (kv head, split) are adjacent in launch
+// order, and the K / V rows they share come from L2.
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ void attn_split_range(int pos, int split, int &t0, int &t1, int &nsplit) {
     int n = pos + 1;
@@ -499,9 +538,11 @@ constexpr int ATTN_PART_STRIDE = HEAD_DIM + 4; // acc[128], m, l, pad
 template <int KVMUL>
 __global__ void __launch_bounds__(128) k_attn_partial(const float *__restrict__ q, const float *__restrict__ kc,
                                                       const float *__restrict__ vc, float *part, const int *pos_p,
-                                                      int KV, int n_heads) {
-    const int kvh = blockIdx.x, split = blockIdx.y;
-    const int pos = *pos_p;
+                                                      int KV, int n_heads, int ntok) {
+    const int kvh = blockIdx.x / ntok, tok = blockIdx.x % ntok, split = blockIdx.y;
+    const int pos = *pos_p + tok;
+    q += (size_t)tok * n_heads * HEAD_DIM;
+    part += (size_t)tok * n_heads * ATTN_MAX_SPLITS * ATTN_PART_STRIDE;
     int t0, t1, nsplit;
     attn_split_range(pos, split, t0, t1, nsplit);
     if (split >= nsplit) return;
@@ -583,12 +624,18 @@ __global__ void __launch_bounds__(128) k_attn_partial(const float *__restrict__ 
 }
 
 // Merge split partials of one query head, normalise, and group-quantise the result
-// (the quantize() before o_proj, qwen3.rs:152).  grid = n_heads, 128 threads (one per dim).
+// (the quantize() before o_proj, qwen3.rs:152).  grid = (n_heads, tokens), 128 threads (one per dim);
+// token t = blockIdx.y at position *pos_p + t reads partials block t and writes row t of xb / q / s.
 template <int GS>
 __global__ void __launch_bounds__(128) k_attn_combine_quant(const float *__restrict__ part, const int *pos_p,
                                                             float *xb, int8_t *q, float *s) {
     const int head = blockIdx.x, d = threadIdx.x;
-    const int pos = *pos_p;
+    const int pos = *pos_p + blockIdx.y;
+    const size_t AH = (size_t)gridDim.x * HEAD_DIM;
+    part += blockIdx.y * (size_t)gridDim.x * ATTN_MAX_SPLITS * ATTN_PART_STRIDE;
+    xb += blockIdx.y * AH;
+    q += blockIdx.y * AH;
+    s += blockIdx.y * (AH / GS);
     int t0, t1, nsplit;
     attn_split_range(pos, 0, t0, t1, nsplit);
     const float *base = part + (size_t)head * ATTN_MAX_SPLITS * ATTN_PART_STRIDE;
@@ -665,13 +712,15 @@ __global__ void __launch_bounds__(128) k_attn_ordered(const float *__restrict__ 
 
 // ------------------------------------------------------------------------------------------
 // Greedy argmax with the reference's tie rule (sampler.rs:57-59, max_by(total_cmp) keeps the
-// LAST maximum).  One CTA; optionally feeds the token back and advances pos for on-device
-// multi-step decode.
+// LAST maximum).  One CTA per row of logits [rows][n] -> token_out[row]; with one row it can feed the
+// token back and advance pos for on-device multi-step decode.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) k_argmax(const float *__restrict__ logits, int n, int *token_out,
                                                  int *token_feedback, int *pos_advance, int *history,
                                                  int *history_idx) {
     __shared__ long long red[32];
+    logits += (size_t)blockIdx.x * n;
+    token_out += blockIdx.x;
     long long best = (long long)0x8000000000000000LL;
     for (int i = threadIdx.x; i < n; i += 1024) {
         long long key = ((long long)total_key(logits[i]) << 32) | (unsigned)i; // ties -> larger index

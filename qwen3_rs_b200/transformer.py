@@ -68,6 +68,9 @@ ABI = {
     "q3_forward": (_i, [_vp, _i, _i, _vp]),
     "q3_forward_argmax": (_i, [_vp, _i, _i, C.POINTER(_i)]),
     "q3_decode_greedy": (_i, [_vp, _i, _i, _i, _vp]),
+    "q3_forward_multi": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
+    "q3_bench_multi": (_i, [_vp, _i, _i, _i, C.POINTER(_f)]),
+    "q3_decode_speculative": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
     "q3_sampler_set": (_i, [_vp, _f, _f, C.c_ulonglong]),
     "q3_sampler_state": (_i, [_vp, C.POINTER(C.c_ulonglong)]),
     "q3_sampler_skip": (_i, [_vp, _i]),
@@ -176,6 +179,40 @@ class Transformer:
         out = np.zeros(max(n, 1), np.int32)
         _check(load_library().q3_decode_greedy(self._h, int(first_token), int(pos0), int(n), _ptr(out)))
         return out[:n].tolist()
+
+    def forward_multi(self, tokens: Sequence[int], pos0: int, want_logits: bool = False):
+        """q3_forward_multi: tokens[i] at position pos0 + i, 1 <= len(tokens) <= MULTI_MAX, in one pass over the weights ->
+        (argmax [n], logits [n, vocab] or None).  Row i is bit-identical to forward(tokens[i], pos0 + i) on the multi-kernel
+        path after the rows before it (exact mode: the same single-token steps, run one after another)."""
+        t = np.ascontiguousarray(tokens, np.int32).reshape(-1)
+        if not 1 <= t.size <= MULTI_MAX:
+            raise ValueError(f"forward_multi: {t.size} tokens, expected 1 .. {MULTI_MAX}")
+        am = np.empty(t.size, np.int32)
+        lg = np.empty((t.size, self._config.vocab_size), np.float32) if want_logits else None
+        _check(load_library().q3_forward_multi(self._h, _ptr(t), t.size, int(pos0), _ptr(am), _ptr(lg)))
+        return am, lg
+
+    def bench_multi(self, n: int, pos0: int, reps: int) -> float:
+        """Total milliseconds of reps n-token steps at pos0 (q3_bench_multi)."""
+        ms = C.c_float(0)
+        _check(load_library().q3_bench_multi(self._h, int(n), int(pos0), int(reps), C.byref(ms)))
+        return ms.value
+
+    def decode_speculative(self, draft: "Transformer", first_token: int, pos0: int, n: int, k: int):
+        """q3_decode_speculative: n greedy tokens after first_token at pos0, k tokens drafted per round by `draft` and verified
+        with forward_multi -> (tokens, {"rounds", "drafted", "accepted"}).  The tokens (and this transformer's K/V rows) are
+        those of decode_greedy on the multi-kernel path, whatever the draft proposes."""
+        if not isinstance(draft, Transformer):
+            raise TypeError("decode_speculative: draft must be a Transformer")
+        if isinstance(k, bool) or int(k) != k or not 1 <= k <= MULTI_MAX - 1:
+            raise ValueError(f"k must be an integer in 1 .. {MULTI_MAX - 1}, got {k!r}")
+        if isinstance(n, bool) or int(n) != n or n < 0:
+            raise ValueError(f"n must be a non-negative integer, got {n!r}")
+        out = np.zeros(max(int(n), 1), np.int32)
+        r, d, a = C.c_int(0), C.c_int(0), C.c_int(0)
+        _check(load_library().q3_decode_speculative(self._h, draft._h, int(first_token), int(pos0), int(n), int(k), _ptr(out),
+                                                    C.byref(r), C.byref(d), C.byref(a)))
+        return out[:int(n)].tolist(), {"rounds": r.value, "drafted": d.value, "accepted": a.value}
 
     # -- device sampler (sampler.rs on the device) --------------------------------------------
     def sampler_set(self, temperature: float, topp: float, rng_seed: int) -> None:
@@ -476,6 +513,7 @@ def op_logprobs(logits, targets=None, want_argmax: bool = True, device: int = 0)
 
 
 TOPK_MAX = 64  # Q3_TOPK_MAX in include/qwen3_cuda.h
+MULTI_MAX = 8  # Q3_MULTI_MAX in include/qwen3_cuda.h
 
 
 def _topk_k(k) -> int:

@@ -30,6 +30,11 @@ extern "C" {
     fn q3_score_topk(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, k: c_int, topk_ids_out: *mut c_int,
                      topk_logprobs_out: *mut c_float, targets: *const c_int, logprobs_out: *mut c_float, argmax_out: *mut c_int)
                      -> c_int;
+    fn q3_forward_multi(h: *mut Q3Handle, tokens: *const c_int, n: c_int, pos0: c_int, argmax_out: *mut c_int,
+                        logits_host: *mut c_float) -> c_int;
+    fn q3_decode_speculative(target: *mut Q3Handle, draft: *mut Q3Handle, first_token: c_int, pos0: c_int, n: c_int, k: c_int,
+                             tokens_out: *mut c_int, rounds_out: *mut c_int, drafted_out: *mut c_int, accepted_out: *mut c_int)
+                             -> c_int;
     fn q3_reset(h: *mut Q3Handle) -> c_int;
     fn q3_logits_host(h: *mut Q3Handle) -> *mut c_float;
 }
@@ -134,6 +139,37 @@ impl CudaTransformer {
         top.chunks(k.max(1)).zip(lps.chunks(k.max(1)))
             .map(|(t, l)| t.iter().zip(l).map(|(&i, &v)| (i as usize, v)).collect())
             .collect()
+    }
+
+    /// `tokens[i]` at position `pos0 + i` (1 ..= 8 tokens, `Q3_MULTI_MAX`) in one pass over the weights: the greedy token after
+    /// each prefix, each bit-identical to a single-token step of the multi-kernel path.
+    pub fn forward_multi(&mut self, tokens: &[usize], pos0: usize) -> Vec<usize> {
+        let ids: Vec<c_int> = tokens.iter().map(|&t| t as c_int).collect();
+        let mut am = vec![0 as c_int; ids.len()];
+        let rc = unsafe {
+            q3_forward_multi(self.handle, ids.as_ptr(), ids.len() as c_int, pos0 as c_int, am.as_mut_ptr(), std::ptr::null_mut())
+        };
+        if rc != 0 {
+            panic!("{}", last_error());
+        }
+        am.into_iter().map(|t| t as usize).collect()
+    }
+
+    /// `n` greedy tokens after `first_token` at `pos0`, `k` (1 ..= 7) drafted per round by `draft` and verified in one pass:
+    /// the tokens of `decode_greedy` on the multi-kernel path.  Returns the tokens and (rounds, drafted, accepted).
+    pub fn decode_speculative(&mut self, draft: &mut CudaTransformer, first_token: usize, pos0: usize, n: usize, k: usize)
+                              -> (Vec<usize>, (usize, usize, usize)) {
+        let mut out = vec![0 as c_int; n.max(1)];
+        let (mut r, mut d, mut a) = (0 as c_int, 0 as c_int, 0 as c_int);
+        let rc = unsafe {
+            q3_decode_speculative(self.handle, draft.handle, first_token as c_int, pos0 as c_int, n as c_int, k as c_int,
+                                  out.as_mut_ptr(), &mut r, &mut d, &mut a)
+        };
+        if rc != 0 {
+            panic!("{}", last_error());
+        }
+        out.truncate(n);
+        (out.into_iter().map(|t| t as usize).collect(), (r as usize, d as usize, a as usize))
     }
 
     /// Zero the KV cache (a fresh `TransformerBlockBuffers`, qwen3.rs:439-440).
