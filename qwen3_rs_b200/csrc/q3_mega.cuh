@@ -24,9 +24,9 @@
 // The only grid barrier left is the one before the greedy argmax (one per token).
 //
 // HBM "stream" layout (built once at load by k_build_stream): for every GEMV phase, rows are
-// split contiguously over CTAs; a CTA's rows are stored in the exact order its consumers eat
-// them, one "row tile" (KT <= 4096 columns + their f32 scales) per consumer warp per stage,
-// and inside a tile the 16-byte chunks are permuted so that lane l owns whole quantisation
+// split contiguously over CTAs (gate/up: the same counts, units dealt in rounds, see gu_map);
+// a CTA's rows are stored in the exact order its consumers eat them, one "row tile" (KT <= 4096
+// columns + their f32 scales) per consumer warp per stage, and inside a tile the 16-byte chunks are permuted so that lane l owns whole quantisation
 // groups (l, l+32, ...) while every 128-bit shared-memory load stays bank-conflict free.
 //
 // Float semantics are those of the fast multi-kernel path (q3_kernels.cuh): identical per-group
@@ -245,6 +245,35 @@ __device__ __host__ __forceinline__ void cta_share(int units, int nctas, int c, 
     start = c * base + (c < rem ? c : rem);
 }
 
+// Which hidden units (gate/up pairs) the PH_GU segment of CTA c holds.  The per-CTA counts are cta_share's, but the units
+// are dealt in rounds: block s < full of CTA c holds units s * stride + MEGA_GW * c .. + MEGA_GW - 1 (stride = MEGA_GW *
+// nctas), and the units past full * stride (the tail) are split with cta_share, in CTA order, as each CTA's last block.
+// The SwiGLU words then become final in vector order, round after round, on every CTA at once: when the down_proj prologue
+// polls zone H, everything below the last round or two is already there and only the end of the vector races the
+// slowest CTAs.  With a contiguous range per CTA, each CTA's last block -- the words still missing when the prologue
+// starts -- is spread over the whole vector, and every warp of the prologue waits on some of them.  full = 0 (fewer than
+// MEGA_GW units per CTA) is the contiguous split.
+struct GuMap {
+    int full;   // interleaved blocks per CTA
+    int stride; // units per round of blocks, MEGA_GW * nctas
+    int first;  // first unit of the CTA's block 0
+    int tail0;  // first unit of the CTA's tail
+};
+__device__ __host__ __forceinline__ GuMap gu_map(int units, int nctas, int c) {
+    GuMap m;
+    m.full = units / nctas / MEGA_GW;
+    m.stride = MEGA_GW * nctas;
+    m.first = MEGA_GW * c;
+    int ts, tn;
+    cta_share(units - m.full * m.stride, nctas, c, ts, tn);
+    m.tail0 = m.full * m.stride + ts;
+    return m;
+}
+// unit at position j of the CTA's segment (no division: the SwiGLU epilogue calls it)
+__device__ __host__ __forceinline__ int gu_unit(const GuMap &m, int j) {
+    return j < MEGA_GW * m.full ? (j / MEGA_GW) * m.stride + m.first + j % MEGA_GW : m.tail0 + (j - MEGA_GW * m.full);
+}
+
 // ------------------------------------------------------------------------------------------
 // stream builder: row-major int8 [rows][K] + scales [rows][K/GS]  ->  megakernel stream
 // grid = (units, n_kt); one block per unit (row, or gate/up pair) and K tile.
@@ -273,7 +302,7 @@ __global__ void __launch_bounds__(256) k_build_stream(const int8_t *__restrict__
             int blk = j / MEGA_GW, w = j % MEGA_GW, np = n_c - MEGA_GW * blk;
             if (np > MEGA_GW) np = MEGA_GW;
             tile_index = (long long)start * 2 + 2 * MEGA_GW * blk + half * np + w;
-            src_row = (size_t)2 * u + half;
+            src_row = (size_t)2 * gu_unit(gu_map(units, nctas, c), j) + half;
         } else { // batches of 32 rows: [kt][row]
             int b = j / MEGA_BATCH, jb = j % MEGA_BATCH, nb = n_c - MEGA_BATCH * b;
             if (nb > MEGA_BATCH) nb = MEGA_BATCH;
@@ -528,55 +557,55 @@ __device__ __noinline__ void prologue_attn_poll(const MegaArgs &a, unsigned epoc
 }
 
 // down_proj input: poll the SwiGLU outputs (zone H) and group-quantise them into shared memory (layers.rs:478).
-// The loads of the next float4 of a thread are in flight while the current one is checked and quantised.
-template <int GS>
-__device__ __forceinline__ void quant_ll_one(const MegaArgs &a, const unsigned long long *z, unsigned epoch, int i4, int n4, unsigned long long (&w)[4],
-                                             unsigned &spins, uint8_t *sxq, float *sxs, int KT, int G) {
-    float4 y = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (i4 < n4) {
-        while (!(ll_ok(w[0], epoch) && ll_ok(w[1], epoch) && ll_ok(w[2], epoch) && ll_ok(w[3], epoch))) {
-            if (ll_give_up(a, spins, 8)) break;
-            ll_load2(z + (size_t)i4 * 4, w[0], w[1]);
-            ll_load2(z + (size_t)i4 * 4 + 2, w[2], w[3]);
-        }
-        y = make_float4(__uint_as_float((unsigned)w[0]), __uint_as_float((unsigned)w[1]), __uint_as_float((unsigned)w[2]), __uint_as_float((unsigned)w[3]));
-    }
-    uint32_t packed;
-    float scale;
-    quantize_group4<GS>(y, packed, scale); // warp-collective: the caller's loop condition is warp-uniform
-    if (i4 < n4) {
-        xq_store<GS>(sxq, i4, packed, KT, G);
-        if ((i4 % (GS / 4)) == 0) sxs[i4 / (GS / 4)] = scale;
-    }
-}
+// A thread takes its float4s three at a time: the loads of all three are in flight together, each is re-polled until it
+// carries `epoch`, and only then are the three quantised, as three independent chains the scheduler can interleave (a
+// quantisation is a latency-bound chain of shuffles, a division and a rounding).  Six at a time was slower.
 template <int GS>
 __device__ __noinline__ void prologue_quant_ll(const MegaArgs &a, const unsigned long long *z, unsigned epoch, int n, uint8_t *sxq, float *sxs, int KT, int G) {
+    constexpr int D = 3;
     const int tid = threadIdx.x, lane = tid & 31;
     const int n4 = n >> 2;
-    unsigned long long wa[4] = {0, 0, 0, 0}, wb[4] = {0, 0, 0, 0};
     unsigned spins = 0;
-    int i4 = tid;
-    if (i4 < n4) {
-        ll_load2(z + (size_t)i4 * 4, wa[0], wa[1]);
-        ll_load2(z + (size_t)i4 * 4 + 2, wa[2], wa[3]);
-    }
 #pragma unroll 1
-    while (i4 - lane < n4) {
-        int j4 = i4 + MEGA_CTHREADS;
-        if (j4 < n4) {
-            ll_load2(z + (size_t)j4 * 4, wb[0], wb[1]);
-            ll_load2(z + (size_t)j4 * 4 + 2, wb[2], wb[3]);
+    for (int i0 = tid; i0 - lane < n4; i0 += D * MEGA_CTHREADS) {
+        unsigned long long w[D][4];
+#pragma unroll
+        for (int d = 0; d < D; d++) {
+            const int i4 = i0 + d * MEGA_CTHREADS;
+            w[d][0] = w[d][1] = w[d][2] = w[d][3] = 0;
+            if (i4 < n4) {
+                ll_load2(z + (size_t)i4 * 4, w[d][0], w[d][1]);
+                ll_load2(z + (size_t)i4 * 4 + 2, w[d][2], w[d][3]);
+            }
         }
-        quant_ll_one<GS>(a, z, epoch, i4, n4, wa, spins, sxq, sxs, KT, G);
-        i4 = j4;
-        if (!(i4 - lane < n4)) break;
-        j4 = i4 + MEGA_CTHREADS;
-        if (j4 < n4) {
-            ll_load2(z + (size_t)j4 * 4, wa[0], wa[1]);
-            ll_load2(z + (size_t)j4 * 4 + 2, wa[2], wa[3]);
+#pragma unroll
+        for (int d = 0; d < D; d++) {
+            const int i4 = i0 + d * MEGA_CTHREADS;
+            if (i4 < n4) {
+                while (!(ll_ok(w[d][0], epoch) && ll_ok(w[d][1], epoch) && ll_ok(w[d][2], epoch) && ll_ok(w[d][3], epoch))) {
+                    if (ll_give_up(a, spins, 8)) break;
+                    ll_load2(z + (size_t)i4 * 4, w[d][0], w[d][1]);
+                    ll_load2(z + (size_t)i4 * 4 + 2, w[d][2], w[d][3]);
+                }
+            }
         }
-        quant_ll_one<GS>(a, z, epoch, i4, n4, wb, spins, sxq, sxs, KT, G);
-        i4 = j4;
+#pragma unroll
+        for (int d = 0; d < D; d++) {
+            const int i4 = i0 + d * MEGA_CTHREADS;
+            if (i4 - lane < n4) { // warp-uniform: quantize_group4 is warp-collective
+                float4 y = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (i4 < n4)
+                    y = make_float4(__uint_as_float((unsigned)w[d][0]), __uint_as_float((unsigned)w[d][1]), __uint_as_float((unsigned)w[d][2]),
+                                    __uint_as_float((unsigned)w[d][3]));
+                uint32_t packed;
+                float scale;
+                quantize_group4<GS>(y, packed, scale);
+                if (i4 < n4) {
+                    xq_store<GS>(sxq, i4, packed, KT, G);
+                    if ((i4 % (GS / 4)) == 0) sxs[i4 / (GS / 4)] = scale;
+                }
+            }
+        }
     }
     csync();
 }
@@ -1000,6 +1029,7 @@ struct PhaseGeom {
 struct MegaShared {
     int start[5], count[5];
     long long seg_off[5], seg_len[5];
+    GuMap gu;
     unsigned long long *part[2][MEGA_MAX_TP];
     float *logits[MEGA_MAX_TP];
     unsigned long long *best[MEGA_MAX_TP];
@@ -1052,6 +1082,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
             sh.seg_off[ph] = st * per_unit;
             sh.seg_len[ph] = cn * per_unit;
         }
+        sh.gu = gu_map(a.g[PH_GU].units, gridDim.x, blockIdx.x);
     }
     if (tid < MEGA_MAX_TP) {
         sh.part[0][tid] = a.part[0][tid];
@@ -1270,7 +1301,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) k_mega_decode(const __grid_co
                     }
                     if (wl < np && lane == 0) {
                         float sw = __fmul_rn(gate, __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-gate))));
-                        ll_store(a.zh + start + p0 + wl, __fmul_rn(sw, up), ep_h);
+                        ll_store(a.zh + gu_unit(sh.gu, p0 + wl), __fmul_rn(sw, up), ep_h);
                     }
                 }
             } else {
